@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the PyMOC time-stepping hot path (BASELINE.json metric: member-timesteps/sec, fp64).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference] [--dump-outputs DIR]
 
 One bench "step" = one fused-kernel pass advancing every member of the ensemble by
 ``--nt`` model time steps (default: the workload's N from SURVEY.md section 8d).  Under
@@ -30,6 +30,9 @@ Keys beyond the base contract:
                 carried streamfunctions back).  ``stateless``: through pmoc_model_run_host, which also re-uploads
                 every parameter array each call (round 1's e2e).  ``cadence120``: the handle called every 120 model
                 steps, the diagnostic cadence of run_JansenNadeau_2018.py:218-226.
+
+``--dump-outputs DIR`` writes what the headline workload's timed launches computed (see dump_outputs), so that two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -110,6 +113,21 @@ NCU_FACTS = {  # round 2, profiles/r2_full_summary.txt (captures of the final ke
     # (block-per-member step kernel; its launches also read the per-member coefficient scratch)
     'C5_4096': dict(pipe=23.7, flops=187792., dram=(870.51e6 + 603.98e6) / 2048, source='profiles/r2_full_summary.txt'),
 }
+
+
+def dump_outputs(ens, out_dir, budget=60e6, seed=0):
+  """Write the arrays a caller of the timed path receives after its last launch -- ``ens.state()`` and
+  ``ens.diagnostics()`` -- as ``out_dir/<name>.npy`` in float64, for a fixed seeded sample of members sized so that
+  all files together stay under 64 MB (``budget`` leaves room for the .npy headers); ``members.npy`` holds the
+  sampled member indices."""
+  outs = {**ens.state(), **ens.diagnostics()}
+  per_member = 8 * (1 + sum(a.size // a.shape[0] for a in outs.values()))
+  n = min(ens.M, int(budget // per_member))
+  idx = np.sort(np.random.default_rng(seed).choice(ens.M, size=n, replace=False))
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, 'members.npy'), idx.astype(np.float64))
+  for name, a in outs.items():
+    np.save(os.path.join(out_dir, name + '.npy'), a[idx].astype(np.float64))
 
 
 def config_of(workload, spec, m_local, world, nt):
@@ -364,6 +382,8 @@ def gpu_arm(args):
   assert gathered.shape[0] == M
   # the lattices hold no member that the (explicit, CFL-limited) reference loses
   assert main['status_counts']['nan'] == 0, '%d of %d members non-finite' % (main['status_counts']['nan'], ens.M)
+  if args.dump_outputs and rank == 0:  # (rank 0's members)
+    dump_outputs(ens, args.dump_outputs)
   del ens
 
   e2e = None
@@ -475,7 +495,11 @@ def main():
   ap.add_argument('--cpu-steps', type=int, default=0, help='model steps per CPU-baseline task (0: sized for ~15 s)')
   ap.add_argument('--no-cpu', action='store_true')
   ap.add_argument('--extras', default='all', help="'all', 'none' or a comma list: other workloads timed in the same run")
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write the outputs of the last timed launch of the headline workload as DIR/<name>.npy')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
   args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
   if args.impl == 'reference':
     reference_arm(args)

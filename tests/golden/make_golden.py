@@ -200,13 +200,19 @@ def run_reference(case, checkpoints, diag_iters=None):
   return snaps
 
 
-def coupled_fixture(fname, spec, members, checkpoints, extra=None):
+def coupled_fixture(fname, spec, members, checkpoints, extra=None, levels=None):
+  """``levels``: store the outputs on the z grid at these levels only (tests/helpers.on_stored_levels)."""
   tree = dict(versions=VERSIONS, name=spec.name, members={})
   if extra:
     tree.update(extra)
+  if levels is not None:
+    tree['levels'] = levels
   for m in members:
     case = spec.member_case(m)
-    tree['members'][str(m)] = dict(case=case, runs=run_reference(case, checkpoints))
+    runs = run_reference(case, checkpoints)
+    if levels is not None:
+      runs = {n: {k: v[levels] if v.shape == spec.z.shape else v for k, v in s.items()} for n, s in runs.items()}
+    tree['members'][str(m)] = dict(case=case, runs=runs)
     print('  %s member %d done' % (fname, m), flush=True)
   save_tree(os.path.join(HERE, fname), tree)
 
@@ -440,8 +446,9 @@ if __name__ == '__main__':
   if want('c5_4096'):
     coupled_fixture('c5_4096.npz', configs.c5_single_global_basin(1, nz=4096, dt_days=0.01), [0], [1, 40])
   # the same grid with the streamfunctions re-diagnosed every 20 iterations (MOC_up_iters is a free parameter of the
-  # script): the block-wide diagnosis kernel is exercised INSIDE a run at nz = 4096, three times in 45 steps
+  # script): the block-wide diagnosis kernel is exercised INSIDE a run at nz = 4096, three times in 45 steps.
+  # Every third level (0 ... 4095) is stored, which keeps the file under 1 MB.
   if want('c5_4096_k20'):
     spec = configs.c5_single_global_basin(2, nz=4096, dt_days=0.01, axes=(2, 1, 1, 1))
     spec.K = 20
-    coupled_fixture('c5_4096_k20.npz', spec, [0, 1], [20, 21, 45])
+    coupled_fixture('c5_4096_k20.npz', spec, [0, 1], [20, 21, 45], levels=np.arange(0, spec.nz, 3))

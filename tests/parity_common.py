@@ -4,7 +4,7 @@ import os
 
 import numpy as np
 
-from helpers import golden, relmax, spec_from_cases
+from helpers import golden, on_stored_levels, relmax, spec_from_cases
 from pymoc_b200.ensemble import Ensemble
 
 # north_star: 1e-10 relative (max-norm per field, SURVEY.md section 8c) on the explicit path
@@ -33,7 +33,7 @@ def run_against_golden(backend, name, nmax, tol=TOL, chunked=False):
       for key, want in d['runs'][str(n)].items():
         if key not in got:
           continue
-        err = relmax(got[key][i], want)
+        err = relmax(on_stored_levels(tree, got[key][i]), want)
         worst = max(worst, err)
         assert err < tol, '%s member %s step %d field %s: rel err %.3e' % (name, m, n, key, err)
     assert not (got['status'] & 1).any(), 'NaN status raised'

@@ -40,6 +40,34 @@ def test_reference_arm_prints_one_json_line():
   assert d['e2e']['h2d_bytes_per_step'] == 0 and d['e2e']['d2h_bytes_per_step'] == 0
 
 
+def test_dump_outputs_writes_a_fixed_sample_of_every_output(tmp_path):
+  """--dump-outputs: every array of state() and diagnostics() as float64 .npy, for the same seeded member sample
+  on every call, within the byte budget (the kernel sources run on the warp emulator)."""
+  import numpy as np
+
+  import bench
+  from emu.emu_backend import EmuBackend
+  from pymoc_b200 import configs
+  from pymoc_b200.ensemble import Ensemble
+  ens = Ensemble(configs.c3_twocol_so(64, axes=(4, 4, 2, 2)), backend=EmuBackend())
+  ens.run(5)
+  outs = {**ens.state(), **ens.diagnostics()}
+  per_member = 8 * (1 + sum(a.size // a.shape[0] for a in outs.values()))
+  for run in ('a', 'b'):
+    bench.dump_outputs(ens, str(tmp_path / run), budget=20 * per_member)
+  files = sorted(p.name for p in (tmp_path / 'a').iterdir())
+  assert files == sorted(['members.npy'] + [k + '.npy' for k in outs])
+  idx = np.load(tmp_path / 'a' / 'members.npy').astype(int)
+  assert idx.size == 20 and len(set(idx)) == 20 and np.array_equal(idx, np.sort(idx))
+  assert sum(os.path.getsize(tmp_path / 'a' / f) for f in files) <= 20 * per_member + 128 * len(files)
+  for name, a in outs.items():
+    got = np.load(tmp_path / 'a' / (name + '.npy'))
+    assert got.dtype == np.float64 and np.array_equal(got, a[idx].astype(np.float64)), name
+    assert np.array_equal(got, np.load(tmp_path / 'b' / (name + '.npy'))), name
+  bench.dump_outputs(ens, str(tmp_path / 'all'))  # a small ensemble fits the budget whole
+  assert np.array_equal(np.load(tmp_path / 'all' / 'members.npy'), np.arange(64))
+
+
 def test_both_arms_print_the_same_config_and_facts_are_consistent():
   """`config` is a function of the command line and the workload definition only (the driver compares the two arms'),
   and every ncu fact / extra workload names a workload that exists."""

@@ -188,9 +188,12 @@ int pmoc_model_diagnose(const pmoc_model* m, void* stream);
  * run_single_global_basin.py:172-229. */
 int pmoc_model_run(const pmoc_model* m, int64_t it0, int64_t nsteps, void* stream);
 
-/* Same as diagnose (when it0 == 0) + run, but every pointer in `m` is a HOST pointer: device
- * buffers are allocated, inputs copied in, the fused kernel run, and state + diagnostics
- * copied back before returning (synchronous).  This is the call a non-torch consumer binds. */
+/* Same as diagnose (when it0 == 0, order 'post') + run, but every pointer in `m` is a HOST pointer: the
+ * stateless form of the handle below (open, one step, close), with the same device mirror and block loop.
+ * Grids, parameters and the state (PMOC_IO_STATE) go up every call, the carried streamfunctions
+ * (PMOC_IO_PSI) when the launch continues an earlier one; the state comes back, the streamfunctions and
+ * diagnostics (PMOC_IO_PSI | PMOC_IO_DIAG) when the call diagnoses, and ml_Psi_s when it steps.
+ * Synchronous.  This is the call a non-torch consumer binds. */
 int pmoc_model_run_host(const pmoc_model* m, int64_t it0, int64_t nsteps);
 /* bytes the last pmoc_model_run_host / pmoc_host_open / pmoc_host_step of this thread copied
  * host->device / device->host */
@@ -200,7 +203,8 @@ void pmoc_host_last_bytes(uint64_t* h2d, uint64_t* d2h);
  * diagnostics every Diag_iters, run_JansenNadeau_2018.py:201-261) for a consumer that keeps its arrays in HOST
  * memory and calls in every few iterations.  pmoc_host_open mirrors every array of `m` (HOST pointers, which must
  * stay valid until pmoc_host_close; pin them for full copy bandwidth) on the device once -- grids, parameters,
- * state -- from a memory pool private to the library, and keeps three streams.  pmoc_host_step advances
+ * state, carried streamfunctions; the diagnostics start at zero -- from a memory pool private to the library,
+ * and keeps three streams.  pmoc_host_step advances
  * iterations [it0, it0 + nsteps) and moves only the array classes asked for, pipelined over blocks of members so
  * that copies overlap the fused kernel:
  *   push: copied host->device before the launch (0 = the device copy is current: nothing goes up);

@@ -14,7 +14,6 @@ namespace pmk {
 
 
 
-#ifndef PMOC_EMU
 #define PM_CUDA_OK(expr)                                                                      \
   do {                                                                                        \
     cudaError_t e_ = (expr);                                                                  \
@@ -23,7 +22,6 @@ namespace pmk {
       return e_ == cudaErrorNoDevice || e_ == cudaErrorInsufficientDriver ? PMOC_ENODEVICE : PMOC_ECUDA; \
     }                                                                                         \
   } while (0)
-#endif
 
 static inline int fail(int code, const char* msg) {
   std::snprintf(g_err, sizeof(g_err), "%s", msg);

@@ -1,6 +1,13 @@
-// Host-buffer entry point (pmoc_model_run_host) and the FP64 roofline probe.
+// Host-buffer entry points and the FP64 roofline probe.
+//
+// The stateless call (pmoc_model_run_host) and the persistent handle (pmoc_host_open / step / close) share one
+// device mirror of the caller's host arrays.  Every per-member array of the mirror carries a class bitmask; a
+// call names the classes that go up before its launches and come back after them, and one block loop moves
+// them (Mirror::pass, with Mirror::copy).  The emulator build runs this same code on host stand-ins of the
+// CUDA runtime calls (pmoc_rt.cuh).
 #include "pmoc_common.cuh"
 
+#include <algorithm>
 #include <mutex>
 #include <new>
 #include <vector>
@@ -12,16 +19,19 @@ extern "C" void pmoc_host_last_bytes(uint64_t* h2d, uint64_t* d2h) {
   if (d2h) *d2h = g_d2h_bytes;
 }
 
-#ifndef PMOC_EMU
 namespace {
 
-// Mirrors the host arrays of a pmoc_model on the device for the duration of one call, and pipelines the
-// call over blocks of members: block c's host->device copies, kernel and device->host copies are queued on
-// stream c % kStreams, so the copies of one block overlap the kernel of another (members are independent).
+// Mirrors the host arrays of a pmoc_model on the device, and pipelines a call over blocks of members: block c's
+// host->device copies, kernel and device->host copies are queued on stream c % kStreams, so the copies of one
+// block overlap the kernel of another (members are independent).
 constexpr int kStreams = 3;
 #ifndef PMOC_HOST_BLOCK_MEMBERS
 #define PMOC_HOST_BLOCK_MEMBERS 4096  // 16 blocks for the 65,536-member bench: fill/drain of the pipeline ~6 % of the copies
 #endif
+
+// Classes besides the public PMOC_IO_STATE / PSI / DIAG, which pmoc_host_step rejects: the per-member parameter
+// vectors, and the arrays every stepping launch writes whether or not it diagnoses (ml_Psi_s, also DIAG).
+constexpr unsigned kIoParam = 8u, kIoStepped = 16u;
 
 struct Mirror {
   struct Field {
@@ -30,18 +40,16 @@ struct Mirror {
     size_t slot;       // byte offset of the pointer inside pmoc_model
     size_t per_member; // bytes per member; 0 = shared by all members
     size_t bytes;      // total bytes
-    bool in, out;      // copied in / copied back (pmoc_model_run_host)
-    unsigned cat;      // PMOC_IO_* class of a state / streamfunction / diagnostic array, 0 for parameters (pmoc_host_step)
+    unsigned cat;      // class bits of a per-member array
   };
   cudaStream_t s[kStreams] = {};
   cudaEvent_t shared_ready = nullptr;
   std::vector<Field> fields;
   std::vector<void*> allocs;
   cudaError_t err = cudaSuccess;
-  const pmoc_model* h;
-  pmoc_model d;
+  pmoc_model d;       // the caller's model with the device pointers
   cudaMemPool_t pool = nullptr;
-  unsigned cat = 0;  // class given to the fields registered next
+  bool fresh = true;  // nothing uploaded yet
 
   // Streams, event and the library's own memory pool.  The pool is private (one per device, created on first
   // use, kept for the life of the process with its memory retained between calls): the embedding application's
@@ -69,15 +77,24 @@ struct Mirror {
       if ((e = cudaStreamCreateWithFlags(&s[i], cudaStreamNonBlocking)) != cudaSuccess) return e;
     return cudaEventCreateWithFlags(&shared_ready, cudaEventDisableTiming);
   }
-  // frees what init() and alloc() acquired, on every path (streams and event may be partly created)
-  cudaError_t fini() {
+  // waits for every stream (they may be partly created); the first error
+  cudaError_t sync() {
     cudaError_t e = cudaSuccess;
-    for (int i = kStreams - 1; i >= 0; --i) {  // stream 0 last: it owns the allocations
-      if (i == 0) release();
+    for (int i = 0; i < kStreams; ++i)
       if (s[i]) {
         const cudaError_t ei = cudaStreamSynchronize(s[i]);
         if (e == cudaSuccess) e = ei;
       }
+    return e;
+  }
+  // frees what init() and alloc() acquired, on every path
+  cudaError_t fini() {
+    cudaError_t e = sync();
+    for (void* p : allocs) cudaFreeAsync(p, s[0]);  // stream 0 owns the allocations; the others are idle now
+    allocs.clear();
+    if (s[0]) {
+      const cudaError_t e0 = cudaStreamSynchronize(s[0]);
+      if (e == cudaSuccess) e = e0;
     }
     for (int i = 0; i < kStreams; ++i)
       if (s[i]) { cudaStreamDestroy(s[i]); s[i] = nullptr; }
@@ -93,30 +110,26 @@ struct Mirror {
   }
   // register the pointer stored at `slot` of the model (hp: its host value)
   template <class P>
-  void add(P* slot, const void* hp, size_t per_member, size_t bytes, bool in, bool out) {
+  void add(P* slot, const void* hp, size_t per_member, size_t bytes, unsigned cat) {
     if (!hp) return;
     char* dp = static_cast<char*>(alloc(bytes));
-    fields.push_back({(char*)hp, dp, (size_t)((char*)slot - (char*)&d), per_member, bytes, in, out, cat});
+    fields.push_back({(char*)hp, dp, (size_t)((char*)slot - (char*)&d), per_member, bytes, cat});
     *slot = reinterpret_cast<P>(dp);
   }
   void vec(pmoc_vec* dv, long long M, size_t len) {  // input vector: per member when mstride != 0
     if (!dv->ptr) return;
     const size_t stride = (size_t)dv->mstride * sizeof(double);
     const size_t bytes = stride ? (size_t)(M - 1) * stride + len * sizeof(double) : len * sizeof(double);
-    add(&dv->ptr, dv->ptr, stride, bytes, true, false);
+    add(&dv->ptr, dv->ptr, stride, bytes, kIoParam);
   }
   template <class T>
-  void shared(const T** dp, size_t n) { add(dp, *dp, 0, n * sizeof(T), true, false); }
+  void shared(const T** dp, size_t n) { add(dp, *dp, 0, n * sizeof(T), 0); }
   template <class T>
-  void state(T** dp, long long M, size_t len, bool upload, bool download = true) {  // per-member in/out array
-    add(dp, *dp, len * sizeof(T), (size_t)M * len * sizeof(T), upload, download);
-  }
+  void state(T** dp, long long M, size_t len, unsigned cat) { add(dp, *dp, len * sizeof(T), (size_t)M * len * sizeof(T), cat); }
   void column(pmoc_column* c, long long M, int nz) {
-    cat = PMOC_IO_STATE;
-    state(&c->b, M, nz, true);
-    state(&c->bbot, M, 1, true);
-    state(&c->var, M, 1, true);
-    cat = 0;
+    state(&c->b, M, nz, PMOC_IO_STATE);
+    state(&c->bbot, M, 1, PMOC_IO_STATE);
+    state(&c->var, M, 1, PMOC_IO_STATE);
     vec(&c->kappa, M, (size_t)c->nvar * nz);
     vec(&c->dAk, M, (size_t)c->nvar * nz);
     vec(&c->Area, M, nz);
@@ -124,71 +137,12 @@ struct Mirror {
     vec(&c->N2min, M, 1);
     vec(&c->bzbot, M, 1);
   }
-  void upload_shared() {
-    for (auto& f : fields)
-      if (!f.per_member && f.in && err == cudaSuccess) {
-        err = cudaMemcpyAsync(f.dev, f.host, f.bytes, cudaMemcpyHostToDevice, s[0]);
-        g_h2d_bytes += f.bytes;
-      }
-    if (err == cudaSuccess) err = cudaEventRecord(shared_ready, s[0]);
-  }
-  // members [m0, m0+n) in, on stream st; the last member of an input vector may be shorter than its stride
-  void upload_block(long long m0, long long n, long long M, cudaStream_t st) {
-    for (auto& f : fields) {
-      if (!f.per_member || err != cudaSuccess) continue;
-      const size_t off = (size_t)m0 * f.per_member;
-      size_t len = (size_t)n * f.per_member;
-      if (off + len > f.bytes) len = f.bytes - off;
-      err = f.in ? cudaMemcpyAsync(f.dev + off, f.host + off, len, cudaMemcpyHostToDevice, st)
-                 : cudaMemsetAsync(f.dev + off, 0, len, st);
-      if (f.in) g_h2d_bytes += len;
-    }
-  }
-  // pmoc_host_step: only the per-member arrays whose class is in `mask` move
-  void push_block(long long m0, long long n, unsigned mask, cudaStream_t st) {
-    for (auto& f : fields) {
-      if (!f.per_member || !(f.cat & mask) || err != cudaSuccess) continue;
-      const size_t off = (size_t)m0 * f.per_member;
-      err = cudaMemcpyAsync(f.dev + off, f.host + off, (size_t)n * f.per_member, cudaMemcpyHostToDevice, st);
-      g_h2d_bytes += (size_t)n * f.per_member;
-    }
-  }
-  void pull_block(long long m0, long long n, unsigned mask, cudaStream_t st) {
-    for (auto& f : fields) {
-      if (!f.per_member || !(f.cat & mask) || err != cudaSuccess) continue;
-      const size_t off = (size_t)m0 * f.per_member;
-      err = cudaMemcpyAsync(f.host + off, f.dev + off, (size_t)n * f.per_member, cudaMemcpyDeviceToHost, st);
-      g_d2h_bytes += (size_t)n * f.per_member;
-    }
-  }
-  void download_block(long long m0, long long n, cudaStream_t st) {
-    for (auto& f : fields) {
-      if (!f.per_member || !f.out || err != cudaSuccess) continue;
-      const size_t off = (size_t)m0 * f.per_member;
-      err = cudaMemcpyAsync(f.host + off, f.dev + off, (size_t)n * f.per_member, cudaMemcpyDeviceToHost, st);
-      g_d2h_bytes += (size_t)n * f.per_member;
-    }
-  }
-  // the device model restricted to members [m0, m0+n)
-  pmoc_model block_model(long long m0, long long n) const {
-    pmoc_model b = d;
-    b.M = n;
-    for (auto& f : fields)
-      if (f.per_member) *reinterpret_cast<char**>((char*)&b + f.slot) = f.dev + (size_t)m0 * f.per_member;
-    return b;
-  }
-  void release() {
-    for (void* p : allocs) cudaFreeAsync(p, s[0]);
-    allocs.clear();
-  }
-
-  // Register every array of the model.  `carry` / `rewritten` say which streamfunctions one stateless call
-  // uploads / brings back (pmoc_model_run_host); the handle API moves them by class instead.
-  void describe(bool carry, bool rewritten, bool stepped) {
+  // register every array of the model, with its class
+  void describe() {
     const long long M = d.M;
     const int nz = d.nz, ny = d.ny, nb = d.nb;
     const unsigned f = d.flags;
-    cat = 0;
+    const unsigned S = PMOC_IO_STATE, P = PMOC_IO_PSI, D = PMOC_IO_DIAG;
     shared(&d.z, nz);
     shared(&d.y, ny);
     column(&d.basin, M, nz);
@@ -197,15 +151,14 @@ struct Mirror {
       column(&d.pac, M, nz);
       vec(&d.zoc_f, M, 1);
       vec(&d.so2_L, M, 1);
-      cat = PMOC_IO_DIAG; state(&d.Psi_zoc, M, nz, false, rewritten);
-      cat = PMOC_IO_PSI; state(&d.Psi_zon_a, M, nz, carry, rewritten);
-      state(&d.Psi_zon_p, M, nz, carry, rewritten);
-      cat = PMOC_IO_DIAG; state(&d.psib2, M, nb, false, rewritten);
-      state(&d.bgrid2, M, nb, false, rewritten);
-      cat = PMOC_IO_PSI; state(&d.Psi_so2, M, nz, carry, rewritten);
-      cat = PMOC_IO_DIAG; state(&d.Psi_Ek2, M, nz, false, rewritten);
-      state(&d.Psi_GM2, M, nz, false, rewritten);
-      cat = 0;
+      state(&d.Psi_zoc, M, nz, D);
+      state(&d.Psi_zon_a, M, nz, P);
+      state(&d.Psi_zon_p, M, nz, P);
+      state(&d.psib2, M, nb, D);
+      state(&d.bgrid2, M, nb, D);
+      state(&d.Psi_so2, M, nz, P);
+      state(&d.Psi_Ek2, M, nz, D);
+      state(&d.Psi_GM2, M, nz, D);
     }
     vec(&d.tw_f, M, 1);
     vec(&d.tw_b2, M, nz);
@@ -221,8 +174,7 @@ struct Mirror {
     shared(&d.so_ek_taper, nz);
     shared(&d.so_top_taper, nz);
     shared(&d.so_bot_taper, nz);
-    cat = PMOC_IO_STATE; state(&d.ml_bs, M, ny, true);
-    cat = 0;
+    state(&d.ml_bs, M, ny, S);
     vec(&d.ml_Ks, M, 1);
     vec(&d.ml_h, M, 1);
     vec(&d.ml_L, M, 1);
@@ -230,18 +182,16 @@ struct Mirror {
     vec(&d.ml_surflux, M, ny);
     vec(&d.ml_rest_mask, M, ny);
     vec(&d.ml_b_rest, M, ny);
-    const bool iso = (f & PMOC_ISO) != 0;
-    cat = iso ? PMOC_IO_DIAG : PMOC_IO_PSI; state(&d.Psi_tw, M, nz, carry && !iso, rewritten);
-    cat = PMOC_IO_PSI; state(&d.Psi_iso_b, M, nz, carry, rewritten);
-    state(&d.Psi_iso_n, M, nz, carry, rewritten);
-    cat = PMOC_IO_DIAG; state(&d.psib, M, nb, false, rewritten);
-    state(&d.bgrid, M, nb, false, rewritten);
-    cat = PMOC_IO_PSI; state(&d.Psi_so, M, nz, carry, rewritten);
-    cat = PMOC_IO_DIAG; state(&d.Psi_Ek, M, nz, false, rewritten);
-    state(&d.Psi_GM, M, nz, false, rewritten);
-    state(&d.ml_Psi_s, M, ny, false, stepped);
-    cat = PMOC_IO_STATE; state(&d.status, M, 1, true);
-    cat = 0;
+    state(&d.Psi_tw, M, nz, (f & PMOC_ISO) ? D : P);
+    state(&d.Psi_iso_b, M, nz, P);
+    state(&d.Psi_iso_n, M, nz, P);
+    state(&d.psib, M, nb, D);
+    state(&d.bgrid, M, nb, D);
+    state(&d.Psi_so, M, nz, P);
+    state(&d.Psi_Ek, M, nz, D);
+    state(&d.Psi_GM, M, nz, D);
+    state(&d.ml_Psi_s, M, ny, D | kIoStepped);
+    state(&d.status, M, 1, S);
   }
   // blocks of members: enough of them to overlap copies with kernels, each large enough to fill the GPU; one
   // scratch buffer per stream for the block-per-member kernels (nz > 256)
@@ -255,7 +205,7 @@ struct Mirror {
     per = (M + nblk - 1) / nblk;
     d.scratch = nullptr;
     d.scratch_bytes = 0;
-    pmoc_model one = *h;
+    pmoc_model one = d;
     one.M = per;
     const uint64_t need = pmoc_model_scratch_bytes(&one);
     if (need) {
@@ -263,67 +213,103 @@ struct Mirror {
       d.scratch_bytes = need;
     }
   }
+  // The shared arrays go up on stream 0 behind the allocations, and the other streams wait for both.
+  void upload_shared() {
+    for (auto& f : fields)
+      if (!f.per_member && err == cudaSuccess) {
+        err = cudaMemcpyAsync(f.dev, f.host, f.bytes, cudaMemcpyHostToDevice, s[0]);
+        g_h2d_bytes += f.bytes;
+      }
+    if (err == cudaSuccess) err = cudaEventRecord(shared_ready, s[0]);
+    for (int i = 1; i < kStreams && err == cudaSuccess; ++i) err = cudaStreamWaitEvent(s[i], shared_ready, 0);
+  }
+  // streams, a device copy of every array of `m`, the shared arrays uploaded
+  cudaError_t open(const pmoc_model* m) {
+    d = *m;
+    err = init();
+    if (err == cudaSuccess) {
+      describe();
+      plan_blocks();
+    }
+    if (err == cudaSuccess) upload_shared();
+    return err;
+  }
+
+  // Members [m0, m0+n) of the per-member arrays whose class is in `mask`, host->device (`up`) or back, on
+  // stream st; the last member of a parameter vector may be shorter than its stride.  With `fill`, the device
+  // copy of every other per-member array is zeroed.
+  void copy(long long m0, long long n, unsigned mask, bool up, bool fill, cudaStream_t st) {
+    for (auto& f : fields) {
+      if (!f.per_member || err != cudaSuccess) continue;
+      const size_t off = (size_t)m0 * f.per_member, len = std::min((size_t)n * f.per_member, f.bytes - off);
+      if (!(f.cat & mask)) {
+        if (fill) err = cudaMemsetAsync(f.dev + off, 0, len, st);
+      } else if (up) {
+        err = cudaMemcpyAsync(f.dev + off, f.host + off, len, cudaMemcpyHostToDevice, st);
+        g_h2d_bytes += len;
+      } else {
+        err = cudaMemcpyAsync(f.host + off, f.dev + off, len, cudaMemcpyDeviceToHost, st);
+        g_d2h_bytes += len;
+      }
+    }
+  }
+  // the device model restricted to members [m0, m0+n), with the scratch of stream `si`
+  pmoc_model block_model(long long m0, long long n, int si) const {
+    pmoc_model b = d;
+    b.M = n;
+    for (auto& f : fields)
+      if (f.per_member) *reinterpret_cast<char**>((char*)&b + f.slot) = f.dev + (size_t)m0 * f.per_member;
+    b.scratch = scratch[si];
+    return b;
+  }
+  // One call, block by block: the classes in `push` go up (the first upload zeroes every other per-member
+  // array), the block is diagnosed (`diag`) and run (`run`), and the classes in `pull` come back.  Returns the
+  // first launch error; a CUDA error is left in `err`.
+  int pass(unsigned push, bool diag, bool run, long long it0, long long nsteps, unsigned pull) {
+    int rc = PMOC_OK;
+    for (long long c = 0; c < nblk && rc == PMOC_OK && err == cudaSuccess; ++c) {
+      const long long m0 = c * per, n = std::min(per, d.M - m0);
+      if (n <= 0) break;
+      const int si = (int)(c % kStreams);
+      copy(m0, n, push, true, fresh, s[si]);
+      pmoc_model blk = block_model(m0, n, si);
+      if (diag) rc = pmoc_model_diagnose(&blk, s[si]);
+      if (rc == PMOC_OK && run) rc = pmoc_model_run(&blk, it0, nsteps, s[si]);
+      if (rc == PMOC_OK) copy(m0, n, pull, false, false, s[si]);
+    }
+    fresh = false;
+    return rc;
+  }
 };
 
 }  // namespace
-#endif
 
 extern "C" int pmoc_model_run_host(const pmoc_model* m, int64_t it0, int64_t nsteps) {
   if (!m) return fail(PMOC_EINVAL, "model is NULL");
   g_h2d_bytes = g_d2h_bytes = 0;
-#ifdef PMOC_EMU
-  if (it0 == 0 && !(m->flags & PMOC_ORDER_JN))
-    if (int rc = pmoc_model_diagnose(m, nullptr)) return rc;
-  return pmoc_model_run(m, it0, nsteps, nullptr);
-#else
   if (m->M <= 0 || m->nz < 3) return fail(PMOC_EINVAL, "bad M / nz");
-  const long long M = m->M;
-  const unsigned f = m->flags;
+  // Diagnostics: the kernel rewrites all of them at the last iteration with ii % K == 0 of the launch (and the
+  // pre-loop diagnosis of an order-'post' model at it0 == 0 does); without such an iteration they are left
+  // alone on both sides.  Only the streamfunctions the step loop carries from an earlier launch are inputs.
+  const long long K = m->K > 0 ? m->K : 1;
+  const bool jn = (m->flags & PMOC_ORDER_JN) != 0;
+  const bool rewritten = (!jn && it0 == 0) || (nsteps > 0 && ((it0 + nsteps - 1) / K) * K >= it0);
+  const bool carry = jn ? (it0 % K != 0) : (it0 > 0);
+  const unsigned push = kIoParam | PMOC_IO_STATE | (carry ? PMOC_IO_PSI : 0);
+  const unsigned pull = PMOC_IO_STATE | (rewritten ? PMOC_IO_PSI | PMOC_IO_DIAG : 0) | (nsteps > 0 ? kIoStepped : 0);
   Mirror mr;
-  mr.h = m;
-  mr.d = *m;
   int rc = PMOC_OK;
-  mr.err = mr.init();
-  if (mr.err == cudaSuccess) {
-    // Diagnostics: the kernel rewrites all of them at the last iteration with ii % K == 0 of the launch (and the
-    // pre-loop diagnosis of an order-'post' model at it0 == 0 does); without such an iteration they are left
-    // alone on both sides.  Only the streamfunctions the step loop carries from an earlier launch are inputs.
-    const long long K = m->K > 0 ? m->K : 1;
-    const bool jn = (f & PMOC_ORDER_JN) != 0;
-    const bool rewritten = (!jn && it0 == 0) || (nsteps > 0 && ((it0 + nsteps - 1) / K) * K >= it0);
-    const bool carry = jn ? (it0 % K != 0) : (it0 > 0);
-    mr.describe(carry, rewritten, nsteps > 0);
-    mr.plan_blocks();
-  }
-  if (mr.err == cudaSuccess) {
-    mr.upload_shared();
-    for (int i = 1; i < kStreams && mr.err == cudaSuccess; ++i) mr.err = cudaStreamWaitEvent(mr.s[i], mr.shared_ready, 0);
-    for (long long c = 0; c < mr.nblk && rc == PMOC_OK && mr.err == cudaSuccess; ++c) {
-      const long long m0 = c * mr.per, n = (m0 + mr.per <= M ? mr.per : M - m0);
-      if (n <= 0) break;
-      cudaStream_t st = mr.s[c % kStreams];
-      mr.upload_block(m0, n, M, st);
-      pmoc_model blk = mr.block_model(m0, n);
-      blk.scratch = mr.scratch[c % kStreams];
-      if (it0 == 0 && !(f & PMOC_ORDER_JN)) rc = pmoc_model_diagnose(&blk, st);
-      if (rc == PMOC_OK) rc = pmoc_model_run(&blk, it0, nsteps, st);
-      if (rc == PMOC_OK) mr.download_block(m0, n, st);
-    }
-  }
+  if (mr.open(m) == cudaSuccess) rc = mr.pass(push, !jn && it0 == 0, true, it0, nsteps, pull);
   const cudaError_t e = mr.fini();  // every path: streams, event and device memory are returned
   if (rc != PMOC_OK) return rc;
   PM_CUDA_OK(mr.err);
   PM_CUDA_OK(e);
   return PMOC_OK;
-#endif
 }
 
 // ---- persistent handle: parameters uploaded once, streams and device mirrors kept between calls ------------
 struct pmoc_host {
-#ifndef PMOC_EMU
   Mirror mr;
-#endif
-  pmoc_model host;  // the caller's struct (host pointers), copied
   bool diagnosed = false;
 };
 
@@ -333,37 +319,17 @@ extern "C" int pmoc_host_open(const pmoc_model* m, pmoc_host** out) {
   if (m->M <= 0 || m->nz < 3) return fail(PMOC_EINVAL, "bad M / nz");
   pmoc_host* h = new (std::nothrow) pmoc_host();
   if (!h) return fail(PMOC_EINVAL, "out of host memory");
-  h->host = *m;
   g_h2d_bytes = g_d2h_bytes = 0;
-#ifndef PMOC_EMU
   Mirror& mr = h->mr;
-  mr.h = &h->host;
-  mr.d = *m;
-  mr.err = mr.init();
-  if (mr.err == cudaSuccess) {
-    mr.describe(true, true, true);
-    mr.plan_blocks();
-  }
-  if (mr.err == cudaSuccess) {  // everything goes up once: grids, parameters, state, carried streamfunctions
-    mr.upload_shared();
-    for (auto& f : mr.fields) {
-      if (!f.per_member || mr.err != cudaSuccess) continue;
-      if (f.cat == PMOC_IO_DIAG) {  // outputs
-        mr.err = cudaMemsetAsync(f.dev, 0, f.bytes, mr.s[0]);
-        continue;
-      }
-      mr.err = cudaMemcpyAsync(f.dev, f.host, f.bytes, cudaMemcpyHostToDevice, mr.s[0]);
-      g_h2d_bytes += f.bytes;
-    }
-    if (mr.err == cudaSuccess) mr.err = cudaStreamSynchronize(mr.s[0]);
-  }
+  // everything goes up once: grids, parameters, state, carried streamfunctions; the diagnostics start at zero
+  if (mr.open(m) == cudaSuccess) mr.pass(kIoParam | PMOC_IO_STATE | PMOC_IO_PSI, false, false, 0, 0, 0);
+  if (mr.err == cudaSuccess) mr.err = mr.sync();
   if (mr.err != cudaSuccess) {
     const cudaError_t keep = mr.err;
     mr.fini();
     delete h;
     PM_CUDA_OK(keep);
   }
-#endif
   *out = h;
   return PMOC_OK;
 }
@@ -373,57 +339,32 @@ extern "C" int pmoc_host_step(pmoc_host* h, int64_t it0, int64_t nsteps, uint32_
   if ((push | pull) & ~(PMOC_IO_STATE | PMOC_IO_PSI | PMOC_IO_DIAG)) return fail(PMOC_EINVAL, "unknown PMOC_IO_* bit");
   if (push & PMOC_IO_DIAG) return fail(PMOC_EINVAL, "diagnostics are outputs: they cannot be pushed");
   g_h2d_bytes = g_d2h_bytes = 0;
-  const bool jn = (h->host.flags & PMOC_ORDER_JN) != 0;
+  Mirror& mr = h->mr;
+  const bool jn = (mr.d.flags & PMOC_ORDER_JN) != 0;
   // an order-'post' loop is entered with diagnosed streamfunctions (the scripts' pre-loop solve()): at it0 == 0,
   // and whenever the caller replaces the state without supplying streamfunctions that match it
   const bool need_diag = !jn && (it0 == 0 || ((push & PMOC_IO_STATE) && !(push & PMOC_IO_PSI) && !h->diagnosed));
-#ifdef PMOC_EMU
-  if (need_diag)
-    if (int rc = pmoc_model_diagnose(&h->host, nullptr)) return rc;
-  h->diagnosed = true;
-  return pmoc_model_run(&h->host, it0, nsteps, nullptr);
-#else
-  Mirror& mr = h->mr;
-  const long long M = mr.d.M;
-  int rc = PMOC_OK;
-  for (long long c = 0; c < mr.nblk && rc == PMOC_OK && mr.err == cudaSuccess; ++c) {
-    const long long m0 = c * mr.per, n = (m0 + mr.per <= M ? mr.per : M - m0);
-    if (n <= 0) break;
-    cudaStream_t st = mr.s[c % kStreams];
-    if (push) mr.push_block(m0, n, push, st);
-    pmoc_model blk = mr.block_model(m0, n);
-    blk.scratch = mr.scratch[c % kStreams];
-    if (need_diag) rc = pmoc_model_diagnose(&blk, st);
-    if (rc == PMOC_OK && nsteps > 0) rc = pmoc_model_run(&blk, it0, nsteps, st);
-    if (rc == PMOC_OK && pull) mr.pull_block(m0, n, pull, st);
-  }
-  cudaError_t e = cudaSuccess;
-  for (int i = 0; i < kStreams; ++i) {
-    const cudaError_t ei = cudaStreamSynchronize(mr.s[i]);
-    if (e == cudaSuccess) e = ei;
-  }
+  const int rc = mr.pass(push, need_diag, nsteps > 0, it0, nsteps, pull);
+  const cudaError_t e = mr.sync();
   if (rc != PMOC_OK) return rc;
   PM_CUDA_OK(mr.err);
   PM_CUDA_OK(e);
   h->diagnosed = true;
   return PMOC_OK;
-#endif
 }
 
 extern "C" int pmoc_host_close(pmoc_host* h) {
   if (!h) return PMOC_OK;
-#ifndef PMOC_EMU
   const cudaError_t e = h->mr.fini();
   delete h;
   PM_CUDA_OK(e);
-#else
-  delete h;
-#endif
   return PMOC_OK;
 }
 
 // ------------------------------------------------------------------------------------------
-#ifndef PMOC_EMU
+#ifdef PMOC_EMU
+extern "C" int pmoc_fp64_peak(double*, double*, void*) { return fail(PMOC_ENODEVICE, "the FP64 probe needs a GPU"); }
+#else
 namespace {
 // 8 independent DFMA chains per thread, nothing else: what the FP64 pipe sustains.
 __global__ void k_fp64_peak(double* out, int iters, double seed) {
@@ -438,13 +379,8 @@ __global__ void k_fp64_peak(double* out, int iters, double seed) {
   if (s == 12345.678) out[0] = s;  // keep the chains alive
 }
 }  // namespace
-#endif
 
 extern "C" int pmoc_fp64_peak(double* tflops, double* sm_mhz_est, void* stream) {
-#ifdef PMOC_EMU
-  (void)tflops; (void)sm_mhz_est; (void)stream;
-  return fail(PMOC_ENODEVICE, "the FP64 probe needs a GPU");
-#else
   int dev = 0, sms = 0;
   PM_CUDA_OK(cudaGetDevice(&dev));
   PM_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -476,5 +412,5 @@ extern "C" int pmoc_fp64_peak(double* tflops, double* sm_mhz_est, void* stream) 
   // 64 DFMA lanes per SM and clock
   if (sm_mhz_est) *sm_mhz_est = best * 1e12 / (2.0 * 64.0 * sms) / 1e6;
   return PMOC_OK;
-#endif
 }
+#endif

@@ -15,7 +15,10 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 CSRC = os.path.join(ROOT, 'pymoc_b200', 'csrc')
 OBJ = os.path.join(HERE, 'build')
 LIB = os.path.join(HERE, '_pmoc_emu.so')
-FLAGS = ['-O2', '-std=c++17', '-fPIC', '-ffp-contract=off', '-DPMOC_EMU', '-I', HERE, '-Wno-unknown-pragmas']
+# blocks of two members in the host-buffer entry points: a test-sized ensemble already spans several blocks
+# and all three streams
+FLAGS = ['-O2', '-std=c++17', '-fPIC', '-ffp-contract=off', '-DPMOC_EMU', '-DPMOC_HOST_BLOCK_MEMBERS=2', '-I', HERE,
+         '-Wno-unknown-pragmas']
 LPLS = (2, 3, 4, 5, 6, 7, 8)
 
 

@@ -127,9 +127,9 @@ def test_f2010_smoother_is_the_converged_solution(emu):
   f2010_smoother_converged(emu, sizes=(46, 80), bvp_tol=1e-8, tol=1e-8)
 
 
-def test_host_handle_api(emu):
-  """pmoc_host_open / step / close through the emulator build (host pointers are its native currency): same
-  results as pmoc_model_diagnose + pmoc_model_run, argument checks."""
+def test_host_handle_round_trip_and_argument_checks(emu):
+  """pmoc_host_open / step / close through the emulator build: state and streamfunctions pulled after one call and
+  pushed back before the next give the results of pmoc_model_diagnose + pmoc_model_run; argument checks."""
   import ctypes
 
   from pymoc_b200 import _abi, configs
@@ -138,7 +138,7 @@ def test_host_handle_api(emu):
   a = Ensemble(spec, backend=emu)
   a.run(30)
   b = HostEnsemble(spec, backend=emu)
-  b.run(13, pull=0)
+  b.run(13, pull=HostEnsemble.IO_STATE | HostEnsemble.IO_PSI)
   b.run(17, push=HostEnsemble.IO_STATE | HostEnsemble.IO_PSI)
   for k, v in a.state().items():
     assert np.array_equal(v, b.state()[k]), k
@@ -146,6 +146,7 @@ def test_host_handle_api(emu):
     assert np.array_equal(a.diagnostics()[k], b.diagnostics()[k]), k
   lib = emu.lib
   assert lib.pmoc_host_step(b._handle, 30, 1, 8, 0) == _abi.EINVAL            # unknown class bit
+  assert lib.pmoc_host_step(b._handle, 30, 1, 0, 16) == _abi.EINVAL           # (pull side too)
   assert lib.pmoc_host_step(b._handle, 30, 1, HostEnsemble.IO_DIAG, 0) == _abi.EINVAL  # diagnostics are outputs
   assert lib.pmoc_host_step(None, 0, 1, 0, 0) == _abi.EINVAL
   assert lib.pmoc_host_open(None, ctypes.byref(ctypes.c_void_p())) == _abi.EINVAL

@@ -236,12 +236,14 @@ int pmoc_column_timestep(int64_t M, int32_t nz, const double* z, const pmoc_colu
 int pmoc_thermwind_solve(int64_t M, int32_t nz, const double* z, pmoc_vec b1, pmoc_vec b2, pmoc_vec f,
                          pmoc_vec gmid, double* Psi, void* stream);
 
-/* Psi_Thermwind.Psib / Psibz (psi_thermwind.py:137-208).  Outputs optional except psib. */
+/* Psi_Thermwind.Psib / Psibz (psi_thermwind.py:137-208).  Outputs optional except psib.
+ * PMOC_EUNSUPPORTED when nb needs more shared memory than one block has (nb > 3816 at nz = 256). */
 int pmoc_thermwind_psib(int64_t M, int32_t nz, int32_t nb, pmoc_vec Psi, pmoc_vec b1, pmoc_vec b2,
                         double* psib, double* bgrid, double* iso_b, double* iso_n, void* stream);
 
 /* Psi_SO.solve (psi_SO.py:333-354) with ys/calc_Ekman/calc_GM inside.  `so` reuses the
- * Psi_SO fields of pmoc_model (so_*, y, ny, z, nz, M); b is the basin profile. */
+ * Psi_SO fields of pmoc_model (so_*, y, ny, z, nz, M); b is the basin profile.
+ * PMOC_EUNSUPPORTED when ny needs more shared memory than one block has (ny > 2136 at nz = 256). */
 int pmoc_so_solve(const pmoc_model* so, pmoc_vec b, pmoc_vec bs, double* Psi, double* Psi_Ek, double* Psi_GM,
                   double* ys, uint32_t* status, void* stream);
 

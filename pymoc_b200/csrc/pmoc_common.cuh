@@ -32,6 +32,7 @@ PM_DEV double vat(const pmoc_vec& v, long long m) { return v.ptr[m * v.mstride];
 PM_DEV const double* vrow(const pmoc_vec& v, long long m) { return v.ptr + m * v.mstride; }
 
 constexpr int kWarpsPerBlock = 4;  // per-module kernels; the fused kernel picks its own per launch (launch_model)
+constexpr size_t kMaxSmemPerBlock = 227 * 1024;  // dynamic shared memory one block of sm_100 may opt in to
 
 // ------------------------------------------------------------------------------------------
 // shared-memory plan (in doubles).  Per block: the grid tables; per warp (= member): the
@@ -214,6 +215,9 @@ PM_DEV void col_advance_exact(ColRegs<LPL>& c, const pm::ExactCol& X, const pm::
 #ifdef PMOC_EMU
 template <class K, class A>
 int launch(K kern, long long grid, int block, size_t smem, void*, const A& args) {
+  // the device refuses more dynamic shared memory than one block may opt in to (cudaFuncSetAttribute fails)
+  if (smem > kMaxSmemPerBlock)
+    return fail(PMOC_ECUDA, "emulated cudaFuncSetAttribute: dynamic shared memory above the per-block limit");
   pmemu::launch(grid, block, smem, [=]() { kern(args); });
   return PMOC_OK;
 }

@@ -215,6 +215,13 @@ PM_GLOBAL void k_ml(MlArgs a) {
   if (a.status && L == 0) a.status[m] |= status;
 }
 
+// A per-module kernel whose shared memory grows with nb / ny: refuse sizes one block cannot hold.
+static int fail_smem(const char* what, int n, size_t bytes) {
+  std::snprintf(g_err, sizeof(g_err), "%s = %d needs %zu bytes of shared memory per block, more than the %zu one block can use",
+                what, n, bytes, kMaxSmemPerBlock);
+  return PMOC_EUNSUPPORTED;
+}
+
 static int lpl_for(int nz) { return nz <= 64 ? 2 : (nz + 31) / 32; }
 
 #define PM_DISPATCH_LPL(nz, CALL)                          \
@@ -380,8 +387,9 @@ int pmoc_thermwind_psib(int64_t M, int32_t nz, int32_t nb, pmoc_vec Psi, pmoc_ve
   a.nbp = (nb + 3) & ~3;
   PM_DISPATCH_LPL(nz, {
     a.nzp = 32 * LPL;
-    return launch(k_psib<LPL>, blocks_for(M), 32 * kWarpsPerBlock,
-                  sizeof(double) * (size_t)(6 * a.nzp + a.nbp + a.nbp / 2 + 2) * kWarpsPerBlock, stream, a);
+    const size_t smem = sizeof(double) * (size_t)(6 * a.nzp + a.nbp + a.nbp / 2 + 2) * kWarpsPerBlock;
+    if (smem > kMaxSmemPerBlock) return fail_smem("nb", nb, smem);
+    return launch(k_psib<LPL>, blocks_for(M), 32 * kWarpsPerBlock, smem, stream, a);
   });
   return PMOC_OK;
 }
@@ -401,6 +409,7 @@ int pmoc_so_solve(const pmoc_model* so, pmoc_vec b, pmoc_vec bs, double* Psi, do
     a.nzp = 32 * LPL;
     const size_t smem =
         sizeof(double) * (size_t)(a.nzp + 4 + a.nyp + 4 * a.nzp + 3 * a.nyp * kWarpsPerBlock);
+    if (smem > kMaxSmemPerBlock) return fail_smem("ny", so->ny, smem);
     if (bvp) return launch(k_so<LPL, true>, blocks_for(so->M), 32 * kWarpsPerBlock, smem, stream, a);
     return launch(k_so<LPL, false>, blocks_for(so->M), 32 * kWarpsPerBlock, smem, stream, a);
   });

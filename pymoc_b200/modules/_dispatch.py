@@ -51,7 +51,11 @@ class Call:
     self.keep.append(buf)
     return buf
 
-  def check(self, rc):
+  def check(self, rc, who=None):
+    """Raise on an error return.  ``who``: the drop-in class, whose size limits (the library's EUNSUPPORTED) are
+    a ValueError, like its nz limit."""
+    if who is not None and rc == _abi.EUNSUPPORTED:
+      raise ValueError('pymoc_b200.modules.%s: %s' % (who, self.lib.pmoc_last_error().decode()))
     _abi.check(self.lib, rc)
 
   def get(self, buf):

@@ -56,7 +56,7 @@ class Psi_SO(object):
     outs = [c.out((1, z.size)) for _ in range(4)]
     status = c.out((1,), np.uint32)
     c.check(c.lib.pmoc_so_solve(byref(m), c.vec(b_profile), c.vec(self.bs(y) + 0 * y), *[c.be.ptr(o) for o in outs],
-                                c.be.ptr(status), c.be.stream()))
+                                c.be.ptr(status), c.be.stream()), 'Psi_SO')
     psi, ek_sv, gm_sv, ys = (c.get(o)[0] for o in outs)
     st = int(c.get(status).view(np.uint32)[0])
     if st & _abi.ST_BRENT_SIGN:

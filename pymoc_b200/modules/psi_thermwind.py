@@ -61,7 +61,7 @@ class Psi_Thermwind(object):
     iso_n = c.out((1, z.size)) if want_z else None
     c.check(c.lib.pmoc_thermwind_psib(1, z.size, int(nb), c.vec(np.asarray(self.Psi, dtype=np.float64)), c.vec(b1),
                                       c.vec(b2), c.be.ptr(psib), c.be.ptr(bgrid), c.be.ptr(iso_b), c.be.ptr(iso_n),
-                                      c.be.stream()))
+                                      c.be.stream()), 'Psi_Thermwind')
     self.bgrid = c.get(bgrid)[0]
     return c.get(psib)[0], (c.get(iso_b)[0] if want_z else None), (c.get(iso_n)[0] if want_z else None)
 

@@ -13,6 +13,8 @@ namespace pmemu {
 namespace {
 
 constexpr size_t kStack = 256 * 1024;
+constexpr size_t kMaxSmem = 227 * 1024;  // dynamic shared memory one block of sm_100 may opt in to
+constexpr size_t kGuard = 8 * 1024;      // checked after every block: catches writes past the kernel's plan
 
 struct Warp {
   alignas(16) unsigned char slot[2][32][16];
@@ -108,6 +110,10 @@ void block_barrier() {
 }
 
 void launch(long long grid, int block, size_t smem_bytes, const std::function<void()>& body) {
+  if (smem_bytes > kMaxSmem) {
+    std::fprintf(stderr, "pmemu: launch with %zu bytes of dynamic shared memory, more than one block can use\n", smem_bytes);
+    std::abort();
+  }
   if (block % 32 != 0) {
     std::fprintf(stderr, "pmemu: block size must be a multiple of 32\n");
     std::abort();
@@ -123,11 +129,19 @@ void launch(long long grid, int block, size_t smem_bytes, const std::function<vo
     blk.fibers.resize(block);
     blk.warps.resize(block / 32);
     for (auto& f : blk.fibers) f.stack = (char*)std::malloc(kStack);
-    std::vector<char> smem(smem_bytes + 16);
+    // The device does not clear shared memory: NaN bytes make a read of a value nobody wrote show in the results.
+    std::vector<unsigned char> smem(smem_bytes + kGuard);
     for (;;) {
       long long bid = next.fetch_add(1);
       if (bid >= grid) break;
-      run_block(blk, bid, grid, block, smem.data(), body);
+      std::memset(smem.data(), 0xFF, smem.size());
+      run_block(blk, bid, grid, block, reinterpret_cast<char*>(smem.data()), body);
+      for (size_t i = smem_bytes; i < smem.size(); ++i)
+        if (smem[i] != 0xFF) {
+          std::fprintf(stderr, "pmemu: block %lld wrote shared memory byte %zu, past the %zu bytes launched with\n", bid,
+                       i, smem_bytes);
+          std::abort();
+        }
     }
     for (auto& f : blk.fibers) std::free(f.stack);
   };

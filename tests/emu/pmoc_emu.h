@@ -25,6 +25,8 @@ Ctx* cur();
 // lanes, returns a pointer to the 32 published slots (16-byte stride), valid until the next one.
 const unsigned char* exchange(const void* val, int bytes);
 void block_barrier();
+// Aborts when smem_bytes exceeds what one block of the device may use: the device would refuse that launch, so the
+// library must have refused it before.
 void launch(long long grid, int block, size_t smem_bytes, const std::function<void()>& body);
 
 }  // namespace pmemu

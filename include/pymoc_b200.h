@@ -27,7 +27,9 @@ extern "C" {
 
 #define PMOC_ABI_VERSION 3
 #define PMOC_MAX_NZ_WARP 256 /* one warp per member up to this many levels */
-#define PMOC_MAX_NZ_WIDE 4096 /* one CTA per member up to this many levels ('jn' topology only) */
+#define PMOC_MAX_NZ_WIDE 4096 /* one CTA per member up to this many levels: the 'jn' topology and the explicit
+                                 'post' topologies (HAS_TW, HAS_SO, HAS_TW|HAS_SO, HAS_NORTH|HAS_TW|ISO and
+                                 HAS_NORTH|HAS_TW|ISO|HAS_SO without so_c or so_tau_on_y) */
 #define PMOC_MAX_NY_ML 64    /* SO_ML surface points per member */
 
 typedef enum {
@@ -163,8 +165,9 @@ typedef struct {
   double *Psi_so2, *Psi_Ek2, *Psi_GM2;     /* [M, nz] Sv: Psi_SO of the pac sector */
   uint32_t* status;                       /* [M] PMOC_ST_* bits, OR-ed */
 
-  /* device scratch, needed only when nz > PMOC_MAX_NZ_WARP: pmoc_model_scratch_bytes(m) bytes.
-     The library never allocates device memory itself (except in pmoc_model_run_host). */
+  /* device scratch, needed only when nz > PMOC_MAX_NZ_WARP (block-per-member kernels of both orders):
+     pmoc_model_scratch_bytes(m) bytes.  The library never allocates device memory itself (except in
+     pmoc_model_run_host). */
   void* scratch;
   uint64_t scratch_bytes;
 } pmoc_model;
@@ -181,8 +184,12 @@ uint64_t pmoc_model_scratch_bytes(const pmoc_model* m); /* 0 when nz <= PMOC_MAX
 int pmoc_model_diagnose(const pmoc_model* m, void* stream);
 
 /* Advance every member by `nsteps` iterations of the script loop, iteration counter starting
- * at `it0` (streamfunctions are re-diagnosed on iterations with it % K == 0).  One fused
- * kernel: state stays on-chip for all `nsteps`.  Replaces the loop bodies
+ * at `it0` (streamfunctions are re-diagnosed on iterations with it % K == 0).  Up to
+ * PMOC_MAX_NZ_WARP levels one fused kernel: state stays on-chip for all `nsteps`.  Above that (up to
+ * PMOC_MAX_NZ_WIDE, the topologies listed there) one CTA per member: step launches alternate with
+ * diagnosis launches, the state stays on chip between two diagnoses.  Other topologies above
+ * PMOC_MAX_NZ_WARP (the F2010 smoother, tau on y, the two-basin model) return PMOC_EUNSUPPORTED.
+ * Replaces the loop bodies
  * examples/example_timestepping.py:73-80, example_twocol.py:85-96,
  * example_twocol_plusSO.py:99-115, run_JansenNadeau_2018.py:201-261,
  * run_single_global_basin.py:172-229. */

@@ -1,13 +1,16 @@
-// Block-per-member kernels for columns too tall for one warp (256 < nz <= 4096): the 'jn'
-// topology of examples/run_single_global_basin.py / run_JansenNadeau_2018.py (two convecting
-// columns, thermal wind with isopycnal remap, explicit Psi_SO, SO_ML).
+// Block-per-member kernels for columns too tall for one warp (256 < nz <= 4096).  Two loop orders:
+//  - 'jn' (examples/run_single_global_basin.py / run_JansenNadeau_2018.py): two convecting columns, thermal wind
+//    with isopycnal remap, explicit Psi_SO, SO_ML; stepped by k_wide_steps2.
+//  - 'post' (example_timestepping.py, example_twocol.py, example_twocol_plusSO.py with the explicit GM closure):
+//    one column with thermal wind against a fixed profile and/or Psi_SO, or two columns with the isopycnal remap
+//    and optionally Psi_SO; stepped by k_wide_post.
 //
-// One CTA owns one member.  k_wide_steps2 keeps both buoyancy profiles and the geometry of the
-// thread's levels in registers and -weff / kappa in shared memory for all the steps of a launch (see
-// the comment on the kernel); the arithmetic is the bit-faithful step of pm::col_step_exact, level
-// by level.  At the stable time step of such grids the streamfunctions are re-diagnosed once in tens
-// of thousands of steps (K = 72 000 at nz = 4096), so the diagnosis is a separate, plain kernel
-// (k_wide_refresh) and the host loop in pmoc_run_model_wide alternates the two.
+// One CTA owns one member.  The step kernels keep the buoyancy profiles and the geometry of the thread's levels in
+// registers and -weff / kappa in shared memory for all the steps of a launch (see the comments on the kernels); the
+// arithmetic is the bit-faithful step of pm::col_step_exact, level by level.  At the stable time step of such grids
+// the streamfunctions are re-diagnosed once in hundreds to tens of thousands of steps (K = 72 000 at nz = 4096 in
+// the 'jn' model), so the diagnosis is a separate, plain kernel (k_wide_refresh, shared by both orders) and the host
+// loop in pmoc_run_model_wide alternates the two.
 #include "pmoc_common.cuh"
 
 #include <cstdlib>
@@ -106,12 +109,16 @@ PM_GLOBAL void k_wide_geo(WideArgs a) {
 }
 
 // ---- diagnosis of the streamfunctions -----------------------------------------------------------
-// Psi_Thermwind.solve + Psibz + Psi_SO.solve for one member per CTA, results to global memory
+// Psi_Thermwind.solve (+ Psibz) + Psi_SO.solve for one member per CTA, results to global memory
 // (same expressions as pm::tw_solve / tw_psib / interp_bgrid / so_solve, level loops instead of
-// register chunks).
+// register chunks).  The parts follow the model's flags: the thermal wind against the northern column
+// or the fixed profile tw_b2, the remap only with PMOC_ISO, Psi_SO on the mixed layer's bs ('jn') or on
+// so_bs ('post').  The rounding-noise bookkeeping of the 'jn' switches (PMOC_ST_CARRY_*) is 'jn' only.
 PM_GLOBAL void k_wide_refresh(WideArgs a) {
   const pmoc_model& M = a.m;
-  const int nz = M.nz, ny = M.ny, nb = M.nb, T = wnthr(), t = wtid();
+  const bool JN = (M.flags & PMOC_ORDER_JN) != 0, NORTH = (M.flags & PMOC_HAS_NORTH) != 0;
+  const bool TW = (M.flags & PMOC_HAS_TW) != 0, ISO = (M.flags & PMOC_ISO) != 0, SO = (M.flags & PMOC_HAS_SO) != 0;
+  const int nz = M.nz, ny = SO ? M.ny : 0, nb = ISO ? M.nb : 0, T = wnthr(), t = wtid();
   const long long m = rt::block_idx();
   double* sm = rt::smem();
   // six level arrays: the two profiles and four work arrays
@@ -127,225 +134,237 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
   const double* z = M.z;
   unsigned status = 0;
 
+  const double* b2src = NORTH ? M.north.b + m * nz : (TW ? vrow(M.tw_b2, m) : nullptr);
   for (int i = t; i < nz; i += T) {
     b1[i] = M.basin.b[m * nz + i];
-    b2[i] = M.north.b[m * nz + i];
+    b2[i] = b2src ? b2src[i] : 0.0;
   }
+  const double* bsrc = JN ? M.ml_bs + m * ny : (SO ? vrow(M.so_bs, m) : nullptr);
   for (int i = t; i < nyp; i += T) {
     ysm[i] = M.y[i < ny ? i : ny - 1];
-    bs_s[i] = M.ml_bs[m * ny + (i < ny ? i : ny - 1)];
+    bs_s[i] = bsrc[i < ny ? i : ny - 1];
   }
   rt::syncblock();
 
-  // --- thermal wind: Psi'' = (b2-b1)/f (psi_thermwind.py:123-135), see pm::tw_solve.  A = T (Simpson
-  // increments of Psi'), B = their exclusive prefix, C = cell integrals -> exclusive prefix, P = Psi (Sv)
-  const double rf = 1. / vat(M.tw_f, m);
-  for (int i = t; i < nz; i += T) {
-    double tt = 0.0;
-    if (i < nz - 1) {
-      const double gi = rf * (b2[i] - b1[i]), gi1 = rf * (b2[i + 1] - b1[i + 1]);
-      const double h = z[i + 1] - z[i], gm = 0.5 * (gi + gi1);
-      tt = h / 6. * (gi + 4. * gm + gi1);
-    }
-    A[i] = tt;
-    B[i] = tt;
-  }
-  rt::syncblock();
-  block_scan_excl(B, nz, red + 64, false);
-  for (int i = t; i < nz; i += T) {
-    double cell = 0.0;
-    if (i < nz - 1) {
-      const double gi = rf * (b2[i] - b1[i]), gi1 = rf * (b2[i + 1] - b1[i + 1]);
-      const double h = z[i + 1] - z[i];
-      cell = h * B[i] + h * A[i] / 2. - h * h / 12. * (gi1 - gi);
-    }
-    C[i] = cell;
-  }
-  rt::syncblock();
-  block_scan_excl(C, nz, red + 64, false);
-  {
-    const double total = C[nz - 1], z0 = z[0], H = z[nz - 1] - z[0];
-    for (int i = t; i < nz; i += T) {
-      const double v = pm::div_const(C[i] - total * ((z[i] - z0) / H), pm::kSv, 1.0 / pm::kSv);
-      P[i] = v;
-      M.Psi_tw[m * nz + i] = v;
-    }
-  }
-  rt::syncblock();
-
-  // --- isopycnal remap (psi_thermwind.py:170-208), see pm::tw_psib
-  double lo = INFINITY, hi = -INFINITY;
-  bool unsorted = false;
-  for (int i = t; i < nz; i += T) {
-    lo = b1[i] < lo ? b1[i] : lo;
-    lo = b2[i] < lo ? b2[i] : lo;
-    hi = b1[i] > hi ? b1[i] : hi;
-    hi = b2[i] > hi ? b2[i] : hi;
-    if (i < nz - 1) {
-      const double u = -(P[i + 1] - P[i]);
-      unsorted |= !(b1[i + 1] >= b1[i]) || !(b2[i + 1] >= b2[i]) || u != u;
-      if (u < 0 ? pm::remap_tie(b2[i], b2[i + 1], u, i == 0) : pm::remap_tie(b1[i], b1[i + 1], u, i == 0)) status |= PMOC_ST_TIE_CELL;
-    }
-  }
-  lo = rt::wmin(lo);
-  hi = rt::wmax(hi);
-  if (rt::lane() == 0) {
-    red[rt::warp_in_block()] = lo;
-    red[32 + rt::warp_in_block()] = hi;
-  }
-  rt::syncblock();
-  for (int w = 0; w < rt::warps_per_block(); ++w) {
-    const double l = red[w], h2 = red[32 + w];
-    lo = (l < lo || lo != lo) ? l : lo;
-    hi = (h2 > hi || hi != hi) ? h2 : hi;
-  }
-  rt::syncblock();
-  pm::BGrid G;
-  G.lo = lo;
-  G.hi = hi;
-  G.nb = nb;
-  G.step = (hi - lo) / (double)(nb - 1);
-  G.rstep = 1.0 / G.step;
-  const bool direct = block_any(unsorted, ibox);
-  // transport of cell c and the column it is taken from
-  auto cell_u = [&](int c) { return -(P[c + 1] - P[c]); };
-  if (!direct) {
-    // A = S_1, B = S_2: S_X[k] = sum_{c >= k} [cell c uses X] u_c  (exclusive suffix + own)
-    for (int i = t; i < nz; i += T) {
-      const double u = i < nz - 1 ? cell_u(i) : 0.0;
-      A[i] = u < 0 ? 0.0 : u;
-      B[i] = u < 0 ? u : 0.0;
-    }
-    rt::syncblock();
-    block_scan_excl(A, nz, red + 64, true);
-    block_scan_excl(B, nz, red + 64, true);
-    for (int i = t; i < nz; i += T) {
-      const double u = i < nz - 1 ? cell_u(i) : 0.0;
-      A[i] = A[i] + (u < 0 ? 0.0 : u);
-      B[i] = B[i] + (u < 0 ? u : 0.0);
-    }
-    for (int i = t; i <= nb; i += T) cnt[i] = 0;
-    rt::syncblock();
-    for (int i = t; i < nz; i += T) {
-      rt::atomic_add_shared(&cnt[pm::bgrid_count_le(G, b1[i])], 1);
-      rt::atomic_add_shared(&cnt[pm::bgrid_count_le(G, b2[i])], 1 << 16);
-    }
-    rt::syncblock();
-    if (t == 0) {  // inclusive prefix over the classes (nb is a few hundred)
-      int run = 0;
-      for (int i = 0; i <= nb; ++i) {
-        run += cnt[i];
-        cnt[i] = run;
-      }
-    }
-    rt::syncblock();
-    for (int i = t; i < nb; i += T) {
-      const double x = G.at(i);
-      const int k1 = cnt[i] & 0xffff, k2 = cnt[i] >> 16;  // #{levels with bX < x}
-      double c1 = 0.0, c2 = 0.0;
-      if (k1 < nz) {
-        const double bk = b1[k1];
-        c1 = A[k1];
-        if (k1 > 0 && bk != x) {
-          const double u = cell_u(k1 - 1);
-          c1 = c1 + (bk - x) * (u < 0 ? 0.0 : u / (bk - b1[k1 - 1]));
-        }
-        if (bk == x)  // flat cells taken from column 1 sitting exactly on the class: 0/0 in the reference
-          for (int c = k1; c + 1 < nz && b1[c + 1] == x; ++c)
-            if (!(cell_u(c) < 0)) c1 = NAN;
-      }
-      if (k2 < nz) {
-        const double bk = b2[k2];
-        c2 = B[k2];
-        if (k2 > 0 && bk != x) {
-          const double u = cell_u(k2 - 1);
-          c2 = c2 + (bk - x) * (u < 0 ? u / (bk - b2[k2 - 1]) : 0.0);
-        }
-        if (bk == x)
-          for (int c = k2; c + 1 < nz && b2[c + 1] == x; ++c)
-            if (cell_u(c) < 0) c2 = NAN;
-      }
-      psib_s[i] = c1 + c2;
-    }
-  } else {
-    // direct path: every class against every cell (inverted cells / NaN)
-    for (int i = t; i < nb; i += T) {
-      const double bg = G.at(i);
-      double acc = 0.0;
-      for (int c = 0; c < nz - 1; ++c) {
-        const double u = cell_u(c);
-        const bool from2 = u < 0;
-        const double bot = from2 ? b2[c] : b1[c], top = from2 ? b2[c + 1] : b1[c + 1];
-        double f = (top - bg) * (1.0 / (top - bot));
-        f = f < 0. ? 0. : f;
-        f = f > 1. ? 1. : f;
-        acc = rt::fma(f, u, acc);
-      }
-      psib_s[i] = acc;
-    }
-  }
-  rt::syncblock();
-  for (int i = t; i < nb; i += T) {
-    if (M.psib) M.psib[m * nb + i] = psib_s[i];
-    if (M.bgrid) M.bgrid[m * nb + i] = G.at(i);
-  }
-  // what the 'jn' switches of the step kernel read (level 1 of the three streamfunctions), and the scale
-  // against which they count as rounding noise (PMOC_ST_NOISE_SWITCH)
-  double mxl = 0.0, so1 = 0.0, resb1 = 0.0, resn1 = 0.0;
+  double mxl = 0.0, so1 = 0.0, resb1 = 0.0, resn1 = 0.0;  // ('jn' only, see the end)
   bool exact1 = false;
-  for (int i = t; i < nz; i += T) {
-    const double vb = pm::interp_bgrid(b1[i], G, psib_s), vn = pm::interp_bgrid(b2[i], G, psib_s);
-    M.Psi_iso_b[m * nz + i] = vb;
-    M.Psi_iso_n[m * nz + i] = vn;
-    mxl = fabs(vb) > mxl ? fabs(vb) : mxl;
-    mxl = fabs(vn) > mxl ? fabs(vn) : mxl;
-    if (i == 1) { resb1 = vb; resn1 = vn; }
+  if (TW) {
+    // --- thermal wind: Psi'' = (b2-b1)/f (psi_thermwind.py:123-135), see pm::tw_solve.  A = T (Simpson
+    // increments of Psi'), B = their exclusive prefix, C = cell integrals -> exclusive prefix, P = Psi (Sv)
+    const double rf = 1. / vat(M.tw_f, m);
+    for (int i = t; i < nz; i += T) {
+      double tt = 0.0;
+      if (i < nz - 1) {
+        const double gi = rf * (b2[i] - b1[i]), gi1 = rf * (b2[i + 1] - b1[i + 1]);
+        const double h = z[i + 1] - z[i], gm = 0.5 * (gi + gi1);
+        tt = h / 6. * (gi + 4. * gm + gi1);
+      }
+      A[i] = tt;
+      B[i] = tt;
+    }
+    rt::syncblock();
+    block_scan_excl(B, nz, red + 64, false);
+    for (int i = t; i < nz; i += T) {
+      double cell = 0.0;
+      if (i < nz - 1) {
+        const double gi = rf * (b2[i] - b1[i]), gi1 = rf * (b2[i + 1] - b1[i + 1]);
+        const double h = z[i + 1] - z[i];
+        cell = h * B[i] + h * A[i] / 2. - h * h / 12. * (gi1 - gi);
+      }
+      C[i] = cell;
+    }
+    rt::syncblock();
+    block_scan_excl(C, nz, red + 64, false);
+    {
+      const double total = C[nz - 1], z0 = z[0], H = z[nz - 1] - z[0];
+      for (int i = t; i < nz; i += T) {
+        const double v = pm::div_const(C[i] - total * ((z[i] - z0) / H), pm::kSv, 1.0 / pm::kSv);
+        P[i] = v;
+        if (M.Psi_tw) M.Psi_tw[m * nz + i] = v;
+      }
+    }
+    rt::syncblock();
   }
 
-  // --- Psi_SO.solve, explicit GM branch (psi_SO.py:106-140, 218-243, 302-354), see pm::so_solve
-  const pm::SoSurf S = pm::so_scan(ysm, bs_s, sinv, ny);  // every warp redundantly, same values
-  rt::syncblock();
-  if (!S.mono) status |= PMOC_ST_BS_NONMONOTONE;
-  if (S.ndown >= pm::kSawtoothSegments) status |= PMOC_ST_BS_SAWTOOTH;
-  const double tau_ave = pm::mean100(vat(M.so_tau, m));
-  const double sf = vat(M.so_f, m), srho = vat(M.so_rho, m), sL = vat(M.so_L, m), sK = vat(M.so_KGM, m),
-               smax = vat(M.so_smax, m);
-  const double pre = tau_ave / sf / srho * sL, c6 = 1e6, r6 = 1.0 / 1e6;
-  for (int i = t; i < nz; i += T) {
-    const double bi = b1[i];
-    double yo;
-    if (bi < S.mn)
-      yo = S.y0 - 1e3;
-    else if (bi > S.bsN)
-      yo = S.yN;
-    else if (S.mono && S.south < ny - 1)
-      yo = pm::outcrop_monotone(bi, ysm, bs_s, sinv, ny, S.south);
-    else {
-      bool bad = false;
-      yo = pm::outcrop_brent(bi, ysm, bs_s, ny, S.south, &bad);
-      if (bad) status |= PMOC_ST_BRENT_SIGN;
+  if (ISO) {
+    // --- isopycnal remap (psi_thermwind.py:170-208), see pm::tw_psib
+    double lo = INFINITY, hi = -INFINITY;
+    bool unsorted = false;
+    for (int i = t; i < nz; i += T) {
+      lo = b1[i] < lo ? b1[i] : lo;
+      lo = b2[i] < lo ? b2[i] : lo;
+      hi = b1[i] > hi ? b1[i] : hi;
+      hi = b2[i] > hi ? b2[i] : hi;
+      if (i < nz - 1) {
+        const double u = -(P[i + 1] - P[i]);
+        unsorted |= !(b1[i + 1] >= b1[i]) || !(b2[i + 1] >= b2[i]) || u != u;
+        if (u < 0 ? pm::remap_tie(b2[i], b2[i + 1], u, i == 0) : pm::remap_tie(b1[i], b1[i + 1], u, i == 0)) status |= PMOC_ST_TIE_CELL;
+      }
     }
-    const double e = pm::div_const(pre * M.so_sill_taper[i] * M.so_ek_taper[i], c6, r6);
-    double dy = S.yN - yo;
-    dy = 0.1 > dy ? 0.1 : dy;
-    const double sl = pm::qdiv(z[i], dy), ms = -smax;
-    const double mx = (sl >= ms || sl != sl) ? sl : ms;
-    double g = sK * mx * sL * M.so_top_taper[i] * M.so_bot_taper[i];
-    if (i == 1 && !(sl >= ms || sl != sl)) exact1 = true;  // the slope clip: constants only (see pm::so_solve)
-    if (dy > S.yN - S.y0) {
-      const double alt = -e * 1e6;
-      if (i == 1 && !(g >= alt || g != g)) exact1 = true;  // the limiter
-      g = (g >= alt || g != g) ? g : alt;
+    lo = rt::wmin(lo);
+    hi = rt::wmax(hi);
+    if (rt::lane() == 0) {
+      red[rt::warp_in_block()] = lo;
+      red[32 + rt::warp_in_block()] = hi;
     }
-    g = pm::div_const(g, c6, r6);
-    const double v = i == 0 ? 0. : e + g;
-    M.Psi_so[m * nz + i] = v;
-    mxl = fabs(v) > mxl ? fabs(v) : mxl;
-    if (i == 1) so1 = v;
-    if (M.Psi_Ek) M.Psi_Ek[m * nz + i] = e;
-    if (M.Psi_GM) M.Psi_GM[m * nz + i] = g;
+    rt::syncblock();
+    for (int w = 0; w < rt::warps_per_block(); ++w) {
+      const double l = red[w], h2 = red[32 + w];
+      lo = (l < lo || lo != lo) ? l : lo;
+      hi = (h2 > hi || hi != hi) ? h2 : hi;
+    }
+    rt::syncblock();
+    pm::BGrid G;
+    G.lo = lo;
+    G.hi = hi;
+    G.nb = nb;
+    G.step = (hi - lo) / (double)(nb - 1);
+    G.rstep = 1.0 / G.step;
+    const bool direct = block_any(unsorted, ibox);
+    // transport of cell c and the column it is taken from
+    auto cell_u = [&](int c) { return -(P[c + 1] - P[c]); };
+    if (!direct) {
+      // A = S_1, B = S_2: S_X[k] = sum_{c >= k} [cell c uses X] u_c  (exclusive suffix + own)
+      for (int i = t; i < nz; i += T) {
+        const double u = i < nz - 1 ? cell_u(i) : 0.0;
+        A[i] = u < 0 ? 0.0 : u;
+        B[i] = u < 0 ? u : 0.0;
+      }
+      rt::syncblock();
+      block_scan_excl(A, nz, red + 64, true);
+      block_scan_excl(B, nz, red + 64, true);
+      for (int i = t; i < nz; i += T) {
+        const double u = i < nz - 1 ? cell_u(i) : 0.0;
+        A[i] = A[i] + (u < 0 ? 0.0 : u);
+        B[i] = B[i] + (u < 0 ? u : 0.0);
+      }
+      for (int i = t; i <= nb; i += T) cnt[i] = 0;
+      rt::syncblock();
+      for (int i = t; i < nz; i += T) {
+        rt::atomic_add_shared(&cnt[pm::bgrid_count_le(G, b1[i])], 1);
+        rt::atomic_add_shared(&cnt[pm::bgrid_count_le(G, b2[i])], 1 << 16);
+      }
+      rt::syncblock();
+      if (t == 0) {  // inclusive prefix over the classes (nb is a few hundred)
+        int run = 0;
+        for (int i = 0; i <= nb; ++i) {
+          run += cnt[i];
+          cnt[i] = run;
+        }
+      }
+      rt::syncblock();
+      for (int i = t; i < nb; i += T) {
+        const double x = G.at(i);
+        const int k1 = cnt[i] & 0xffff, k2 = cnt[i] >> 16;  // #{levels with bX < x}
+        double c1 = 0.0, c2 = 0.0;
+        if (k1 < nz) {
+          const double bk = b1[k1];
+          c1 = A[k1];
+          if (k1 > 0 && bk != x) {
+            const double u = cell_u(k1 - 1);
+            c1 = c1 + (bk - x) * (u < 0 ? 0.0 : u / (bk - b1[k1 - 1]));
+          }
+          if (bk == x)  // flat cells taken from column 1 sitting exactly on the class: 0/0 in the reference
+            for (int c = k1; c + 1 < nz && b1[c + 1] == x; ++c)
+              if (!(cell_u(c) < 0)) c1 = NAN;
+        }
+        if (k2 < nz) {
+          const double bk = b2[k2];
+          c2 = B[k2];
+          if (k2 > 0 && bk != x) {
+            const double u = cell_u(k2 - 1);
+            c2 = c2 + (bk - x) * (u < 0 ? u / (bk - b2[k2 - 1]) : 0.0);
+          }
+          if (bk == x)
+            for (int c = k2; c + 1 < nz && b2[c + 1] == x; ++c)
+              if (cell_u(c) < 0) c2 = NAN;
+        }
+        psib_s[i] = c1 + c2;
+      }
+    } else {
+      // direct path: every class against every cell (inverted cells / NaN)
+      for (int i = t; i < nb; i += T) {
+        const double bg = G.at(i);
+        double acc = 0.0;
+        for (int c = 0; c < nz - 1; ++c) {
+          const double u = cell_u(c);
+          const bool from2 = u < 0;
+          const double bot = from2 ? b2[c] : b1[c], top = from2 ? b2[c + 1] : b1[c + 1];
+          double f = (top - bg) * (1.0 / (top - bot));
+          f = f < 0. ? 0. : f;
+          f = f > 1. ? 1. : f;
+          acc = rt::fma(f, u, acc);
+        }
+        psib_s[i] = acc;
+      }
+    }
+    rt::syncblock();
+    for (int i = t; i < nb; i += T) {
+      if (M.psib) M.psib[m * nb + i] = psib_s[i];
+      if (M.bgrid) M.bgrid[m * nb + i] = G.at(i);
+    }
+    // what the 'jn' switches of the step kernel read (level 1 of the three streamfunctions), and the scale
+    // against which they count as rounding noise (PMOC_ST_NOISE_SWITCH)
+    for (int i = t; i < nz; i += T) {
+      const double vb = pm::interp_bgrid(b1[i], G, psib_s), vn = pm::interp_bgrid(b2[i], G, psib_s);
+      M.Psi_iso_b[m * nz + i] = vb;
+      M.Psi_iso_n[m * nz + i] = vn;
+      mxl = fabs(vb) > mxl ? fabs(vb) : mxl;
+      mxl = fabs(vn) > mxl ? fabs(vn) : mxl;
+      if (i == 1) { resb1 = vb; resn1 = vn; }
+    }
+  }
+
+  if (SO) {
+    // --- Psi_SO.solve, explicit GM branch (psi_SO.py:106-140, 218-243, 302-354), see pm::so_solve
+    const pm::SoSurf S = pm::so_scan(ysm, bs_s, sinv, ny);  // every warp redundantly, same values
+    rt::syncblock();
+    if (!S.mono) status |= PMOC_ST_BS_NONMONOTONE;
+    if (S.ndown >= pm::kSawtoothSegments) status |= PMOC_ST_BS_SAWTOOTH;
+    const double tau_ave = pm::mean100(vat(M.so_tau, m));
+    const double sf = vat(M.so_f, m), srho = vat(M.so_rho, m), sL = vat(M.so_L, m), sK = vat(M.so_KGM, m),
+                 smax = vat(M.so_smax, m);
+    const double pre = tau_ave / sf / srho * sL, c6 = 1e6, r6 = 1.0 / 1e6;
+    for (int i = t; i < nz; i += T) {
+      const double bi = b1[i];
+      double yo;
+      if (bi < S.mn)
+        yo = S.y0 - 1e3;
+      else if (bi > S.bsN)
+        yo = S.yN;
+      else if (S.mono && S.south < ny - 1)
+        yo = pm::outcrop_monotone(bi, ysm, bs_s, sinv, ny, S.south);
+      else {
+        bool bad = false;
+        yo = pm::outcrop_brent(bi, ysm, bs_s, ny, S.south, &bad);
+        if (bad) status |= PMOC_ST_BRENT_SIGN;
+      }
+      const double e = pm::div_const(pre * M.so_sill_taper[i] * M.so_ek_taper[i], c6, r6);
+      double dy = S.yN - yo;
+      dy = 0.1 > dy ? 0.1 : dy;
+      const double sl = pm::qdiv(z[i], dy), ms = -smax;
+      const double mx = (sl >= ms || sl != sl) ? sl : ms;
+      double g = sK * mx * sL * M.so_top_taper[i] * M.so_bot_taper[i];
+      if (i == 1 && !(sl >= ms || sl != sl)) exact1 = true;  // the slope clip: constants only (see pm::so_solve)
+      if (dy > S.yN - S.y0) {
+        const double alt = -e * 1e6;
+        if (i == 1 && !(g >= alt || g != g)) exact1 = true;  // the limiter
+        g = (g >= alt || g != g) ? g : alt;
+      }
+      g = pm::div_const(g, c6, r6);
+      const double v = i == 0 ? 0. : e + g;
+      M.Psi_so[m * nz + i] = v;
+      mxl = fabs(v) > mxl ? fabs(v) : mxl;
+      if (i == 1) so1 = v;
+      if (M.Psi_Ek) M.Psi_Ek[m * nz + i] = e;
+      if (M.Psi_GM) M.Psi_GM[m * nz + i] = g;
+    }
   }
   const unsigned all = block_or(status, ibox);
+  if (!JN) {
+    if (t == 0 && M.status) M.status[m] = (M.status[m] | all) & ~PMOC_ST_CARRY_MASK;
+    return;
+  }
   mxl = rt::wmax(mxl);
   rt::syncblock();
   if (rt::lane() == 0) red[rt::warp_in_block()] = mxl;
@@ -938,9 +957,220 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
   if (t == 0 && M.status) M.status[m] |= all;
 }
 
+// ---- the steps of the 'post' order (example_twocol_plusSO.py:99-115) ----------------------------
+// NCOL columns (the basin; and the northern column of the two-column models), each advanced by
+// Column.timestep(wA, dt, do_conv) with the streamfunctions of the last diagnosis, which the host loop
+// re-runs in a launch of its own after every iteration with it % K == 0.  Layout as in k_wide_steps2: 256
+// threads own LPT consecutive levels of every column, whose buoyancies, dz, 1/dz and 1/dzc stay in
+// registers for the whole launch; -weff and kappa live in shared memory in owner-major order (slot
+// j*256 + t).  wA is assembled from the carried streamfunctions at launch exactly as k_model's apply():
+// basin (Psi_iso_b or Psi_tw) - Psi_so, north -Psi_iso_n, times 1e6.  The kappa variant is fixed in this
+// order.  Per step, every thread publishes its first and last level of each column and the convection
+// flags (anything above bs, highest stable level); the edges are double-buffered and the flags triple-
+// buffered (read / written / cleared), so a step costs one barrier.  The arithmetic is that of
+// pm::col_step_exact, as in the 'jn' kernel.  At LPT = 4 the kernel is compiled for two CTAs per SM (at most 128
+// registers; it needs about 125 without spilling, against 150 / 194 left free), the wider ones for one.
+template <int LPT, int NCOL>
+PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol, LPT == 4 ? 2 : 1) k_wide_post(WideArgs a) {
+  const pmoc_model& M = a.m;
+  const bool TW = (M.flags & PMOC_HAS_TW) != 0, ISO = (M.flags & PMOC_ISO) != 0, SO = (M.flags & PMOC_HAS_SO) != 0;
+  const int nz = M.nz, t = wtid(), Ln = rt::lane();
+  const long long m = rt::block_idx();
+  const double dt = M.dt;
+  constexpr int nzp = kWideCol * LPT;
+  double* sm = rt::smem();
+  double* nws = sm;                                  // [NCOL][nzp] -weff
+  double* kps = sm + NCOL * nzp;                     // [NCOL][nzp] kappa
+  double* edge = sm + 2 * NCOL * nzp;                // [2][NCOL][2 * kWideCol] first / last level of every thread
+  int* flg = reinterpret_cast<int*>(edge + 4 * NCOL * kWideCol);  // [3][NCOL][2] any level above bs, top stable level
+  int* cbox = flg + 6 * NCOL;                        // the block collectives
+  const double* z = M.z;
+  const int lo = t * LPT;
+  double* rarea = a.memb + (size_t)m * 6 * nz;       // [NCOL][nz] 1 / Area (non-uniform Area)
+
+  const pmoc_column* col[2] = {&M.basin, &M.north};
+  double bs[NCOL], n2[NCOL], bbot[NCOL], bzbot[NCOL], A1[NCOL], rA1[NCOL];
+  bool conv[NCOL], hasz[NCOL];
+  const double* Ar[NCOL];
+  double b[NCOL][LPT], dzu[LPT], rdzu[LPT], rdzc[LPT];
+  double dzu_m = 1., rdzu_m = 1.;  // cell below the thread's first level
+  bool areas_differ = false;
+  PM_UNROLL
+  for (int c = 0; c < NCOL; ++c) {
+    const pmoc_column& d = *col[c];
+    bs[c] = vat(d.bs, m);
+    n2[c] = vat(d.N2min, m);
+    bbot[c] = d.bbot[m];
+    hasz[c] = d.bzbot.ptr != nullptr;
+    bzbot[c] = hasz[c] ? vat(d.bzbot, m) : 0.0;
+    conv[c] = d.do_conv != 0;
+    Ar[c] = vrow(d.Area, m);
+    A1[c] = Ar[c][1];
+    rA1[c] = 1.0 / A1[c];
+    const int var = (d.var && d.nvar > 1) ? d.var[m] : 0;
+    const double* kap = vrow(d.kappa, m) + (size_t)var * nz;
+    const double* dak = vrow(d.dAk, m) + (size_t)var * nz;
+    const double* lega = c == 0 ? (TW ? (ISO ? M.Psi_iso_b : M.Psi_tw) + m * nz : nullptr) : M.Psi_iso_n + m * nz;
+    const double* psos = (c == 0 && SO) ? M.Psi_so + m * nz : nullptr;
+    PM_UNROLL
+    for (int j = 0; j < LPT; ++j) {
+      const int i = lo + j, s = j * kWideCol + t;
+      b[c][j] = 0.;
+      nws[c * nzp + s] = kps[c * nzp + s] = 0.0;  // boundary and padding levels: zero -weff and kappa, an exact no-op
+      if (i < nz) {
+        b[c][j] = d.b[m * nz + i];
+        const bool in = i >= 1 && i < nz - 1;
+        // k_model's apply (pmoc_model.cu): the same expressions, so the same wA bits
+        const double wA = c == 0 ? ((lega ? lega[i] : 0.0) - (psos ? psos[i] : 0.0)) * 1e6 : -lega[i] * 1e6;
+        if (in) {
+          nws[c * nzp + s] = -(wA - dak[i]);
+          kps[c * nzp + s] = kap[i];
+          areas_differ |= Ar[c][i] != A1[c];
+        }
+        rarea[c * nz + i] = 1.0 / Ar[c][i];
+      }
+    }
+  }
+  PM_UNROLL
+  for (int j = 0; j < LPT; ++j) {
+    const int i = lo + j;
+    dzu[j] = rdzu[j] = rdzc[j] = 1.;
+    if (i < nz) {
+      dzu[j] = a.geo[i];
+      rdzu[j] = a.geo[nz + i];
+      rdzc[j] = a.geo[3 * nz + i];
+    }
+  }
+  if (lo >= 1 && lo - 1 < nz) {
+    dzu_m = a.geo[lo - 1];
+    rdzu_m = a.geo[nz + lo - 1];
+  }
+  if (t < 3 * NCOL) {  // every flag buffer starts empty
+    flg[2 * t] = 0;
+    flg[2 * t + 1] = -1;
+  }
+  const bool uniA = !block_any(areas_differ, cbox);  // (its barriers also order the flag reset before the publish)
+
+  // publish the first / last level of every column and the convection flags of this thread's levels
+  bool mine[NCOL];  // the thread's own levels hold something above bs
+  PM_UNROLL
+  for (int c = 0; c < NCOL; ++c) mine[c] = false;
+  const bool owns_top = lo <= nz - 1 && nz - 1 < lo + LPT;
+  auto publish = [&](int e, int q) {
+    PM_UNROLL
+    for (int c = 0; c < NCOL; ++c) {
+      double* ed = edge + (e * NCOL + c) * 2 * kWideCol;
+      ed[2 * t] = b[c][0];
+      ed[2 * t + 1] = b[c][LPT - 1];
+      if (!conv[c]) continue;
+      int top = -1;
+      bool any = false;
+      PM_UNROLL
+      for (int j = 0; j < LPT; ++j)
+        if (lo + j < nz) {
+          if (b[c][j] > bs[c]) any = true;
+          else top = lo + j;
+        }
+      mine[c] = any;
+      const unsigned ma = rt::ballot(any);
+      const int wt = rt::max_i(top);
+      if (Ln == 0) {
+        int* f = flg + (q * NCOL + c) * 2;
+        if (ma) rt::atomic_add_shared(&f[0], 1);
+        rt::atomic_max_shared(&f[1], wt);
+      }
+    }
+  };
+  publish(0, 0);
+  rt::syncblock();
+
+  int e = 0, qr = 0;
+  for (long long it = 0; it < a.nsteps; ++it) {
+    const int qw = qr == 2 ? 0 : qr + 1, qz = qw == 2 ? 0 : qw + 1;
+    PM_UNROLL
+    for (int c = 0; c < NCOL; ++c) {
+      // convective adjustment (column.py:264-271) or the surface value (column.py:230-231) of the own levels and
+      // of the two neighbour values, then the bottom condition (column.py:232-233)
+      const int* f = flg + (qr * NCOL + c) * 2;
+      const bool cv = conv[c] && f[0] != 0;
+      const double zc = z[f[1] >= 0 ? f[1] : 0], bsc = bs[c], n2c = n2[c];
+      auto adj = [&](double v, int i) {
+        if (cv) return v > bsc ? bsc + n2c * (z[i] - zc) : v;
+        return i == nz - 1 ? bsc : v;
+      };
+      if ((cv && mine[c]) || owns_top) {
+        PM_UNROLL
+        for (int j = 0; j < LPT; ++j)
+          if (lo + j < nz) b[c][j] = adj(b[c][j], lo + j);
+      }
+      if (t == 0) b[c][0] = hasz[c] ? b[c][1] - bzbot[c] * dzu[0] : bbot[c];
+      const double* ed = edge + (e * NCOL + c) * 2 * kWideCol;
+      double gp = 0.;  // gradient of the cell below the current level
+      if (lo >= 1 && lo < nz) gp = pm::div_const(b[c][0] - adj(ed[2 * t - 1], lo - 1), dzu_m, rdzu_m);
+      const double ub = lo + LPT < nz ? adj(ed[2 * t + 2], lo + LPT) : 0.;  // level above the thread's last one
+      // bit-faithful explicit step (column.py:235-249), see pm::col_step_exact.  No level tests: at the boundary
+      // and padding levels -weff = kappa = 0 and every operand is finite, so b + dt*0 = b.
+      const double* nw = nws + c * nzp;
+      const double* kp = kps + c * nzp;
+      auto step = [&](auto UA) {
+        constexpr bool ua = decltype(UA)::value;
+        PM_UNROLL
+        for (int j = 0; j < LPT; ++j) {
+          const int s = j * kWideCol + t;
+          const double up = j + 1 < LPT ? b[c][j + 1 < LPT ? j + 1 : j] : ub;
+          const double g = pm::div_const(up - b[c][j], dzu[j], rdzu[j]);
+          const double dzc = 0.5 * (dzu[j] + (j > 0 ? dzu[j > 0 ? j - 1 : 0] : dzu_m));
+          const double bzz = pm::div_const(g - gp, dzc, rdzc[j]);
+          const double nwv = nw[s], sel = nwv > 0 ? g : gp;
+          double Ai = A1[c], rAi = rA1[c];
+          if (!ua) {
+            const int i = lo + j < nz ? lo + j : nz - 1;
+            Ai = Ar[c][i];
+            rAi = rarea[c * nz + i];
+          }
+          const double adv = pm::div_const(nwv * sel, Ai, rAi);
+          b[c][j] = b[c][j] + dt * (adv + kp[s] * bzz);
+          gp = g;
+        }
+      };
+      if (uniA) step(std::true_type{});
+      else step(std::false_type{});
+    }
+    publish(e ^ 1, qw);
+    if (t == 0) {
+      PM_UNROLL
+      for (int c = 0; c < NCOL; ++c) {  // last read in the previous step, next written in the next one
+        flg[(qz * NCOL + c) * 2] = 0;
+        flg[(qz * NCOL + c) * 2 + 1] = -1;
+      }
+    }
+    rt::syncblock();
+    e ^= 1;
+    qr = qw;
+  }
+
+  bool nan = false;
+  PM_UNROLL
+  for (int c = 0; c < NCOL; ++c) {
+    PM_UNROLL
+    for (int j = 0; j < LPT; ++j) {
+      const int i = lo + j;
+      if (i < nz) {
+        col[c]->b[m * nz + i] = b[c][j];
+        nan |= !(fabs(b[c][j]) <= 1.79e308);
+      }
+    }
+  }
+  if (block_any(nan, cbox) && t == 0 && M.status) M.status[m] |= PMOC_ST_NAN;
+}
+
 size_t wide_steps2_smem(int lpt, int ny) {
   const int nyp = (ny + 3) & ~3, nzp = kWideCol * lpt;
   return sizeof(double) * (size_t)(6 * nzp + kWideCol + 2 * kWideCol + 2 + 2 * nyp + 320 + 8 + 10 + pm::kMlSave);
+}
+
+size_t wide_post_smem(int lpt, int ncol) {
+  return sizeof(double) * (size_t)(2 * ncol * kWideCol * lpt + 4 * ncol * kWideCol) + sizeof(int) * (size_t)(6 * ncol + 4);
 }
 
 size_t wide_refresh_smem(int nz, int ny, int nb) {
@@ -950,16 +1180,26 @@ size_t wide_refresh_smem(int nz, int ny, int nb) {
 
 }  // namespace pmk
 
-// Host loop: alternate the diagnosis (top of every iteration with it % K == 0) and step launches.
+// Host loop: alternate the diagnosis and step launches in the model's order.
+//   'jn'   (run_JansenNadeau_2018.py:201-261): the diagnosis at the top of every iteration with it % K == 0, then
+//          the steps up to the next such iteration.
+//   'post' (example_twocol_plusSO.py:99-115): the steps of iterations [ii, stop], stop the first multiple of K at
+//          or after ii, then the diagnosis when stop < it_end (k_model's next0 / hits rule, so that split launches
+//          reproduce one launch bit for bit).
 int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream) {
-  const unsigned need = PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO | PMOC_HAS_ML | PMOC_ORDER_JN;
-  if ((m->flags & need) != need || (m->flags & PMOC_SO_BVP) || m->so_c.ptr || m->so_tau_on_y)
-    return fail(PMOC_EUNSUPPORTED, "nz > 256: only the 'jn' topology (two columns + thermal wind + explicit Psi_SO + SO_ML) "
-                                   "has a block-per-member kernel");
+  const unsigned topo = m->flags & (PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO | PMOC_HAS_ML | PMOC_ORDER_JN);
+  const unsigned jn = PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO | PMOC_HAS_ML | PMOC_ORDER_JN;
+  const bool post = topo == PMOC_HAS_TW || topo == PMOC_HAS_SO || topo == (PMOC_HAS_TW | PMOC_HAS_SO) ||
+                    topo == (PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO) ||
+                    topo == (PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO);
+  if ((topo != jn && !post) || (m->flags & PMOC_SO_BVP) || m->so_c.ptr || m->so_tau_on_y)
+    return fail(PMOC_EUNSUPPORTED, "nz > 256: only the 'jn' topology and the explicit 'post' topologies (one column with "
+                                   "thermal wind and/or Psi_SO, two columns with or without Psi_SO) have block-per-member "
+                                   "kernels; the F2010 smoother and a wind stress on y do not");
   if (m->nz > PMOC_MAX_NZ_WIDE) return fail(PMOC_EUNSUPPORTED, "nz > 4096");
   if (!m->scratch || m->scratch_bytes < pmoc_model_scratch_bytes(m))
     return fail(PMOC_EINVAL, "nz > 256 needs pmoc_model.scratch of pmoc_model_scratch_bytes() bytes");
-  if (!m->Psi_tw || !m->Psi_iso_b || !m->Psi_iso_n || !m->Psi_so) return fail(PMOC_EINVAL, "diagnostic buffers missing");
+  if (!post && (!m->Psi_tw || !m->Psi_iso_b || !m->Psi_iso_n || !m->Psi_so)) return fail(PMOC_EINVAL, "diagnostic buffers missing");
   WideArgs a;
   a.m = *m;
   a.geo = static_cast<double*>(m->scratch);
@@ -968,11 +1208,35 @@ int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, in
   a.nsteps = 0;
   a.force_late = std::getenv("PMOC_WIDE_FORCE_LATE") != nullptr;
   const long long K = m->K, it_end = it0 + nsteps;
-  const size_t sm_r = wide_refresh_smem(m->nz, m->ny, m->nb);
-  if (sm_r > 227 * 1024) return fail(PMOC_EUNSUPPORTED, "nz too large for shared memory");
+  const int nb = (m->flags & PMOC_ISO) ? m->nb : 0, ny = (m->flags & PMOC_HAS_SO) ? m->ny : 0;
+  const size_t sm_r = wide_refresh_smem(m->nz, ny, nb);
+  if (sm_r > kMaxSmemPerBlock) {
+    std::snprintf(g_err, sizeof(g_err), "nz = %d, nb = %d, ny = %d: the diagnosis needs %zu bytes of shared memory per "
+                  "block, more than the %zu one block can use", m->nz, nb, ny, sm_r, kMaxSmemPerBlock);
+    return PMOC_EUNSUPPORTED;
+  }
   if (int rc = launch(k_wide_geo, 64, kWideThreads, 0, stream, a)) return rc;
   if (diagnose_only) return launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a);
   long long ii = it0;
+  if (post) {
+    const bool two = (m->flags & PMOC_HAS_NORTH) != 0;
+    const int lpt = m->nz <= 4 * kWideCol ? 4 : m->nz <= 8 * kWideCol ? 8 : 16;
+    auto kern = lpt == 4 ? (two ? k_wide_post<4, 2> : k_wide_post<4, 1>)
+              : lpt == 8 ? (two ? k_wide_post<8, 2> : k_wide_post<8, 1>)
+                         : (two ? k_wide_post<16, 2> : k_wide_post<16, 1>);
+    const size_t sm_s = wide_post_smem(lpt, two ? 2 : 1);
+    while (ii < it_end) {
+      const long long stop = ((ii + K - 1) / K) * K;  // first iteration with it % K == 0 at or after ii
+      const bool hits = stop < it_end;
+      a.it0 = ii;
+      a.nsteps = (hits ? stop + 1 : it_end) - ii;
+      if (int rc = launch(kern, m->M, kWideCol, sm_s, stream, a)) return rc;
+      ii += a.nsteps;
+      if (hits)
+        if (int rc = launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a)) return rc;
+    }
+    return PMOC_OK;
+  }
   while (ii < it_end) {
     if (ii % K == 0)
       if (int rc = launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a)) return rc;

@@ -53,7 +53,9 @@ typedef struct {
                                      lands on depends discontinuously on bs: rounding differences are amplified to
                                      O(1) (measured: every member of the C5 lattice that misses 1e-10 carries this
                                      bit), so parity is undefined */
-#define PMOC_ST_BRENT_SIGN 4u     /* f(a), f(b) same sign: scipy.optimize.brentq would raise ValueError */
+#define PMOC_ST_BRENT_SIGN 4u     /* f(a), f(b) same sign: scipy.optimize.brentq would raise ValueError.  Only a
+                                     non-finite bs(y) reaches it: b < min(bs) and b > bs[-1] are answered before the
+                                     root search, so a finite bs always brackets a sign change */
 #define PMOC_ST_XP_NONMONOTONE 8u /* b_basin not monotone as np.interp abscissa in SO_ML (SURVEY a15):
                                      numpy's guess-carrying search is followed query by query */
 #define PMOC_ST_BVP_SERIES 32u    /* F2010 smoother: a cell propagator series did not converge (N2 h^2/c^2 huge) */
@@ -71,20 +73,22 @@ typedef struct {
                                      bit of its state there (structural in the 'jn' loop, whose no-flux bottom
                                      condition bbot = b[1] drives b[0] - b[1] to zero); parity is undefined unless
                                      the roundings happen to agree */
-#define PMOC_ST_BS_SAWTOOTH 256u  /* (informational, implies BS_NONMONOTONE) bs(y) decreases on >= 3 segments north of
-                                     its minimum: the reference's mixed layer has gone grid-scale unstable
-                                     (SO_ML.py:124-134 explicit upwind advection + Crank-Nicolson with Ks dt/dy^2 > 1) */
+#define PMOC_ST_BS_SAWTOOTH 256u  /* (informational, implies BS_NONMONOTONE) bs(y) decreases on >= 3 grid intervals
+                                     north of its first minimum, counted one by one whether or not they are adjacent
+                                     (one smooth decrease across three intervals counts): typically the reference's
+                                     mixed layer has gone grid-scale unstable (SO_ML.py:124-134 explicit upwind
+                                     advection + Crank-Nicolson with Ks dt/dy^2 > 1) */
 /* Bits that make parity with the reference UNDEFINED for a member (the reference's own result is decided by
  * rounding noise); the others are informational (a rarer but exactly reproduced code path was taken). */
 #define PMOC_ST_PARITY_UNDEFINED (PMOC_ST_BS_NONMONOTONE | PMOC_ST_NOISE_SWITCH | PMOC_ST_TIE_CELL)
 /* internal, not sticky: the Psi_SO value of level 1 that the 'jn' switches read was produced by state-independent
  * arithmetic (the non-outcropping limiter or the slope clip) and is therefore reproduced bit for bit even when
- * it is rounding noise; carried between launches in the status word */
+ * it is rounding noise; carried between launches in the status word.  Streamfunctions pushed through
+ * pmoc_host_step (PMOC_IO_PSI) do not carry it: the step kernels classify them from their values alone.
+ * The stateless pmoc_model_run_host pushes the status word together with the streamfunctions it carries, so there
+ * the carry bit travels with them: the caller hands back both as an earlier call returned them. */
 #define PMOC_ST_CARRY_SO1_EXACT 0x80000000u
-/* internal, not sticky (block-per-member kernels): which of Psi_so[1], Psi_iso_b[1], Psi_iso_n[1] of the last
- * diagnosis are rounding noise (bits 28..30), handed from the diagnosis kernel to the step kernel */
-#define PMOC_ST_CARRY_NOISE_SHIFT 28
-#define PMOC_ST_CARRY_MASK 0xF0000000u
+#define PMOC_ST_CARRY_MASK 0xF0000000u /* bits reserved for such internal carries */
 
 /* ---- one advective-diffusive column: reference class Column, column.py:19-72 ------------ */
 typedef struct {

@@ -234,6 +234,10 @@ int launch(K kern, long long grid, int block, size_t smem, void* stream, const A
 
 
 static inline long long blocks_for(long long M) { return (M + kWarpsPerBlock - 1) / kWarpsPerBlock; }
+// Internal pmoc_model.flags bit, set by pmoc_host_step for a launch after the caller pushed the carried
+// streamfunctions (PMOC_IO_PSI): the 'jn' step kernels then classify them as rounding noise without the
+// PMOC_ST_CARRY_SO1_EXACT exemption of an earlier diagnosis, which does not describe them.
+constexpr unsigned kFlagPsiPushed = 0x80000000u;
 }  // namespace pmk
 using namespace pmk;
 

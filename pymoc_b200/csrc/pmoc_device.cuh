@@ -870,10 +870,10 @@ struct SoPar {
 struct SoSurf {  // per-refresh scan of bs(y)
   double mn, bsN, y0, yN;
   int south;
-  int ndown;  // segments north of the minimum on which bs decreases
+  int ndown;  // grid intervals north of the minimum on which bs decreases (adjacent ones counted one by one)
   bool mono;  // ndown == 0
 };
-constexpr int kSawtoothSegments = 3;  // PMOC_ST_BS_SAWTOOTH: this many decreasing segments north of the minimum
+constexpr int kSawtoothSegments = 3;  // PMOC_ST_BS_SAWTOOTH: this many decreasing intervals north of the minimum
 // block-cooperative copy of the four host-evaluated taper profiles into lane-major shared memory
 template <int LPL>
 PM_DEV void taper_fill(double* dst, const double* PM_RESTRICT sill, const double* PM_RESTRICT ektap,
@@ -1067,8 +1067,9 @@ PM_COLD bool cell_propagators_adaptive(const double (&Q0)[LPL], const double (&Q
     for (int j = 0; j < LPL; ++j) {
       const double na = (Q0[j] * ak[j] + Q1[j] * am[j]) * inv;
       const double nb = (Q0[j] * bk[j] + Q1[j] * bm[j]) * inv;
-      big |= !((fabs(na) + fabs(an[j])) <= 1e-19 * fabs(A[j]));
-      big |= !((fabs(nb) + fabs(bn[j])) * kk <= 1e-19 * (fabs(Bh[j]) + fabs(D[j])));
+      // (an overflowed sum is not converged: inf <= 1e-19 * inf would pass the test)
+      big |= !((fabs(na) + fabs(an[j])) <= 1e-19 * fabs(A[j]) && fabs(A[j]) <= 1.79e308);
+      big |= !((fabs(nb) + fabs(bn[j])) * kk <= 1e-19 * (fabs(Bh[j]) + fabs(D[j])) && fabs(D[j]) <= 1.79e308);
       A[j] = A[j] + na;
       Bh[j] = Bh[j] + nb;
       D[j] = D[j] + kk * nb;

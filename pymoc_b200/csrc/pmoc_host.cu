@@ -344,7 +344,9 @@ extern "C" int pmoc_host_step(pmoc_host* h, int64_t it0, int64_t nsteps, uint32_
   // an order-'post' loop is entered with diagnosed streamfunctions (the scripts' pre-loop solve()): at it0 == 0,
   // and whenever the caller replaces the state without supplying streamfunctions that match it
   const bool need_diag = !jn && (it0 == 0 || ((push & PMOC_IO_STATE) && !(push & PMOC_IO_PSI) && !h->diagnosed));
+  if (push & PMOC_IO_PSI) mr.d.flags |= kFlagPsiPushed;  // the caller's streamfunctions: no carried exemption
   const int rc = mr.pass(push, need_diag, nsteps > 0, it0, nsteps, pull);
+  mr.d.flags &= ~kFlagPsiPushed;
   const cudaError_t e = mr.sync();
   if (rc != PMOC_OK) return rc;
   PM_CUDA_OK(mr.err);

@@ -133,7 +133,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
   // which of them are rounding noise (bit 0: Psi_so[1], 1: Psi_iso_b[1], 2: Psi_iso_n[1]); so1_exact: Psi_so[1] came
   // out of state-independent arithmetic and is reproduced bit for bit even then (PMOC_ST_CARRY_SO1_EXACT)
   int noise = 0;
-  bool so1_exact = ML && M.status != nullptr && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) != 0;
+  bool so1_exact = ML && M.status != nullptr && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) != 0 && !(M.flags & kFlagPsiPushed);
   if (ML) {
     pm::ml_setup(ml, ysm, ny, vat(M.ml_Ks, m), vat(M.ml_h, m), vat(M.ml_L, m), vat(M.ml_vpist, m),
                  vrow(M.ml_surflux, m), vrow(M.ml_rest_mask, m), vrow(M.ml_b_rest, m), dt, ws + sp.w_scan);

@@ -113,7 +113,7 @@ PM_GLOBAL void k_wide_geo(WideArgs a) {
 // (same expressions as pm::tw_solve / tw_psib / interp_bgrid / so_solve, level loops instead of
 // register chunks).  The parts follow the model's flags: the thermal wind against the northern column
 // or the fixed profile tw_b2, the remap only with PMOC_ISO, Psi_SO on the mixed layer's bs ('jn') or on
-// so_bs ('post').  The rounding-noise bookkeeping of the 'jn' switches (PMOC_ST_CARRY_*) is 'jn' only.
+// so_bs ('post').  The carry bit of the 'jn' switches (PMOC_ST_CARRY_SO1_EXACT) is 'jn' only.
 PM_GLOBAL void k_wide_refresh(WideArgs a) {
   const pmoc_model& M = a.m;
   const bool JN = (M.flags & PMOC_ORDER_JN) != 0, NORTH = (M.flags & PMOC_HAS_NORTH) != 0;
@@ -146,8 +146,7 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
   }
   rt::syncblock();
 
-  double mxl = 0.0, so1 = 0.0, resb1 = 0.0, resn1 = 0.0;  // ('jn' only, see the end)
-  bool exact1 = false;
+  bool exact1 = false;  // ('jn' only, see the end)
   if (TW) {
     // --- thermal wind: Psi'' = (b2-b1)/f (psi_thermwind.py:123-135), see pm::tw_solve.  A = T (Simpson
     // increments of Psi'), B = their exclusive prefix, C = cell integrals -> exclusive prefix, P = Psi (Sv)
@@ -303,15 +302,9 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
       if (M.psib) M.psib[m * nb + i] = psib_s[i];
       if (M.bgrid) M.bgrid[m * nb + i] = G.at(i);
     }
-    // what the 'jn' switches of the step kernel read (level 1 of the three streamfunctions), and the scale
-    // against which they count as rounding noise (PMOC_ST_NOISE_SWITCH)
     for (int i = t; i < nz; i += T) {
-      const double vb = pm::interp_bgrid(b1[i], G, psib_s), vn = pm::interp_bgrid(b2[i], G, psib_s);
-      M.Psi_iso_b[m * nz + i] = vb;
-      M.Psi_iso_n[m * nz + i] = vn;
-      mxl = fabs(vb) > mxl ? fabs(vb) : mxl;
-      mxl = fabs(vn) > mxl ? fabs(vn) : mxl;
-      if (i == 1) { resb1 = vb; resn1 = vn; }
+      M.Psi_iso_b[m * nz + i] = pm::interp_bgrid(b1[i], G, psib_s);
+      M.Psi_iso_n[m * nz + i] = pm::interp_bgrid(b2[i], G, psib_s);
     }
   }
 
@@ -354,8 +347,6 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
       g = pm::div_const(g, c6, r6);
       const double v = i == 0 ? 0. : e + g;
       M.Psi_so[m * nz + i] = v;
-      mxl = fabs(v) > mxl ? fabs(v) : mxl;
-      if (i == 1) so1 = v;
       if (M.Psi_Ek) M.Psi_Ek[m * nz + i] = e;
       if (M.Psi_GM) M.Psi_GM[m * nz + i] = g;
     }
@@ -365,21 +356,12 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
     if (t == 0 && M.status) M.status[m] = (M.status[m] | all) & ~PMOC_ST_CARRY_MASK;
     return;
   }
-  mxl = rt::wmax(mxl);
+  // whether Psi_so[1] came out of state-independent arithmetic, for the step kernel's noise classification
   rt::syncblock();
-  if (rt::lane() == 0) red[rt::warp_in_block()] = mxl;
-  if (t == 1 % T) {  // the thread that owns level 1
-    red[32] = so1; red[33] = resb1; red[34] = resn1; red[35] = exact1 ? 1.0 : 0.0;
-  }
+  if (t == 1 % T) red[0] = exact1 ? 1.0 : 0.0;  // the thread that owns level 1
   rt::syncblock();
-  if (t == 0 && M.status) {
-    double mx = 0.0;
-    for (int w = 0; w < rt::warps_per_block(); ++w) mx = red[w] > mx ? red[w] : mx;
-    const double tiny = 1e-12 * mx, s1 = fabs(red[32]), s2 = fabs(red[33]), s3 = fabs(red[34]);
-    const unsigned noise = ((s1 > 0 && s1 < tiny && red[35] == 0.0) ? 1u : 0u) | ((s2 > 0 && s2 < tiny) ? 2u : 0u) |
-                           ((s3 > 0 && s3 < tiny) ? 4u : 0u);
-    M.status[m] = ((M.status[m] | all) & ~PMOC_ST_CARRY_MASK) | (noise << PMOC_ST_CARRY_NOISE_SHIFT);
-  }
+  if (t == 0 && M.status)
+    M.status[m] = ((M.status[m] | all) & ~PMOC_ST_CARRY_MASK) | (red[0] != 0.0 ? PMOC_ST_CARRY_SO1_EXACT : 0u);
 }
 
 // ---- the steps, state and per-level constants resident on chip ---------------------------------
@@ -462,6 +444,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
   double dzu_m = 1., rdzu_m = 1.;  // cell below the thread's first level
   int fnz = 0x7fffffff, fpos = 0x7fffffff;
   bool areas_differ = false;
+  double mxl = 0.0;  // largest |Psi| of the three streamfunctions: the scale of rounding noise
   PM_UNROLL
   for (int j = 0; j < LPT; ++j) {
     const int i = lo + j;
@@ -479,6 +462,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
       rdzc[j] = a.geo[3 * nz + i];
       const double pso = M.Psi_so[m * nz + i], ib = M.Psi_iso_b[m * nz + i], in_ = M.Psi_iso_n[m * nz + i];
       pm_s[i] = pso;
+      mxl = fmax(mxl, fmax(fabs(pso), fmax(fabs(ib), fabs(in_))));
       if (pso != 0.0 && i < fnz) fnz = i;
       if (pso > 0.0 && i < fpos) fpos = i;
       const bool in = i >= 1 && i < nz - 1;
@@ -501,12 +485,21 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
     rdzu_m = a.geo[nz + lo - 1];
   }
   for (int i = t; i < nyp; i += kWideAll) ysm[i] = M.y[i < ny ? i : ny - 1];
+  mxl = rt::wmax(mxl);
+  if (Ln == 0) scan_s[W] = mxl;  // (scan_s is free until ml_setup, behind the barriers below)
   fnz = block_min(fnz, cbox);
   fpos = block_min(fpos, cbox);
   const bool uniA = !block_any(areas_differ, cbox);
   const double A_b = Ab[1], rA_b = 1.0 / A_b, A_n = An[1], rA_n = 1.0 / A_n;
   const double psi_so1 = M.Psi_so[m * nz + 1], res_b1 = M.Psi_iso_b[m * nz + 1], res_n1 = M.Psi_iso_n[m * nz + 1];
-  const unsigned noise = M.status ? (M.status[m] >> PMOC_ST_CARRY_NOISE_SHIFT) & 7u : 0u;  // set by k_wide_refresh
+  // which of the three are rounding noise (bit 0: Psi_so[1], 1: Psi_iso_b[1], 2: Psi_iso_n[1]), classified from the
+  // loaded streamfunctions as k_model does; Psi_so[1] is exempt when k_wide_refresh produced it by state-independent
+  // arithmetic, unless the caller has replaced the streamfunctions since (kFlagPsiPushed)
+  for (int w = 0; w < rt::warps_per_block(); ++w) mxl = fmax(mxl, scan_s[w]);
+  const bool so1_exact = M.status && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) && !(M.flags & kFlagPsiPushed);
+  const double tiny = 1e-12 * mxl, s1 = fabs(psi_so1), s2 = fabs(res_b1), s3 = fabs(res_n1);
+  const unsigned noise = ((s1 > 0 && s1 < tiny && !so1_exact) ? 1u : 0u) | ((s2 > 0 && s2 < tiny) ? 2u : 0u) |
+                         ((s3 > 0 && s3 < tiny) ? 4u : 0u);
   if (fnz == 0x7fffffff) status |= PMOC_ST_ML_INDEX;
   const double held = pm_s[fnz == 0x7fffffff ? 0 : fnz];
   rt::syncblock();
@@ -954,7 +947,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
     if (M.north.var) M.north.var[m] = var_n;
   }
   const unsigned all = block_or(status, cbox);  // the mixed-layer warp carries SO_ML's bits
-  if (t == 0 && M.status) M.status[m] |= all;
+  if (t == 0 && M.status) M.status[m] = (M.status[m] | all) & ~(so1_exact ? 0u : PMOC_ST_CARRY_SO1_EXACT);
 }
 
 // ---- the steps of the 'post' order (example_twocol_plusSO.py:99-115) ----------------------------
@@ -1238,8 +1231,10 @@ int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, in
     return PMOC_OK;
   }
   while (ii < it_end) {
-    if (ii % K == 0)
+    if (ii % K == 0) {
       if (int rc = launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a)) return rc;
+      a.m.flags &= ~kFlagPsiPushed;  // the streamfunctions are the diagnosis's own from here on
+    }
     long long stop = (ii / K + 1) * K;
     if (stop > it_end) stop = it_end;
     a.it0 = ii;

@@ -238,6 +238,16 @@ static inline long long blocks_for(long long M) { return (M + kWarpsPerBlock - 1
 // streamfunctions (PMOC_IO_PSI): the 'jn' step kernels then classify them as rounding noise without the
 // PMOC_ST_CARRY_SO1_EXACT exemption of an earlier diagnosis, which does not describe them.
 constexpr unsigned kFlagPsiPushed = 0x80000000u;
+
+// The carry of the 'jn' switches (PMOC_ST_CARRY_SO1_EXACT): the member's Psi_so[1] came out of state-independent
+// arithmetic at the last diagnosis, and the carried streamfunctions are still that diagnosis's own.
+PM_DEV bool so1_exact_carried(const pmoc_model& M, long long m) {
+  return M.status && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) && !(M.flags & kFlagPsiPushed);
+}
+// A member's status word after a kernel: the old bits and the kernel's, the internal carries replaced by `carry`.
+PM_DEV unsigned status_word(unsigned old, unsigned bits, bool carry) {
+  return ((old | bits) & ~PMOC_ST_CARRY_MASK) | (carry ? PMOC_ST_CARRY_SO1_EXACT : 0u);
+}
 }  // namespace pmk
 using namespace pmk;
 

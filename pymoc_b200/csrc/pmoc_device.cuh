@@ -279,6 +279,21 @@ PM_DEV void col_nweff(const ExactCol& T, const double (&wA)[LPL], const double* 
   rt::syncwarp();
 }
 
+// One level of the bit-faithful explicit step (column.py:235-249): g_up / g_dn are the gradients of the cells above
+// and below, nweff = -weff, A / rA the Area and its reciprocal.  Every kernel that steps a column this way calls it,
+// so that they all round the same operations in the same order.  The operands that callers keep in memory are taken by
+// reference: each is then loaded where the arithmetic needs it, not ahead of the level's gradients (register pressure
+// of the step loops).
+PM_DEV double exact_level(double b, double g_up, double g_dn, const double& dzc, const double& rdzc,
+                          const double& nweff, const double& kappa, const double& A, const double& rA, double dt) {
+  const double bzz = div_const(g_up - g_dn, dzc, rdzc);
+  const double sel = nweff > 0 ? g_up : g_dn;  // weff < 0  <=>  -weff > 0
+  const double a = A, ra = rA;  // (read before the product: fewer registers in k_wide_post)
+  const double adv = div_const(nweff * sel, a, ra);
+  const double tend = adv + kappa * bzz;
+  return b + dt * tend;
+}
+
 template <int LPL>
 PM_DEV void col_step_exact(double (&b)[LPL], const ExactCol& T, int var, const ExactGeo& G, int nz, double dt) {
   // (offsets from one base pointer, not a run-time pick between two pointers: the loads stay LDS)
@@ -298,14 +313,16 @@ PM_DEV void col_step_exact(double (&b)[LPL], const ExactCol& T, int var, const E
     const int i = lev<LPL>(j), s = lm(j);
     if (i >= 1 && i < nz - 1) {
       const double bzd = j > 0 ? bzu[j > 0 ? j - 1 : 0] : bzprev;
-      const double bzz = div_const(bzu[j] - bzd, G.dzc[s], G.rdzc[s]);
-      const double nw = nweff[s];
-      const double sel = nw > 0 ? bzu[j] : bzd;  // weff < 0  <=>  -weff > 0
-      const double adv = div_const(nw * sel, T.area[s], T.rarea[s]);
-      const double tend = adv + kap[s] * bzz;
-      b[j] = b[j] + dt * tend;
+      b[j] = exact_level(b[j], bzu[j], bzd, G.dzc[s], G.rdzc[s], nweff[s], kap[s], T.area[s], T.rarea[s], dt);
     }
   }
+}
+
+// Convective adjustment of one value (column.py:264-271): with convection (cv) a value above bs becomes
+// bs + N2min (z[i] - zc), zc the depth of the highest stable level; without, only the surface value is reset to bs.
+PM_DEV double convect_level(double v, int i, bool cv, double bs, double n2, double zc, const double* z, int nz) {
+  if (cv) return v > bs ? bs + n2 * (z[i] - zc) : v;
+  return i == nz - 1 ? bs : v;
 }
 
 // Convective adjustment (column.py:264-271).  Strict '>' and un-fused bs + N2min*(z - zconv).
@@ -862,7 +879,7 @@ PM_DEV double mean100(double tau) {
 struct SoPar {
   double tau_ave, f, rho, L, KGM, smax;
   double pre0;  // tau_ave / f / rho * L (psi_SO.py:243, left to right), constant between launches
-  const double *sill, *ektap, *toptap, *bottap;  // taper profiles, lane-major (shared memory)
+  const double *sill, *ektap, *toptap, *bottap;  // taper profiles (so_solve: lane-major in shared memory)
   const double* tau_y;                           // tau on the y grid (shared memory) or nullptr for a float tau
   double c;                                      // F2010 phase speed (BVP branch only)
   int with_Ek;
@@ -1271,6 +1288,32 @@ PM_DEV void outcrop_monotone_all(double (&yo)[LPL], const double (&b)[LPL], cons
   }
 }
 
+// One level of Psi_SO's explicit branch (psi_SO.py:302-354) for the member's parameters P: level i, taper slot s.
+// Shared by so_solve and the block-per-member diagnosis.  exact1 is set when at level 1, with a wind stress
+// independent of y, the slope clip or the limiter chose a value made of the member's constants only: Psi_so[1] is
+// then reproduced bit for bit whatever the state (PMOC_ST_CARRY_SO1_EXACT).
+// Ekman transport, Sv (pre = tau / f / rho * L)
+PM_DEV double so_ekman(double pre, const SoPar& P, int s) {
+  return div_const(pre * P.sill[s] * P.ektap[s], 1e6, 1.0 / 1e6);
+}
+// GM transport with the slope sl = z / dy clipped at -smax, before the limiter
+PM_DEV double so_gm_clip(double sl, const SoPar& P, int s, int i, bool& exact1) {
+  const double ms = -P.smax;
+  const double mx = (sl >= ms || sl != sl) ? sl : ms;
+  const double g = P.KGM * mx * P.L * P.toptap[s] * P.bottap[s];
+  if (i == 1 && !(sl >= ms || sl != sl) && P.tau_y == nullptr) exact1 = true;  // the slope clip: constants only
+  return g;
+}
+// the limiter where the outcrop lies south of the channel (dy > span = yN - y0): GM >= -Ek; then GM in Sv
+PM_DEV double so_gm_limit(double gm, double ek, double dy, double span, const SoPar& P, int i, bool& exact1) {
+  if (dy > span) {
+    const double alt = -ek * 1e6;
+    if (i == 1 && !(gm >= alt || gm != gm) && P.tau_y == nullptr) exact1 = true;  // Psi = Ek - (Ek*1e6)/1e6
+    gm = (gm >= alt || gm != gm) ? gm : alt;
+  }
+  return div_const(gm, 1e6, 1.0 / 1e6);
+}
+
 // Psi_SO.solve (psi_SO.py:106-140, 218-243, 302-354): outcrop latitudes, Ekman transport, GM
 // transport with the explicit slope clip or (BVP) the F2010 smoother.  Sv.  The four taper
 // profiles are read lane-major (slot lm(j)) from P.sill/ektap/toptap/bottap.
@@ -1280,7 +1323,6 @@ PM_DEV void so_solve(double (&psi)[LPL], double (&ek)[LPL], double (&gm)[LPL], d
                      const SoSurf& S, const SoPar& P, const double* zs, int nz, unsigned* status,
                      bool* psi1_exact = nullptr) {
   const double pre0 = P.pre0;
-  const double c6 = 1e6, r6 = 1.0 / 1e6;
   if (S.mono && S.south < ny - 1) {
     outcrop_monotone_all<LPL>(ysv, b, ygrid, bs, sinv, ny, S);
   } else {
@@ -1320,20 +1362,15 @@ PM_DEV void so_solve(double (&psi)[LPL], double (&ek)[LPL], double (&gm)[LPL], d
     const int i = lev<LPL>(j), s = lm(j);
     const bool in = i < nz;
     const double yo = in ? ysv[j] : 0.0;
-    const double pre = prev[j];
-    const double e = div_const(pre * P.sill[s] * P.ektap[s], c6, r6);
+    const double e = so_ekman(prev[j], P, s);
     double dy = S.yN - yo;
     dy = 0.1 > dy ? 0.1 : dy;
     const double z = zs[i < nz ? i : nz - 1];
     double g;
-    if (BVP) {
+    if (BVP)
       g = rt::div_normal(P.KGM * z, dy) * P.L * P.toptap[s] * P.bottap[s];  // dy >= 0.1
-    } else {
-      const double sl = rt::div_normal(z, dy), ms = -P.smax;  // dy >= 0.1, |z| <= H: in range
-      const double mx = (sl >= ms || sl != sl) ? sl : ms;
-      g = P.KGM * mx * P.L * P.toptap[s] * P.bottap[s];
-      if (i == 1 && !(sl >= ms || sl != sl) && P.tau_y == nullptr) exact1 = true;  // the slope clip: constants only
-    }
+    else
+      g = so_gm_clip(rt::div_normal(z, dy), P, s, i, exact1);  // dy >= 0.1, |z| <= H: in range
     ek[j] = in ? e : 0.0;
     gm[j] = in ? g : 0.0;
     dyv[j] = in ? dy : 1.0;
@@ -1350,13 +1387,7 @@ PM_DEV void so_solve(double (&psi)[LPL], double (&ek)[LPL], double (&gm)[LPL], d
   PM_UNROLL
   for (int j = 0; j < LPL; ++j) {
     const int i = lev<LPL>(j);
-    double t = gm[j];
-    if (dyv[j] > S.yN - S.y0) {
-      const double alt = -ek[j] * 1e6;
-      if (i == 1 && !(t >= alt || t != t) && P.tau_y == nullptr) exact1 = true;  // the limiter: Psi = Ek - (Ek*1e6)/1e6
-      t = (t >= alt || t != t) ? t : alt;
-    }
-    const double g = div_const(t, c6, r6);
+    const double g = so_gm_limit(gm[j], ek[j], dyv[j], S.yN - S.y0, P, i, exact1);
     const bool in = i < nz;
     gm[j] = in ? g : 0.0;
     psi[j] = (in && i != 0) ? ek[j] + g : 0.0;
@@ -1781,6 +1812,48 @@ PM_DEV bool ml_bind_basin(const double (&b)[LPL], int nz, double* bb_s) {
   const bool sorted = rt::ballot(bad) == 0;  // ballot also orders the stores before the reads
   rt::syncwarp();
   return sorted;
+}
+
+// ---- the 'jn' bottom-boundary switches (run_JansenNadeau_2018.py:233-254), shared by the warp- and block-per-member
+// kernels.  psi_so1, res_b1, res_n1: Psi[1] of Psi_SO, Psi_iso_b and Psi_iso_n; bb0, bb1 / nb0, nb1: levels 0 and 1
+// of the basin / northern column before the step; bs0: bs[0] of the mixed layer.
+//
+// Which of psi_so1, res_b1, res_n1 are rounding noise (bits 0, 1, 2): non-zero and below 1e-12 of mx, the largest
+// |Psi| of the three streamfunctions.  psi_so1 is exempt when so1_exact: it came out of state-independent arithmetic
+// (PMOC_ST_CARRY_SO1_EXACT).
+PM_DEV unsigned jn_noise(double psi_so1, double res_b1, double res_n1, double mx, bool so1_exact) {
+  const double tiny = 1e-12 * mx, s1 = fabs(psi_so1), s2 = fabs(res_b1), s3 = fabs(res_n1);
+  return ((s1 > 0 && s1 < tiny && !so1_exact) ? 1u : 0u) | ((s2 > 0 && s2 < tiny) ? 2u : 0u) |
+         ((s3 > 0 && s3 < tiny) ? 4u : 0u);
+}
+// the basin's bottom value and kappa variant (both kept when no branch applies, e.g. for a NaN psi_so1)
+PM_DEV void jn_switch_basin(double psi_so1, double res_b1, double bb1, double nb0, double bs0, double& bbot, int& var) {
+  if (psi_so1 < 0) {
+    bbot = bs0;
+    var = 1;
+  }
+  if (res_b1 > 0 && nb0 < bb1 && nb0 < bs0) {
+    bbot = nb0;
+    var = 1;
+  } else if (psi_so1 >= 0) {
+    bbot = bb1;
+    var = 0;
+  }
+}
+// the northern column's bottom value and kappa variant
+PM_DEV void jn_switch_north(double res_n1, double bb0, double nb1, double& bbot, int& var) {
+  if (res_n1 < 0 && bb0 < nb1) {
+    bbot = bb0;
+    var = 1;
+  } else {
+    bbot = nb1;
+    var = 0;
+  }
+}
+// PMOC_ST_NOISE_SWITCH when the outcome of a switch hung on the sign of a noise value (the other operands let it through)
+PM_DEV void jn_noise_hit(unsigned noise, double bb0, double bb1, double nb0, double nb1, double bs0, unsigned* status) {
+  if (noise != 0 && ((noise & 1u) || ((noise & 2u) && nb0 < bb1 && nb0 < bs0) || ((noise & 4u) && bb0 < nb1)))
+    *status |= 64u;  // PMOC_ST_NOISE_SWITCH
 }
 
 }  // namespace pm

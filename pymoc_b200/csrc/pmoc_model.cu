@@ -130,10 +130,9 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
   double* const bb_s = ws + (ML ? sp.w_bb : 0);
   double* const pm_s = ws + (ML ? sp.w_pm : 0);
   double psi_so1 = 0., res_b1 = 0., res_n1 = 0.;  // Psi[1] of the three streamfunctions ('jn' switches)
-  // which of them are rounding noise (bit 0: Psi_so[1], 1: Psi_iso_b[1], 2: Psi_iso_n[1]); so1_exact: Psi_so[1] came
-  // out of state-independent arithmetic and is reproduced bit for bit even then (PMOC_ST_CARRY_SO1_EXACT)
-  int noise = 0;
-  bool so1_exact = ML && M.status != nullptr && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) != 0 && !(M.flags & kFlagPsiPushed);
+  // which of them are rounding noise (pm::jn_noise); so1_exact: Psi_so[1] came out of state-independent arithmetic
+  unsigned noise = 0;
+  bool so1_exact = ML && so1_exact_carried(M, m);
   if (ML) {
     pm::ml_setup(ml, ysm, ny, vat(M.ml_Ks, m), vat(M.ml_h, m), vat(M.ml_L, m), vat(M.ml_vpist, m),
                  vrow(M.ml_surflux, m), vrow(M.ml_rest_mask, m), vrow(M.ml_b_rest, m), dt, ws + sp.w_scan);
@@ -189,9 +188,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
         mx = a2 > mx ? a2 : mx;
         mx = a3 > mx ? a3 : mx;
       }
-      const double tiny = 1e-12 * rt::wmax(mx);
-      const double s1 = fabs(psi_so1), s2 = fabs(res_b1), s3 = fabs(res_n1);
-      noise = ((s1 > 0 && s1 < tiny && !so1_exact) ? 1 : 0) | ((s2 > 0 && s2 < tiny) ? 2 : 0) | ((s3 > 0 && s3 < tiny) ? 4 : 0);
+      noise = pm::jn_noise(psi_so1, res_b1, res_n1, rt::wmax(mx), so1_exact);
     }
   };
 
@@ -363,27 +360,9 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
         const double nb0 = rt::shfl(cn.b[0], 0), nb1 = rt::shfl(cn.b[1], 0);
         const double bs0 = rt::shfl(ml.bs[0], 0);
         int vb = cb.var, vn = cn.var;
-        if (psi_so1 < 0) {
-          cb.bbot = bs0;
-          vb = 1;
-        }
-        if (res_b1 > 0 && nb0 < bb1 && nb0 < bs0) {
-          cb.bbot = nb0;
-          vb = 1;
-        } else if (psi_so1 >= 0) {
-          cb.bbot = bb1;
-          vb = 0;
-        }
-        if (res_n1 < 0 && bb0 < nb1) {
-          cn.bbot = bb0;
-          vn = 1;
-        } else {
-          cn.bbot = nb1;
-          vn = 0;
-        }
-        // a switch whose outcome hung on the sign of a noise value (the other operands let it through)
-        if (noise != 0 && ((noise & 1) || ((noise & 2) && nb0 < bb1 && nb0 < bs0) || ((noise & 4) && bb0 < nb1)))
-          status |= PMOC_ST_NOISE_SWITCH;
+        pm::jn_switch_basin(psi_so1, res_b1, bb1, nb0, bs0, cb.bbot, vb);
+        pm::jn_switch_north(res_n1, bb0, nb1, cn.bbot, vn);
+        pm::jn_noise_hit(noise, bb0, bb1, nb0, nb1, bs0, &status);
         if (two_var_b) cb.var = vb;
         if (two_var_n) cn.var = vn;
         col_advance_exact<LPL>(cb, xb, EG, G, nz, dt);
@@ -396,11 +375,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
     }
   }
   auto put_status = [&]() {
-    if (M.status && L == 0) {
-      unsigned w = (M.status[m] | status) & ~PMOC_ST_CARRY_SO1_EXACT;
-      if (ML && so1_exact) w |= PMOC_ST_CARRY_SO1_EXACT;
-      M.status[m] = w;
-    }
+    if (M.status && L == 0) M.status[m] = status_word(M.status[m], status, ML && so1_exact);
   };
   if (dg) {
     put_status();

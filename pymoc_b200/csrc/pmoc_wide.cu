@@ -315,9 +315,12 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
     if (!S.mono) status |= PMOC_ST_BS_NONMONOTONE;
     if (S.ndown >= pm::kSawtoothSegments) status |= PMOC_ST_BS_SAWTOOTH;
     const double tau_ave = pm::mean100(vat(M.so_tau, m));
-    const double sf = vat(M.so_f, m), srho = vat(M.so_rho, m), sL = vat(M.so_L, m), sK = vat(M.so_KGM, m),
-                 smax = vat(M.so_smax, m);
-    const double pre = tau_ave / sf / srho * sL, c6 = 1e6, r6 = 1.0 / 1e6;
+    pm::SoPar P{};  // (constant wind stress: tau_y = nullptr; tapers in natural order)
+    P.L = vat(M.so_L, m);
+    P.KGM = vat(M.so_KGM, m);
+    P.smax = vat(M.so_smax, m);
+    P.sill = M.so_sill_taper; P.ektap = M.so_ek_taper; P.toptap = M.so_top_taper; P.bottap = M.so_bot_taper;
+    const double pre = tau_ave / vat(M.so_f, m) / vat(M.so_rho, m) * P.L;
     for (int i = t; i < nz; i += T) {
       const double bi = b1[i];
       double yo;
@@ -332,19 +335,11 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
         yo = pm::outcrop_brent(bi, ysm, bs_s, ny, S.south, &bad);
         if (bad) status |= PMOC_ST_BRENT_SIGN;
       }
-      const double e = pm::div_const(pre * M.so_sill_taper[i] * M.so_ek_taper[i], c6, r6);
+      const double e = pm::so_ekman(pre, P, i);
       double dy = S.yN - yo;
       dy = 0.1 > dy ? 0.1 : dy;
-      const double sl = pm::qdiv(z[i], dy), ms = -smax;
-      const double mx = (sl >= ms || sl != sl) ? sl : ms;
-      double g = sK * mx * sL * M.so_top_taper[i] * M.so_bot_taper[i];
-      if (i == 1 && !(sl >= ms || sl != sl)) exact1 = true;  // the slope clip: constants only (see pm::so_solve)
-      if (dy > S.yN - S.y0) {
-        const double alt = -e * 1e6;
-        if (i == 1 && !(g >= alt || g != g)) exact1 = true;  // the limiter
-        g = (g >= alt || g != g) ? g : alt;
-      }
-      g = pm::div_const(g, c6, r6);
+      double g = pm::so_gm_clip(pm::qdiv(z[i], dy), P, i, i, exact1);
+      g = pm::so_gm_limit(g, e, dy, S.yN - S.y0, P, i, exact1);
       const double v = i == 0 ? 0. : e + g;
       M.Psi_so[m * nz + i] = v;
       if (M.Psi_Ek) M.Psi_Ek[m * nz + i] = e;
@@ -353,15 +348,14 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
   }
   const unsigned all = block_or(status, ibox);
   if (!JN) {
-    if (t == 0 && M.status) M.status[m] = (M.status[m] | all) & ~PMOC_ST_CARRY_MASK;
+    if (t == 0 && M.status) M.status[m] = status_word(M.status[m], all, false);
     return;
   }
   // whether Psi_so[1] came out of state-independent arithmetic, for the step kernel's noise classification
   rt::syncblock();
   if (t == 1 % T) red[0] = exact1 ? 1.0 : 0.0;  // the thread that owns level 1
   rt::syncblock();
-  if (t == 0 && M.status)
-    M.status[m] = ((M.status[m] | all) & ~PMOC_ST_CARRY_MASK) | (red[0] != 0.0 ? PMOC_ST_CARRY_SO1_EXACT : 0u);
+  if (t == 0 && M.status) M.status[m] = status_word(M.status[m], all, red[0] != 0.0);
 }
 
 // ---- the steps, state and per-level constants resident on chip ---------------------------------
@@ -492,14 +486,10 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
   const bool uniA = !block_any(areas_differ, cbox);
   const double A_b = Ab[1], rA_b = 1.0 / A_b, A_n = An[1], rA_n = 1.0 / A_n;
   const double psi_so1 = M.Psi_so[m * nz + 1], res_b1 = M.Psi_iso_b[m * nz + 1], res_n1 = M.Psi_iso_n[m * nz + 1];
-  // which of the three are rounding noise (bit 0: Psi_so[1], 1: Psi_iso_b[1], 2: Psi_iso_n[1]), classified from the
-  // loaded streamfunctions as k_model does; Psi_so[1] is exempt when k_wide_refresh produced it by state-independent
-  // arithmetic, unless the caller has replaced the streamfunctions since (kFlagPsiPushed)
+  // which of the three are rounding noise, classified from the loaded streamfunctions as k_model does
   for (int w = 0; w < rt::warps_per_block(); ++w) mxl = fmax(mxl, scan_s[w]);
-  const bool so1_exact = M.status && (M.status[m] & PMOC_ST_CARRY_SO1_EXACT) && !(M.flags & kFlagPsiPushed);
-  const double tiny = 1e-12 * mxl, s1 = fabs(psi_so1), s2 = fabs(res_b1), s3 = fabs(res_n1);
-  const unsigned noise = ((s1 > 0 && s1 < tiny && !so1_exact) ? 1u : 0u) | ((s2 > 0 && s2 < tiny) ? 2u : 0u) |
-                         ((s3 > 0 && s3 < tiny) ? 4u : 0u);
+  const bool so1_exact = so1_exact_carried(M, m);
+  const unsigned noise = pm::jn_noise(psi_so1, res_b1, res_n1, mxl, so1_exact);
   if (fnz == 0x7fffffff) status |= PMOC_ST_ML_INDEX;
   const double held = pm_s[fnz == 0x7fffffff ? 0 : fnz];
   rt::syncblock();
@@ -566,108 +556,90 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
   if (col) publish(0);
   rt::syncblock();
 
+  // the owner re-reads its levels of kappa variant v of one column: -weff of both variants from the scratch buffer
+  // (nw0, nw1), kappa from the model (variant 1 at offset nv)
+  auto load_variant = [&](double* nw, double* kp, const double* nw0, const double* nw1, const double* kap, int nv,
+                          int v) {
+    PM_UNROLL
+    for (int j = 0; j < LPT; ++j) {
+      const int i = lo + j, s = j * kWideCol + t;
+      if (i < nz) {
+        nw[s] = v ? nw1[i] : nw0[i];
+        kp[s] = (i >= 1 && i < nz - 1) ? kap[(v ? nv : 0) + i] : 0.0;
+      }
+    }
+  };
+  // one SO_ML step of the mixed-layer warp on the profile published with the flags of buffer q; b_basin sorted?
+  // inside the threads and warps: flagged by publish; across the warps: here.  bs[0] goes to dbox[0].
+  auto ml_published = [&](pm::MlState& s, int q) {
+    bool bad = ibox[8 * q + 4] != 0;
+    const int e = (Ln + 1) * 32 * LPT;  // first level of the next warp
+    if (Ln < kWideCol / 32 - 1 && e < nz) bad |= !(bbx[e] >= bbx[e - 1]);
+    pm::ml_step(s, bbx, pm_s, nz, rt::ballot(bad) == 0, bs_s, dt, &status);
+    if (Ln == 0) dbox[0] = s.bs[0];
+  };
+
   int p = 0;
   if constexpr (PIPE) {
-    // one SO_ML step of the mixed-layer warp on the published profile (flags of buffer q)
-    auto ml_one = [&](int q) {
-      // b_basin sorted?  inside the threads and warps: flagged by publish; across the warps: here
-      bool bad = ibox[8 * q + 4] != 0;
-      const int e = (Ln + 1) * 32 * LPT;  // first level of the next warp
-      if (Ln < kWideCol / 32 - 1 && e < nz) bad |= !(bbx[e] >= bbx[e - 1]);
-      const bool sorted = rt::ballot(bad) == 0;
-      if (PIPE) {
-        pm::ml_step(ml, bbx, pm_s, nz, sorted, bs_s, dt, &status);
-        if (Ln == 0) dbox[0] = ml.bs[0];
-      } else {
-        pm::MlState tmp;
-        pm::ml_unpark(tmp, mlp, scan_s);
-        pm::ml_step(tmp, bbx, pm_s, nz, sorted, bs_s, dt, &status);
-        pm::ml_park(tmp, mlp, false);
-        if (Ln == 0) dbox[0] = tmp.bs[0];
-      }
-    };
-    auto ml_phase1 = [&](long long it, int q) {  // SO_ML of the previous iteration + the flags this iteration publishes
-      if (it > 0) ml_one(q);
-      if (Ln == 0) {  // (last read in the previous iteration)
-        int* f = ibox + 8 * (q ^ 1);
-        f[0] = 0; f[1] = 0; f[2] = -1; f[3] = -1; f[4] = 0;
-      }
-    };
     for (long long it = 0; it < a.nsteps; ++it, p ^= 1) {
       // ---------------------------------------------------------------- phase 1
       double gb1 = 0.;   // thread 0: gradient of basin cell 1-2 (kept for the deferred bottom levels)
       // the basin's kappa profile hangs on bs[0] of the SO_ML step still running (block-uniform: every thread,
       // the mixed-layer warp included, evaluates it from the published values)
       const bool late = (psi_so1 >= 0 && res_b1 > 0 && bne[0] < bbp[1] && M.basin.nvar > 1) || a.force_late != 0;
-      if (PIPE && mlw) {
-        ml_phase1(it, p);
+      if (mlw) {
+        // SO_ML of the previous iteration, then clear the flags this iteration publishes (last read in the previous one)
+        if (it > 0) ml_published(ml, p);
+        if (Ln == 0) {
+          int* f = ibox + 8 * (p ^ 1);
+          f[0] = 0; f[1] = 0; f[2] = -1; f[3] = -1; f[4] = 0;
+        }
       } else {
-        // what the switches need apart from bs[0] (run_JansenNadeau_2018.py:233-254); every thread evaluates them
-        // from the published values
-        const double bb0 = bbp[0], bb1 = bbp[1], nb0 = bne[0], nb1 = bne[2 * kWideCol];
+        // what the switches need apart from bs[0]; every thread evaluates them from the published values
+        const double bb0 = bbp[0], nb1 = bne[2 * kWideCol];
         int vn = var_n;
-        if (res_n1 < 0 && bb0 < nb1) { bbot_n = bb0; vn = 1; }
-        else { bbot_n = nb1; vn = 0; }
+        pm::jn_switch_north(res_n1, bb0, nb1, bbot_n, vn);
         if (M.north.nvar < 2) vn = 0;
         int vb = psi_so1 < 0 ? 1 : 0;  // (exact unless late; then phase 2 decides)
         if (M.basin.nvar < 2) vb = 0;
-        auto load_variant_b = [&](int v) {  // the owner re-reads its levels of the other variant
-          var_b = v;
-          PM_UNROLL
-          for (int j = 0; j < LPT; ++j) {
-            const int i = lo + j, s = j * kWideCol + t;
-            if (i < nz) {
-              nwb[s] = v ? nwb1[i] : nwb0[i];
-              kb[s] = (i >= 1 && i < nz - 1) ? kapb[(v ? nvb : 0) + i] : 0.0;
-            }
-          }
-        };
-        if (!late && vb != var_b) load_variant_b(vb);
+        if (!late && vb != var_b) {
+          var_b = vb;
+          load_variant(nwb, kb, nwb0, nwb1, kapb, nvb, vb);
+        }
         if (vn != var_n) {
           var_n = vn;
-          PM_UNROLL
-          for (int j = 0; j < LPT; ++j) {
-            const int i = lo + j, s = j * kWideCol + t;
-            if (i < nz) {
-              nwn[s] = vn ? nwn1[i] : nwn0[i];
-              kn[s] = (i >= 1 && i < nz - 1) ? kapn[(vn ? nvn : 0) + i] : 0.0;
-            }
-          }
+          load_variant(nwn, kn, nwn0, nwn1, kapn, nvn, vn);
         }
-        // convective adjustment (column.py:264-271) of the own levels and of the two neighbour values
+        // convective adjustment of the own levels and of the two neighbour values
         const int* f = ibox + 8 * p;
         const bool cvb = f[0] != 0, cvn = f[1] != 0;
         const double zcb = z[f[2] >= 0 ? f[2] : 0], zcn = z[f[3] >= 0 ? f[3] : 0];
-        auto adj = [&](double v, int i, bool cv, double bs, double n2, double zc) {
-          if (cv) return v > bs ? bs + n2 * (z[i] - zc) : v;
-          return i == nz - 1 ? bs : v;
-        };
         if ((cvb && mine_b) || (cvn && mine_n) || owns_top) {
           PM_UNROLL
           for (int j = 0; j < LPT; ++j) {
             const int i = lo + j;
             if (i < nz) {
-              bb[j] = adj(bb[j], i, cvb, bs_b, n2_b, zcb);
-              bn[j] = adj(bn[j], i, cvn, bs_n, n2_n, zcn);
+              bb[j] = pm::convect_level(bb[j], i, cvb, bs_b, n2_b, zcb, z, nz);
+              bn[j] = pm::convect_level(bn[j], i, cvn, bs_n, n2_n, zcn, z, nz);
             }
           }
         }
         if (t == 0) bn[0] = bbot_n;  // column.py:232 (the basin's bottom value waits for bs[0]: phase 2)
         double gpb = 0., gpn = 0.;  // gradient of the cell below the current level
         if (lo >= 1 && lo < nz) {
-          const double vb_ = adj(bbx[lo - 1], lo - 1, cvb, bs_b, n2_b, zcb);
-          const double vn_ = adj(bne[2 * (t - 1) + 1], lo - 1, cvn, bs_n, n2_n, zcn);
+          const double vb_ = pm::convect_level(bbx[lo - 1], lo - 1, cvb, bs_b, n2_b, zcb, z, nz);
+          const double vn_ = pm::convect_level(bne[2 * (t - 1) + 1], lo - 1, cvn, bs_n, n2_n, zcn, z, nz);
           gpb = pm::div_const(bb[0] - vb_, dzu_m, rdzu_m);
           gpn = pm::div_const(bn[0] - vn_, dzu_m, rdzu_m);
         }
         double ub = 0., un = 0.;  // level above the thread's last one
         if (lo + LPT < nz) {
-          ub = adj(bbx[lo + LPT], lo + LPT, cvb, bs_b, n2_b, zcb);
-          un = adj(bne[2 * (t + 1)], lo + LPT, cvn, bs_n, n2_n, zcn);
+          ub = pm::convect_level(bbx[lo + LPT], lo + LPT, cvb, bs_b, n2_b, zcb, z, nz);
+          un = pm::convect_level(bne[2 * (t + 1)], lo + LPT, cvn, bs_n, n2_n, zcn, z, nz);
         }
-        // bit-faithful explicit step (column.py:235-249), see pm::col_step_exact.  No level tests: at
-        // the boundary and padding levels -weff = kappa = 0 and every operand is finite, so b + dt*0 = b.
-        // BASIN: both columns (false: the northern one only); thread 0 leaves basin levels 0 and 1 to phase 2.
+        // the explicit step.  No level tests: at the boundary and padding levels -weff = kappa = 0 and every operand
+        // is finite, so b + dt*0 = b.  BASIN: both columns (false: the northern one only); thread 0 leaves basin
+        // levels 0 and 1 to phase 2.
         auto step = [&](auto UA, auto BASIN) {
           constexpr bool ua = decltype(UA)::value, basin = decltype(BASIN)::value;
           PM_UNROLL
@@ -684,22 +656,13 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
             }
             if (basin) {
               const double gb = pm::div_const(upb - bb[j], dzu[j], rdzu[j]);
-              if (j >= 2 || t != 0) {
-                const double bzz = pm::div_const(gb - gpb, dzc, rdzc[j]);
-                const double nw = nwb[s], sel = nw > 0 ? gb : gpb;
-                const double adv = pm::div_const(nw * sel, Ai_b, rAi_b);
-                bb[j] = bb[j] + dt * (adv + kb[s] * bzz);
-              } else if (j == 1) {
+              if (j >= 2 || t != 0)
+                bb[j] = pm::exact_level(bb[j], gb, gpb, dzc, rdzc[j], nwb[s], kb[s], Ai_b, rAi_b, dt);
+              else if (j == 1)
                 gb1 = gb;
-              }
               gpb = gb;
             }
-            {
-              const double bzz = pm::div_const(gn - gpn, dzc, rdzc[j]);
-              const double nw = nwn[s], sel = nw > 0 ? gn : gpn;
-              const double adv = pm::div_const(nw * sel, Ai_n, rAi_n);
-              bn[j] = bn[j] + dt * (adv + kn[s] * bzz);
-            }
+            bn[j] = pm::exact_level(bn[j], gn, gpn, dzc, rdzc[j], nwn[s], kn[s], Ai_n, rAi_n, dt);
             gpn = gn;
           }
         };
@@ -710,7 +673,6 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
           if (uniA) step(std::true_type{}, std::false_type{});
           else step(std::false_type{}, std::false_type{});
         }
-        if (!PIPE && mlw) ml_phase1(it, p);
       }
       rt::syncblock();  // SO_ML of the previous iteration is done; every neighbour value of this step has been read
       // ---------------------------------------------------------------- phase 2
@@ -718,36 +680,23 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
         // the switches as the script writes them, now that bs[0] is known
         const double bb0 = bbp[0], bb1 = bbp[1], nb0 = bne[0], nb1 = bne[2 * kWideCol], bs0 = dbox[0];
         int vb = var_b;
-        if (psi_so1 < 0) { bbot_b = bs0; vb = 1; }
-        if (res_b1 > 0 && nb0 < bb1 && nb0 < bs0) { bbot_b = nb0; vb = 1; }
-        else if (psi_so1 >= 0) { bbot_b = bb1; vb = 0; }
-        if (noise != 0 && ((noise & 1u) || ((noise & 2u) && nb0 < bb1 && nb0 < bs0) || ((noise & 4u) && bb0 < nb1)))
-          status |= PMOC_ST_NOISE_SWITCH;  // the outcome hung on the sign of a noise value
+        pm::jn_switch_basin(psi_so1, res_b1, bb1, nb0, bs0, bbot_b, vb);
+        pm::jn_noise_hit(noise, bb0, bb1, nb0, nb1, bs0, &status);
         if (M.basin.nvar < 2) vb = 0;
         if (late) {
           // the whole basin column, serially after SO_ML (the values the neighbours need are still the published ones)
           if (vb != var_b) {
             var_b = vb;
-            PM_UNROLL
-            for (int j = 0; j < LPT; ++j) {
-              const int i = lo + j, s = j * kWideCol + t;
-              if (i < nz) {
-                nwb[s] = vb ? nwb1[i] : nwb0[i];
-                kb[s] = (i >= 1 && i < nz - 1) ? kapb[(vb ? nvb : 0) + i] : 0.0;
-              }
-            }
+            load_variant(nwb, kb, nwb0, nwb1, kapb, nvb, vb);
           }
           const int* f = ibox + 8 * p;
           const bool cvb = f[0] != 0;
           const double zcb = z[f[2] >= 0 ? f[2] : 0];
-          auto adjb = [&](double v, int i) {
-            if (cvb) return v > bs_b ? bs_b + n2_b * (z[i] - zcb) : v;
-            return i == nz - 1 ? bs_b : v;
-          };
           if (t == 0) bb[0] = bbot_b;
           double gpb = 0.;
-          if (lo >= 1 && lo < nz) gpb = pm::div_const(bb[0] - adjb(bbx[lo - 1], lo - 1), dzu_m, rdzu_m);
-          const double ub = lo + LPT < nz ? adjb(bbx[lo + LPT], lo + LPT) : 0.;
+          if (lo >= 1 && lo < nz)
+            gpb = pm::div_const(bb[0] - pm::convect_level(bbx[lo - 1], lo - 1, cvb, bs_b, n2_b, zcb, z, nz), dzu_m, rdzu_m);
+          const double ub = lo + LPT < nz ? pm::convect_level(bbx[lo + LPT], lo + LPT, cvb, bs_b, n2_b, zcb, z, nz) : 0.;
           PM_UNROLL
           for (int j = 0; j < LPT; ++j) {
             const int s = j * kWideCol + t;
@@ -755,10 +704,9 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
             const double gb = pm::div_const(upb - bb[j], dzu[j], rdzu[j]);
             const double dzc = 0.5 * (dzu[j] + (j > 0 ? dzu[j > 0 ? j - 1 : 0] : dzu_m));
             const int i = lo + j < nz ? lo + j : nz - 1;
-            const double bzz = pm::div_const(gb - gpb, dzc, rdzc[j]);
-            const double nw = nwb[s], sel = nw > 0 ? gb : gpb;
-            const double adv = pm::div_const(nw * sel, uniA ? A_b : Ab[i], uniA ? rA_b : rab[i]);
-            bb[j] = bb[j] + dt * (adv + kb[s] * bzz);
+            // (the Area as a value: bound to a reference, the select would let the compiler read Ab[i] unconditionally)
+            bb[j] = pm::exact_level(bb[j], gb, gpb, dzc, rdzc[j], nwb[s], kb[s], double(uniA ? A_b : Ab[i]),
+                                    double(uniA ? rA_b : rab[i]), dt);
             gpb = gb;
           }
         } else if (t == 0) {
@@ -766,18 +714,16 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
           bb[0] = bbot_b;
           const double g0 = pm::div_const(bb[1] - bb[0], dzu[0], rdzu[0]);
           const double dzc = 0.5 * (dzu[1] + dzu[0]);
-          const double bzz = pm::div_const(gb1 - g0, dzc, rdzc[1]);
           const int s = 1 * kWideCol + 0;
-          const double nw = nwb[s], sel = nw > 0 ? gb1 : g0;
-          const double adv = pm::div_const(nw * sel, uniA ? A_b : Ab[1], uniA ? rA_b : rab[1]);
-          bb[1] = bb[1] + dt * (adv + kb[s] * bzz);
+          bb[1] = pm::exact_level(bb[1], gb1, g0, dzc, rdzc[1], nwb[s], kb[s], double(uniA ? A_b : Ab[1]),
+                                  double(uniA ? rA_b : rab[1]), dt);
         }
       }
       if (late) rt::syncblock();  // the serial basin step read the published neighbour values: only now overwrite them
       if (col) publish(p ^ 1);
       rt::syncblock();
     }
-    if (mlw && a.nsteps > 0) ml_one(p);  // SO_ML of the last iteration
+    if (mlw && a.nsteps > 0) ml_published(ml, p);  // SO_ML of the last iteration
     rt::syncblock();
 
   } else {
@@ -785,56 +731,34 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
     // barrier) -- the deferral logic of the pipelined form costs registers this variant does not have
     for (long long it = 0; it < a.nsteps; ++it, p ^= 1) {
       if (col) {
-        // bottom boundary condition and bottom-boundary-layer kappa (run_JansenNadeau_2018.py:233-254);
-        // every thread evaluates the switches from the published values
+        // bottom boundary condition and bottom-boundary-layer kappa; every thread evaluates the switches from the
+        // published values
         const double bb0 = bbp[0], bb1 = bbp[1], nb0 = bne[0], nb1 = bne[2 * kWideCol], bs0 = dbox[0];
         int vb = var_b, vn = var_n;
-        if (psi_so1 < 0) { bbot_b = bs0; vb = 1; }
-        if (res_b1 > 0 && nb0 < bb1 && nb0 < bs0) { bbot_b = nb0; vb = 1; }
-        else if (psi_so1 >= 0) { bbot_b = bb1; vb = 0; }
-        if (res_n1 < 0 && bb0 < nb1) { bbot_n = bb0; vn = 1; }
-        else { bbot_n = nb1; vn = 0; }
-        if (noise != 0 && ((noise & 1u) || ((noise & 2u) && nb0 < bb1 && nb0 < bs0) || ((noise & 4u) && bb0 < nb1)))
-          status |= PMOC_ST_NOISE_SWITCH;  // the outcome hung on the sign of a noise value
+        pm::jn_switch_basin(psi_so1, res_b1, bb1, nb0, bs0, bbot_b, vb);
+        pm::jn_switch_north(res_n1, bb0, nb1, bbot_n, vn);
+        pm::jn_noise_hit(noise, bb0, bb1, nb0, nb1, bs0, &status);
         if (M.basin.nvar < 2) vb = 0;
         if (M.north.nvar < 2) vn = 0;
-        if (vb != var_b) {  // the owner re-reads its levels of the other variant
+        if (vb != var_b) {
           var_b = vb;
-          PM_UNROLL
-          for (int j = 0; j < LPT; ++j) {
-            const int i = lo + j, s = j * kWideCol + t;
-            if (i < nz) {
-              nwb[s] = vb ? nwb1[i] : nwb0[i];
-              kb[s] = (i >= 1 && i < nz - 1) ? kapb[(vb ? nvb : 0) + i] : 0.0;
-            }
-          }
+          load_variant(nwb, kb, nwb0, nwb1, kapb, nvb, vb);
         }
         if (vn != var_n) {
           var_n = vn;
-          PM_UNROLL
-          for (int j = 0; j < LPT; ++j) {
-            const int i = lo + j, s = j * kWideCol + t;
-            if (i < nz) {
-              nwn[s] = vn ? nwn1[i] : nwn0[i];
-              kn[s] = (i >= 1 && i < nz - 1) ? kapn[(vn ? nvn : 0) + i] : 0.0;
-            }
-          }
+          load_variant(nwn, kn, nwn0, nwn1, kapn, nvn, vn);
         }
-        // convective adjustment (column.py:264-271) of the own levels and of the two neighbour values
+        // convective adjustment of the own levels and of the two neighbour values
         const int* f = ibox + 8 * p;
         const bool cvb = f[0] != 0, cvn = f[1] != 0;
         const double zcb = z[f[2] >= 0 ? f[2] : 0], zcn = z[f[3] >= 0 ? f[3] : 0];
-        auto adj = [&](double v, int i, bool cv, double bs, double n2, double zc) {
-          if (cv) return v > bs ? bs + n2 * (z[i] - zc) : v;
-          return i == nz - 1 ? bs : v;
-        };
         if ((cvb && mine_b) || (cvn && mine_n) || owns_top) {
           PM_UNROLL
           for (int j = 0; j < LPT; ++j) {
             const int i = lo + j;
             if (i < nz) {
-              bb[j] = adj(bb[j], i, cvb, bs_b, n2_b, zcb);
-              bn[j] = adj(bn[j], i, cvn, bs_n, n2_n, zcn);
+              bb[j] = pm::convect_level(bb[j], i, cvb, bs_b, n2_b, zcb, z, nz);
+              bn[j] = pm::convect_level(bn[j], i, cvn, bs_n, n2_n, zcn, z, nz);
             }
           }
         }
@@ -844,18 +768,18 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
         }
         double gpb = 0., gpn = 0.;  // gradient of the cell below the current level
         if (lo >= 1 && lo < nz) {
-          const double vb_ = adj(bbx[lo - 1], lo - 1, cvb, bs_b, n2_b, zcb);
-          const double vn_ = adj(bne[2 * (t - 1) + 1], lo - 1, cvn, bs_n, n2_n, zcn);
+          const double vb_ = pm::convect_level(bbx[lo - 1], lo - 1, cvb, bs_b, n2_b, zcb, z, nz);
+          const double vn_ = pm::convect_level(bne[2 * (t - 1) + 1], lo - 1, cvn, bs_n, n2_n, zcn, z, nz);
           gpb = pm::div_const(bb[0] - vb_, dzu_m, rdzu_m);
           gpn = pm::div_const(bn[0] - vn_, dzu_m, rdzu_m);
         }
         double ub = 0., un = 0.;  // level above the thread's last one
         if (lo + LPT < nz) {
-          ub = adj(bbx[lo + LPT], lo + LPT, cvb, bs_b, n2_b, zcb);
-          un = adj(bne[2 * (t + 1)], lo + LPT, cvn, bs_n, n2_n, zcn);
+          ub = pm::convect_level(bbx[lo + LPT], lo + LPT, cvb, bs_b, n2_b, zcb, z, nz);
+          un = pm::convect_level(bne[2 * (t + 1)], lo + LPT, cvn, bs_n, n2_n, zcn, z, nz);
         }
-        // bit-faithful explicit step (column.py:235-249), see pm::col_step_exact.  No level tests: at
-        // the boundary and padding levels -weff = kappa = 0 and every operand is finite, so b + dt*0 = b.
+        // the explicit step.  No level tests: at the boundary and padding levels -weff = kappa = 0 and every operand
+        // is finite, so b + dt*0 = b.
         auto step = [&](auto UA) {
           constexpr bool ua = decltype(UA)::value;
           PM_UNROLL
@@ -871,18 +795,8 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
               const int i = lo + j < nz ? lo + j : nz - 1;
               Ai_b = Ab[i]; rAi_b = rab[i]; Ai_n = An[i]; rAi_n = ran[i];
             }
-            {
-              const double bzz = pm::div_const(gb - gpb, dzc, rdzc[j]);
-              const double nw = nwb[s], sel = nw > 0 ? gb : gpb;
-              const double adv = pm::div_const(nw * sel, Ai_b, rAi_b);
-              bb[j] = bb[j] + dt * (adv + kb[s] * bzz);
-            }
-            {
-              const double bzz = pm::div_const(gn - gpn, dzc, rdzc[j]);
-              const double nw = nwn[s], sel = nw > 0 ? gn : gpn;
-              const double adv = pm::div_const(nw * sel, Ai_n, rAi_n);
-              bn[j] = bn[j] + dt * (adv + kn[s] * bzz);
-            }
+            bb[j] = pm::exact_level(bb[j], gb, gpb, dzc, rdzc[j], nwb[s], kb[s], Ai_b, rAi_b, dt);
+            bn[j] = pm::exact_level(bn[j], gn, gpn, dzc, rdzc[j], nwn[s], kn[s], Ai_n, rAi_n, dt);
             gpb = gb;
             gpn = gn;
           }
@@ -896,18 +810,12 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
       publish(p ^ 1);
       rt::syncblock();
       if (mlw) {
-        // b_basin sorted?  inside the threads and warps: flagged by publish; across the warps: here
-        bool bad = ibox[8 * (p ^ 1) + 4] != 0;
-        const int e = (Ln + 1) * 32 * LPT;  // first level of the next warp
-        if (Ln < kWideCol / 32 - 1 && e < nz) bad |= !(bbx[e] >= bbx[e - 1]);
-        const bool sorted = rt::ballot(bad) == 0;
         pm::MlState ml;
         pm::ml_unpark(ml, mlp, scan_s);
-        pm::ml_step(ml, bbx, pm_s, nz, sorted, bs_s, dt, &status);
+        ml_published(ml, p ^ 1);
         pm::ml_park(ml, mlp, false);
-        if (Ln == 0) {
-          dbox[0] = ml.bs[0];
-          int* f = ibox + 8 * p;  // read during this step; refilled by the publish of the next one
+        if (Ln == 0) {  // read during this step; refilled by the publish of the next one
+          int* f = ibox + 8 * p;
           f[0] = 0; f[1] = 0; f[2] = -1; f[3] = -1; f[4] = 0;
         }
       }
@@ -947,7 +855,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
     if (M.north.var) M.north.var[m] = var_n;
   }
   const unsigned all = block_or(status, cbox);  // the mixed-layer warp carries SO_ML's bits
-  if (t == 0 && M.status) M.status[m] = (M.status[m] | all) & ~(so1_exact ? 0u : PMOC_ST_CARRY_SO1_EXACT);
+  if (t == 0 && M.status) M.status[m] = status_word(M.status[m], all, so1_exact);
 }
 
 // ---- the steps of the 'post' order (example_twocol_plusSO.py:99-115) ----------------------------
@@ -1082,27 +990,25 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol, LPT == 4 ? 2 : 1) k_wide_post(WideArgs
     const int qw = qr == 2 ? 0 : qr + 1, qz = qw == 2 ? 0 : qw + 1;
     PM_UNROLL
     for (int c = 0; c < NCOL; ++c) {
-      // convective adjustment (column.py:264-271) or the surface value (column.py:230-231) of the own levels and
-      // of the two neighbour values, then the bottom condition (column.py:232-233)
+      // convective adjustment or the surface value (column.py:230-231) of the own levels and of the two neighbour
+      // values, then the bottom condition (column.py:232-233)
       const int* f = flg + (qr * NCOL + c) * 2;
       const bool cv = conv[c] && f[0] != 0;
       const double zc = z[f[1] >= 0 ? f[1] : 0], bsc = bs[c], n2c = n2[c];
-      auto adj = [&](double v, int i) {
-        if (cv) return v > bsc ? bsc + n2c * (z[i] - zc) : v;
-        return i == nz - 1 ? bsc : v;
-      };
       if ((cv && mine[c]) || owns_top) {
         PM_UNROLL
         for (int j = 0; j < LPT; ++j)
-          if (lo + j < nz) b[c][j] = adj(b[c][j], lo + j);
+          if (lo + j < nz) b[c][j] = pm::convect_level(b[c][j], lo + j, cv, bsc, n2c, zc, z, nz);
       }
       if (t == 0) b[c][0] = hasz[c] ? b[c][1] - bzbot[c] * dzu[0] : bbot[c];
       const double* ed = edge + (e * NCOL + c) * 2 * kWideCol;
       double gp = 0.;  // gradient of the cell below the current level
-      if (lo >= 1 && lo < nz) gp = pm::div_const(b[c][0] - adj(ed[2 * t - 1], lo - 1), dzu_m, rdzu_m);
-      const double ub = lo + LPT < nz ? adj(ed[2 * t + 2], lo + LPT) : 0.;  // level above the thread's last one
-      // bit-faithful explicit step (column.py:235-249), see pm::col_step_exact.  No level tests: at the boundary
-      // and padding levels -weff = kappa = 0 and every operand is finite, so b + dt*0 = b.
+      if (lo >= 1 && lo < nz)
+        gp = pm::div_const(b[c][0] - pm::convect_level(ed[2 * t - 1], lo - 1, cv, bsc, n2c, zc, z, nz), dzu_m, rdzu_m);
+      // level above the thread's last one
+      const double ub = lo + LPT < nz ? pm::convect_level(ed[2 * t + 2], lo + LPT, cv, bsc, n2c, zc, z, nz) : 0.;
+      // the explicit step.  No level tests: at the boundary and padding levels -weff = kappa = 0 and every operand
+      // is finite, so b + dt*0 = b.
       const double* nw = nws + c * nzp;
       const double* kp = kps + c * nzp;
       auto step = [&](auto UA) {
@@ -1113,16 +1019,9 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol, LPT == 4 ? 2 : 1) k_wide_post(WideArgs
           const double up = j + 1 < LPT ? b[c][j + 1 < LPT ? j + 1 : j] : ub;
           const double g = pm::div_const(up - b[c][j], dzu[j], rdzu[j]);
           const double dzc = 0.5 * (dzu[j] + (j > 0 ? dzu[j > 0 ? j - 1 : 0] : dzu_m));
-          const double bzz = pm::div_const(g - gp, dzc, rdzc[j]);
-          const double nwv = nw[s], sel = nwv > 0 ? g : gp;
-          double Ai = A1[c], rAi = rA1[c];
-          if (!ua) {
-            const int i = lo + j < nz ? lo + j : nz - 1;
-            Ai = Ar[c][i];
-            rAi = rarea[c * nz + i];
-          }
-          const double adv = pm::div_const(nwv * sel, Ai, rAi);
-          b[c][j] = b[c][j] + dt * (adv + kp[s] * bzz);
+          const int i = lo + j < nz ? lo + j : nz - 1;
+          b[c][j] = pm::exact_level(b[c][j], g, gp, dzc, rdzc[j], nw[s], kp[s], ua ? A1[c] : Ar[c][i],
+                                    ua ? rA1[c] : rarea[c * nz + i], dt);
           gp = g;
         }
       };

@@ -199,6 +199,31 @@ int pmoc_model_diagnose(const pmoc_model* m, void* stream);
  * run_single_global_basin.py:172-229. */
 int pmoc_model_run(const pmoc_model* m, int64_t it0, int64_t nsteps, void* stream);
 
+/* pmoc_model_run for the listed members only (device list of indices in [0, M), any order, no repeats); the others
+ * are untouched.
+ * Each listed member ends exactly as pmoc_model_run would leave it -- state, carried streamfunctions, diagnostics
+ * and status -- and the state stays in place (nothing is gathered).  n == 0 launches nothing. */
+int pmoc_model_run_members(const pmoc_model* m, const int64_t* members, int64_t n, int64_t it0, int64_t nsteps,
+                           void* stream);
+
+/* Run [it0, it0 + max_steps) to equilibrium: in chunks of `every` iterations (a multiple of K; max_steps a multiple
+ * of K too, else PMOC_EINVAL), after each chunk freeze the members whose state moved by <= tol since the previous
+ * check -- |b_now - b_prev| <= tol at every level of every column and, with PMOC_HAS_ML, at every point of the mixed
+ * layer's bs -- and step only the others.  A member with a non-finite value is frozen as not converged.  The last
+ * chunk may be shorter than `every`.
+ *   stopped_at[M] (device): the iteration each member stopped at (it0 + max_steps when it never stopped);
+ *   converged[M] (device, uint8): 1 if the criterion was met, 0 if non-finite or still moving at the end.
+ * A member frozen at iteration n holds exactly what pmoc_model_run over [it0, n) gives it.  The loop reads the
+ * iteration counter only modulo K and every stop is it0 plus a multiple of K, so after the call all members can be
+ * run on together from it0 + max_steps: each continues from its own stop.  An order-'post' model must have been
+ * diagnosed, as for pmoc_model_run.
+ * `work`: caller-provided device memory of pmoc_equilibrate_work_bytes(m) bytes (the snapshot of the state, two
+ * active lists, a counter).  The library allocates nothing; the host reads the 8-byte counter back after every
+ * check (one copy and one stream synchronisation), so the call returns when the work is done. */
+uint64_t pmoc_equilibrate_work_bytes(const pmoc_model* m);
+int pmoc_model_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                           int64_t* stopped_at, uint8_t* converged, void* work, uint64_t work_bytes, void* stream);
+
 /* Same as diagnose (when it0 == 0, order 'post') + run, but every pointer in `m` is a HOST pointer: the
  * stateless form of the handle below (open, one step, close), with the same device mirror and block loop.
  * Grids, parameters and the state (PMOC_IO_STATE) go up every call, the carried streamfunctions

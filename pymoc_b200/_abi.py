@@ -63,7 +63,8 @@ class Model(C.Structure):
 
 EXPORTS = ('pmoc_abi_version', 'pmoc_last_error', 'pmoc_device_info', 'pmoc_model_scratch_bytes', 'pmoc_model_diagnose', 'pmoc_model_run',
            'pmoc_model_run_host', 'pmoc_host_last_bytes', 'pmoc_host_open', 'pmoc_host_step', 'pmoc_host_close', 'pmoc_column_timestep', 'pmoc_thermwind_solve', 'pmoc_thermwind_psib',
-           'pmoc_so_solve', 'pmoc_ml_timestep', 'pmoc_fp64_peak')
+           'pmoc_so_solve', 'pmoc_ml_timestep', 'pmoc_fp64_peak', 'pmoc_model_run_members', 'pmoc_equilibrate_work_bytes',
+           'pmoc_model_equilibrate')
 
 
 def declare(lib):
@@ -92,10 +93,15 @@ def declare(lib):
                                 C.c_void_p]
   lib.pmoc_ml_timestep.argtypes = [P(Model), Vec, Vec, C.c_double, C.c_void_p, C.c_void_p]
   lib.pmoc_fp64_peak.argtypes = [P(C.c_double), P(C.c_double), C.c_void_p]
+  lib.pmoc_model_run_members.argtypes = [P(Model), C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]
+  lib.pmoc_equilibrate_work_bytes.argtypes = [P(Model)]
+  lib.pmoc_model_equilibrate.argtypes = [P(Model), C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_uint64, C.c_void_p]
   for name in EXPORTS:
-    if name not in ('pmoc_last_error', 'pmoc_model_scratch_bytes', 'pmoc_host_last_bytes'):
+    if name not in ('pmoc_last_error', 'pmoc_model_scratch_bytes', 'pmoc_host_last_bytes', 'pmoc_equilibrate_work_bytes'):
       getattr(lib, name).restype = C.c_int
   lib.pmoc_model_scratch_bytes.restype = C.c_uint64
+  lib.pmoc_equilibrate_work_bytes.restype = C.c_uint64
   if lib.pmoc_abi_version() != ABI_VERSION:
     raise RuntimeError('pymoc_b200: ABI version mismatch (library %d, python %d)' %
                        (lib.pmoc_abi_version(), ABI_VERSION))

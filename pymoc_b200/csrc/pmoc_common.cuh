@@ -136,12 +136,21 @@ PM_DEV pm::ExactCol exactcol_of(double* ws, const SmemPlan& sp, int which) {
   return pm::ExactCol{{t, t + sp.nzp}, t + 2 * sp.nzp, t + 3 * sp.nzp, {n, n + sp.nzp}};
 }
 
+// Active list of a launch (pmoc_model_run_members): slot s steps member members[s], in place; NULL = every member,
+// slot s = member s.  Every kernel reads and writes through the real member index, so nothing is gathered.
+struct MemberList {
+  const int64_t* members;
+  long long n;
+  PM_HD long long slots(long long M) const { return members ? n : M; }
+};
+
 struct RunArgs {
   pmoc_model m;
   SmemPlan sp;
   long long it0, nsteps;
   int diagnose_only;
   int sync_refresh;  // CTA barrier before every diagnosis: the CTA's warps then run its long instruction stream together
+  MemberList list;
 };
 
 // per-column registers
@@ -248,15 +257,20 @@ PM_DEV bool so1_exact_carried(const pmoc_model& M, long long m) {
 PM_DEV unsigned status_word(unsigned old, unsigned bits, bool carry) {
   return ((old | bits) & ~PMOC_ST_CARRY_MASK) | (carry ? PMOC_ST_CARRY_SO1_EXACT : 0u);
 }
+
+// the checks pmoc_model_run applies to a model before it dispatches (pmoc_ops.cu)
+int check_model(const pmoc_model* m);
 }  // namespace pmk
 using namespace pmk;
 
 // block-per-member path for nz > PMOC_MAX_NZ_WARP (pmoc_wide.cu)
-int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream);
+int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream,
+                        pmk::MemberList list);
 
 // several members per warp for the column + thermal-wind topology (pmoc_twcol.cu)
 bool pmoc_twcol_supported(const pmoc_model* m);
-int pmoc_launch_twcol(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream);
+int pmoc_launch_twcol(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream,
+                      pmk::MemberList list);
 
 // one launcher per levels-per-lane, each in its own translation unit (pmoc_model.cu)
 #define PM_DECL_MODEL(n) int pmoc_launch_model_##n(const RunArgs& ra, void* stream);

@@ -34,7 +34,9 @@ constexpr int max_warps(unsigned topo) {
                               : (((topo & PMOC_HAS_NORTH) && !(topo & PMOC_SO_BVP)) ? PM_WARPS_MULTI : PM_WARPS_SINGLE);
 }
 
-template <int LPL, unsigned TOPO>
+// LIST: launched over an active list (a.list.members != NULL).  A separate instantiation, so that the plain launch
+// compiles to the same code it had without lists (the member index stays a function of the grid position).
+template <int LPL, unsigned TOPO, bool LIST>
 PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
   constexpr bool NORTH = (TOPO & PMOC_HAS_NORTH) != 0, TW = (TOPO & PMOC_HAS_TW) != 0;
   constexpr bool ISO = (TOPO & PMOC_ISO) != 0, SO = (TOPO & PMOC_HAS_SO) != 0;
@@ -61,8 +63,9 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
   rt::syncblock();
   const pm::GeoTab G = geo_of(sm, sp);
   const double* zs = G.zs;
-  const long long m = rt::block_idx() * rt::warps_per_block() + W;
-  if (m >= M.M) return;
+  const long long slot = rt::block_idx() * rt::warps_per_block() + W;
+  if (slot >= (LIST ? a.list.n : M.M)) return;
+  const long long m = LIST ? a.list.members[slot] : slot;
   const double dt = M.dt;
 
   ColRegs<LPL> cb, cn, cp;
@@ -329,7 +332,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(32 * max_warps(TOPO), 1) k_model(RunArgs a) {
   for (;;) {
     if (refresh_next) {
 #ifndef PMOC_EMU
-      if (a.sync_refresh) __syncthreads();  // (warps of members beyond M have exited: they do not count)
+      if (a.sync_refresh) __syncthreads();  // (warps past the last slot have exited: they do not count)
 #endif
       refresh(wr);
       refresh_next = false;
@@ -444,7 +447,7 @@ int launch_model(const RunArgs& ra, void* stream) {
     const int w = std::atoi(e);
     if (w >= 1 && w <= cap && resident(w) > 0) wpb = w;
   }
-  const long long grid = (ra.m.M + wpb - 1) / wpb;
+  const long long grid = (ra.list.slots(ra.m.M) + wpb - 1) / wpb;
   const int block = 32 * wpb;
   const size_t smem = ra.sp.bytes(wpb);
   // A CTA barrier in front of every diagnosis re-aligns the CTA's warps, which then walk its ~9 000-instruction
@@ -454,8 +457,10 @@ int launch_model(const RunArgs& ra, void* stream) {
   RunArgs ra2 = ra;
   ra2.sync_refresh = (t & PMOC_ISO) != 0;
   if (const char* e = std::getenv("PMOC_REFRESH_SYNC")) ra2.sync_refresh = std::atoi(e);
-#define PM_CASE(T) \
-  case (T): return launch(k_model<LPL, (T)>, grid, block, smem, stream, ra2);
+#define PM_CASE(T)                                                                      \
+  case (T):                                                                             \
+    return ra.list.members ? launch(k_model<LPL, (T), true>, grid, block, smem, stream, ra2) \
+                           : launch(k_model<LPL, (T), false>, grid, block, smem, stream, ra2);
   switch (t) {
     PM_CASE(PMOC_HAS_TW)
     PM_CASE(PMOC_HAS_SO)

@@ -291,12 +291,14 @@ int check_model(const pmoc_model* m) {
   return PMOC_OK;
 }
 
-int run_model(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream) {
+int run_model(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream,
+              MemberList list = MemberList{nullptr, 0}) {
   if (int rc = check_model(m)) return rc;
   if (nsteps < 0 || it0 < 0) return fail(PMOC_EINVAL, "negative it0 / nsteps");
   if (!diagnose_only && nsteps == 0) return PMOC_OK;
-  if (m->nz > PMOC_MAX_NZ_WARP) return pmoc_run_model_wide(m, it0, nsteps, diagnose_only, stream);
-  if (pmoc_twcol_supported(m) && !std::getenv("PMOC_NO_TWCOL")) return pmoc_launch_twcol(m, it0, nsteps, diagnose_only, stream);
+  if (m->nz > PMOC_MAX_NZ_WARP) return pmoc_run_model_wide(m, it0, nsteps, diagnose_only, stream, list);
+  if (pmoc_twcol_supported(m) && !std::getenv("PMOC_NO_TWCOL"))
+    return pmoc_launch_twcol(m, it0, nsteps, diagnose_only, stream, list);
   RunArgs ra;
   ra.m = *m;
   ra.m.flags &= ~PMOC_SO_BVP;
@@ -305,6 +307,7 @@ int run_model(const pmoc_model* m, long long it0, long long nsteps, int diagnose
   ra.nsteps = nsteps;
   ra.diagnose_only = diagnose_only;
   ra.sync_refresh = 0;
+  ra.list = list;
   const int lpl = lpl_for(m->nz);
   ra.sp = plan_smem(lpl, m->ny, m->nb, ra.m.flags);
   switch (lpl) {
@@ -354,6 +357,14 @@ int pmoc_model_diagnose(const pmoc_model* m, void* stream) { return run_model(m,
 
 int pmoc_model_run(const pmoc_model* m, int64_t it0, int64_t nsteps, void* stream) {
   return run_model(m, it0, nsteps, 0, stream);
+}
+
+int pmoc_model_run_members(const pmoc_model* m, const int64_t* members, int64_t n, int64_t it0, int64_t nsteps,
+                           void* stream) {
+  if (m && (n < 0 || n > m->M)) return fail(PMOC_EINVAL, "member count outside [0, M]");
+  if (n > 0 && !members) return fail(PMOC_EINVAL, "member list is NULL");
+  if (n == 0 && nsteps > 0) nsteps = 0;  // an empty list validates the model and launches nothing
+  return run_model(m, it0, nsteps, 0, stream, MemberList{members, n});
 }
 
 int pmoc_column_timestep(int64_t M, int32_t nz, const double* z, const pmoc_column* col, pmoc_vec wA, pmoc_vec vdx_in,
@@ -432,3 +443,7 @@ int pmoc_ml_timestep(const pmoc_model* ml, pmoc_vec b_basin, pmoc_vec Psi_b, dou
 }
 
 }  // extern "C"
+
+// Runs to equilibrium (pmoc_model_equilibrate, pmoc_equilibrate_work_bytes) extend the C ABI of this unit and are
+// compiled with it.
+#include "pmoc_equil.cu"

@@ -20,9 +20,11 @@ struct TwColArgs {
   pmoc_model m;
   long long it0, nsteps;
   int diagnose_only;
+  MemberList list;
 };
 
-template <int G, int LPL>
+// LIST: launched over an active list (a.list.members != NULL); the plain launch compiles without its extra path
+template <int G, int LPL, bool LIST>
 PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
   constexpr int MPW = 32 / G;   // members per warp
   constexpr int NL = G * LPL;   // level slots of a member
@@ -51,10 +53,12 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
     }
   }
   rt::syncblock();
-  const long long m_raw = (rt::block_idx() * rt::warps_per_block() + W) * MPW + grp;
-  const bool live = m_raw < M.M;
-  const long long m = live ? m_raw : M.M - 1;  // (groups past the end shadow the last member and store nothing)
+  const long long s_raw = (rt::block_idx() * rt::warps_per_block() + W) * MPW + grp, ns = LIST ? a.list.n : M.M;
+  const bool live = s_raw < ns;
+  const long long slot = live ? s_raw : ns - 1;  // (groups past the end shadow the last slot and store nothing)
+  const long long m = LIST ? a.list.members[slot] : slot;
   if (rt::ballot(live) == 0) return;
+  auto group_mask = [&]() { return (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (grp * G); };
   // per-member tables (slot j*G + s): the four stream-function independent products of the folded stencil, d(A kappa)/dz
   double* mt = sm + 9 * NL + (size_t)(W * MPW + grp) * 5 * NL;
   double *m_pk = mt, *m_qk = mt + NL, *m_pa = mt + 2 * NL, *m_qa = mt + 3 * NL, *m_dak = mt + 4 * NL;
@@ -86,19 +90,36 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
   // table words per step instead of ten (the kernel is otherwise bound by shared-memory reads: ncu
   // short_scoreboard 2.2 warps per issue cycle).  Decided per warp; anything else takes the tabulated path.
   const double h0 = M.z[1] - M.z[0];
-  bool odd = false;
-  {
-    const double* area = vrow(M.basin.Area, m);
+  auto odd_of = [&](long long mm) {  // this lane's levels of member mm break the uniform path
+    const double* area = vrow(M.basin.Area, mm);
+    bool odd = false;
     PM_UNROLL
     for (int j = 0; j < LPL; ++j) {
       const int i = s * LPL + j;
       if (i < nz - 1) odd |= !(fabs(t_h[j * G + s] - h0) <= 1e-13 * fabs(h0));
       if (i >= 1 && i < nz - 1) odd |= area[i] != area[1];
     }
+    return odd;
+  };
+  // The two paths round differently, so with an active list a member takes the decision of its home warp in a run
+  // of every member (members m - m % MPW ... + MPW - 1, the last member standing in past the end): each group
+  // re-checks those members.  Groups of one warp that then disagree run both paths and keep their own (`mixed`).
+  bool fast, mine = true, mixed = false;
+  if (!LIST) {
+    fast = rt::ballot(odd_of(m)) == 0 && nz >= 3;
+  } else {
+    bool odd = false;
+    for (int q = 0; q < MPW; ++q) {
+      const long long mm = m - m % MPW + q;
+      odd |= odd_of(mm < M.M ? mm : M.M - 1);
+    }
+    mine = (rt::ballot(odd) & group_mask()) == 0 && nz >= 3;
+    const unsigned all = rt::ballot(mine);
+    fast = all == 0xffffffffu;
+    mixed = all != 0 && !fast;
   }
-  const bool fast = rt::ballot(odd) == 0 && nz >= 3;
   const double u_hh = 0.5 * h0, u_a = h0 * h0 / 3., u_c = h0 * h0 / 6., u_rn = 1.0 / (double)(nz - 1);
-  const double u_pa = fast ? (dt / vrow(M.basin.Area, m)[1]) / h0 : 0.0;
+  const double u_pa = fast || (LIST && mixed) ? (dt / vrow(M.basin.Area, m)[1]) / h0 : 0.0;
 
   // folded stencil coefficients from the streamfunction in Sv (column.py:241-248, see pm::col_coeffs)
   auto coeffs_as = [&](const double(&psi)[LPL], auto FAST) {
@@ -120,8 +141,22 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
     }
   };
   auto coeffs = [&](const double(&psi)[LPL]) {
-    if (fast) coeffs_as(psi, std::true_type{});
-    else coeffs_as(psi, std::false_type{});
+    if (fast) {
+      coeffs_as(psi, std::true_type{});
+    } else if (!LIST || !mixed) {
+      coeffs_as(psi, std::false_type{});
+    } else {
+      double ps[LPL], qs[LPL];
+      coeffs_as(psi, std::false_type{});
+      PM_UNROLL
+      for (int j = 0; j < LPL; ++j) { ps[j] = p[j]; qs[j] = q[j]; }
+      coeffs_as(psi, std::true_type{});
+      PM_UNROLL
+      for (int j = 0; j < LPL; ++j) {
+        p[j] = mine ? p[j] : ps[j];
+        q[j] = mine ? q[j] : qs[j];
+      }
+    }
   };
   // Psi_Thermwind.solve for the current state
   auto solve_as = [&](double(&psi)[LPL], auto FAST) {
@@ -183,8 +218,17 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
     }
   };
   auto solve = [&](double(&psi)[LPL]) {
-    if (fast) solve_as(psi, std::true_type{});
-    else solve_as(psi, std::false_type{});
+    if (fast) {
+      solve_as(psi, std::true_type{});
+    } else if (!LIST || !mixed) {
+      solve_as(psi, std::false_type{});
+    } else {  // (the scans stay inside the G-lane groups: both paths are warp-uniform)
+      double pf[LPL];
+      solve_as(psi, std::false_type{});
+      solve_as(pf, std::true_type{});
+      PM_UNROLL
+      for (int j = 0; j < LPL; ++j) psi[j] = mine ? pf[j] : psi[j];
+    }
   };
   auto store_psi = [&](const double(&psi)[LPL]) {
     if (!live) return;
@@ -246,7 +290,7 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
   }
   // NaN flag per member: any lane of the group
   unsigned any = rt::ballot(bad);
-  const unsigned gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (grp * G);
+  const unsigned gmask = group_mask();
   if (live && s == 0 && M.status) M.status[m] |= (any & gmask) ? PMOC_ST_NAN : 0u;
 }
 
@@ -254,9 +298,10 @@ template <int G, int LPL>
 static int launch_twcol(const TwColArgs& a, void* stream) {
   constexpr int wpb = 4, MPW = 32 / G, NL = G * LPL;
   const long long per_block = (long long)wpb * MPW;
-  const long long grid = (a.m.M + per_block - 1) / per_block;
+  const long long grid = (a.list.slots(a.m.M) + per_block - 1) / per_block;
   const size_t smem = sizeof(double) * (size_t)(9 * NL + wpb * MPW * 5 * NL);
-  return launch(k_twcol<G, LPL>, grid, 32 * wpb, smem, stream, a);
+  if (a.list.members) return launch(k_twcol<G, LPL, true>, grid, 32 * wpb, smem, stream, a);
+  return launch(k_twcol<G, LPL, false>, grid, 32 * wpb, smem, stream, a);
 }
 
 }  // namespace pmk
@@ -268,12 +313,14 @@ bool pmoc_twcol_supported(const pmoc_model* m) {
          m->tw_b2.ptr && m->Psi_tw;
 }
 
-int pmoc_launch_twcol(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream) {
+int pmoc_launch_twcol(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream,
+                      pmk::MemberList list) {
   pmk::TwColArgs a;
   a.m = *m;
   a.it0 = it0;
   a.nsteps = nsteps;
   a.diagnose_only = diagnose_only;
+  a.list = list;
   const int nz = m->nz;
 #define PM_TWCOL(G, N) if (nz <= (G) * (N)) return pmk::launch_twcol<G, N>(a, stream);
   PM_TWCOL(8, 3) PM_TWCOL(8, 5) PM_TWCOL(8, 7) PM_TWCOL(8, 9) PM_TWCOL(16, 6) PM_TWCOL(16, 7) PM_TWCOL(16, 8) PM_TWCOL(16, 9)

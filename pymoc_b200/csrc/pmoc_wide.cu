@@ -26,9 +26,16 @@ struct WideArgs {
   double* geo;   // scratch: [4][nz] dzu, 1/dzu, dzc, 1/dzc (shared by all members)
   double* memb;  // scratch: per member [6][nz]: -weff basin v0, v1, -weff north v0, v1, 1/Area basin, 1/Area north
   int force_late;  // test hook (PMOC_WIDE_FORCE_LATE=1): always take the serial schedule of the basin column
+  MemberList list;
 };
 
 PM_DEV int wtid() { return rt::warp_in_block() * 32 + rt::lane(); }
+// The member of this CTA (one CTA per slot of the active list).  LIST (a.list.members != NULL) is a template
+// parameter of the kernels, so that a plain launch compiles to the code it had without lists.
+template <bool LIST>
+PM_DEV long long wide_member(const WideArgs& a) {
+  return LIST ? a.list.members[rt::block_idx()] : rt::block_idx();
+}
 PM_DEV int wnthr() { return rt::warps_per_block() * 32; }
 
 // ---- small block collectives on shared memory ------------------------------------------------
@@ -114,12 +121,13 @@ PM_GLOBAL void k_wide_geo(WideArgs a) {
 // register chunks).  The parts follow the model's flags: the thermal wind against the northern column
 // or the fixed profile tw_b2, the remap only with PMOC_ISO, Psi_SO on the mixed layer's bs ('jn') or on
 // so_bs ('post').  The carry bit of the 'jn' switches (PMOC_ST_CARRY_SO1_EXACT) is 'jn' only.
+template <bool LIST>
 PM_GLOBAL void k_wide_refresh(WideArgs a) {
   const pmoc_model& M = a.m;
   const bool JN = (M.flags & PMOC_ORDER_JN) != 0, NORTH = (M.flags & PMOC_HAS_NORTH) != 0;
   const bool TW = (M.flags & PMOC_HAS_TW) != 0, ISO = (M.flags & PMOC_ISO) != 0, SO = (M.flags & PMOC_HAS_SO) != 0;
   const int nz = M.nz, ny = SO ? M.ny : 0, nb = ISO ? M.nb : 0, T = wnthr(), t = wtid();
-  const long long m = rt::block_idx();
+  const long long m = wide_member<LIST>(a);
   double* sm = rt::smem();
   // six level arrays: the two profiles and four work arrays
   double *b1 = sm, *b2 = sm + nz, *A = sm + 2 * nz, *B = sm + 3 * nz, *C = sm + 4 * nz, *P = sm + 5 * nz;
@@ -389,14 +397,14 @@ PM_GLOBAL void k_wide_refresh(WideArgs a) {
 // Measured gain of the pipelined form: nz = 1024 +18 %, nz = 2048 +10 %.
 constexpr int kWideCol = 256;
 
-template <int LPT, int SH, bool PIPE>
+template <int LPT, int SH, bool PIPE, bool LIST>
 PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(WideArgs a) {
   constexpr int kWideAll = kWideCol + (PIPE ? 32 : 0);
   static_assert((1 << SH) == LPT && LPT >= 2, "LPT = 2^SH >= 2");
   const pmoc_model& M = a.m;
   const int nz = M.nz, ny = M.ny, t = wtid(), W = rt::warp_in_block(), Ln = rt::lane();
   const bool col = t < kWideCol, mlw = W == (PIPE ? kWideCol / 32 : kWideCol / 32 - 1);
-  const long long m = rt::block_idx();
+  const long long m = wide_member<LIST>(a);
   const double dt = M.dt;
   constexpr int nzp = kWideCol * LPT;
   const int nyp = (ny + 3) & ~3;
@@ -871,12 +879,12 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
 // buffered (read / written / cleared), so a step costs one barrier.  The arithmetic is that of
 // pm::col_step_exact, as in the 'jn' kernel.  At LPT = 4 the kernel is compiled for two CTAs per SM (at most 128
 // registers; it needs about 125 without spilling, against 150 / 194 left free), the wider ones for one.
-template <int LPT, int NCOL>
+template <int LPT, int NCOL, bool LIST>
 PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol, LPT == 4 ? 2 : 1) k_wide_post(WideArgs a) {
   const pmoc_model& M = a.m;
   const bool TW = (M.flags & PMOC_HAS_TW) != 0, ISO = (M.flags & PMOC_ISO) != 0, SO = (M.flags & PMOC_HAS_SO) != 0;
   const int nz = M.nz, t = wtid(), Ln = rt::lane();
-  const long long m = rt::block_idx();
+  const long long m = wide_member<LIST>(a);
   const double dt = M.dt;
   constexpr int nzp = kWideCol * LPT;
   double* sm = rt::smem();
@@ -1070,15 +1078,63 @@ size_t wide_refresh_smem(int nz, int ny, int nb) {
   return sizeof(double) * (size_t)(6 * nz + nbp + nbp / 2 + 2 + 64 + kWideThreads + 3 * nyp + 4);
 }
 
-}  // namespace pmk
-
 // Host loop: alternate the diagnosis and step launches in the model's order.
 //   'jn'   (run_JansenNadeau_2018.py:201-261): the diagnosis at the top of every iteration with it % K == 0, then
 //          the steps up to the next such iteration.
 //   'post' (example_twocol_plusSO.py:99-115): the steps of iterations [ii, stop], stop the first multiple of K at
 //          or after ii, then the diagnosis when stop < it_end (k_model's next0 / hits rule, so that split launches
 //          reproduce one launch bit for bit).
-int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream) {
+// Over `ctas` members (LIST: the members of the active list); pmoc_run_model_wide has checked the model.
+template <bool LIST>
+static int wide_loop(WideArgs a, bool post, int diagnose_only, long long nsteps, long long ctas, size_t sm_r,
+                     void* stream) {
+  if (diagnose_only) return launch(k_wide_refresh<LIST>, ctas, kWideThreads, sm_r, stream, a);
+  long long ii = a.it0;
+  const long long K = a.m.K, it_end = a.it0 + nsteps;
+  if (post) {
+    const bool two = (a.m.flags & PMOC_HAS_NORTH) != 0;
+    const int lpt = a.m.nz <= 4 * kWideCol ? 4 : a.m.nz <= 8 * kWideCol ? 8 : 16;
+    auto kern = lpt == 4 ? (two ? k_wide_post<4, 2, LIST> : k_wide_post<4, 1, LIST>)
+              : lpt == 8 ? (two ? k_wide_post<8, 2, LIST> : k_wide_post<8, 1, LIST>)
+                         : (two ? k_wide_post<16, 2, LIST> : k_wide_post<16, 1, LIST>);
+    const size_t sm_s = wide_post_smem(lpt, two ? 2 : 1);
+    while (ii < it_end) {
+      const long long stop = ((ii + K - 1) / K) * K;  // first iteration with it % K == 0 at or after ii
+      const bool hits = stop < it_end;
+      a.it0 = ii;
+      a.nsteps = (hits ? stop + 1 : it_end) - ii;
+      if (int rc = launch(kern, ctas, kWideCol, sm_s, stream, a)) return rc;
+      ii += a.nsteps;
+      if (hits)
+        if (int rc = launch(k_wide_refresh<LIST>, ctas, kWideThreads, sm_r, stream, a)) return rc;
+    }
+    return PMOC_OK;
+  }
+  while (ii < it_end) {
+    if (ii % K == 0) {
+      if (int rc = launch(k_wide_refresh<LIST>, ctas, kWideThreads, sm_r, stream, a)) return rc;
+      a.m.flags &= ~kFlagPsiPushed;  // the streamfunctions are the diagnosis's own from here on
+    }
+    long long stop = (ii / K + 1) * K;
+    if (stop > it_end) stop = it_end;
+    a.it0 = ii;
+    a.nsteps = stop - ii;
+    int rc;
+    if (a.m.nz <= 4 * kWideCol)
+      rc = launch(k_wide_steps2<4, 2, true, LIST>, ctas, kWideCol + 32, wide_steps2_smem(4, a.m.ny), stream, a);
+    else if (a.m.nz <= 8 * kWideCol)
+      rc = launch(k_wide_steps2<8, 3, true, LIST>, ctas, kWideCol + 32, wide_steps2_smem(8, a.m.ny), stream, a);
+    else
+      rc = launch(k_wide_steps2<16, 4, false, LIST>, ctas, kWideCol, wide_steps2_smem(16, a.m.ny), stream, a);
+    if (rc) return rc;
+    ii = stop;
+  }
+  return PMOC_OK;
+}
+}  // namespace pmk
+
+int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, int diagnose_only, void* stream,
+                        MemberList list) {
   const unsigned topo = m->flags & (PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO | PMOC_HAS_ML | PMOC_ORDER_JN);
   const unsigned jn = PMOC_HAS_NORTH | PMOC_HAS_TW | PMOC_ISO | PMOC_HAS_SO | PMOC_HAS_ML | PMOC_ORDER_JN;
   const bool post = topo == PMOC_HAS_TW || topo == PMOC_HAS_SO || topo == (PMOC_HAS_TW | PMOC_HAS_SO) ||
@@ -1099,7 +1155,8 @@ int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, in
   a.it0 = it0;
   a.nsteps = 0;
   a.force_late = std::getenv("PMOC_WIDE_FORCE_LATE") != nullptr;
-  const long long K = m->K, it_end = it0 + nsteps;
+  a.list = list;
+  const long long ctas = list.slots(m->M);  // one per member of the active list
   const int nb = (m->flags & PMOC_ISO) ? m->nb : 0, ny = (m->flags & PMOC_HAS_SO) ? m->ny : 0;
   const size_t sm_r = wide_refresh_smem(m->nz, ny, nb);
   if (sm_r > kMaxSmemPerBlock) {
@@ -1107,46 +1164,8 @@ int pmoc_run_model_wide(const pmoc_model* m, long long it0, long long nsteps, in
                   "block, more than the %zu one block can use", m->nz, nb, ny, sm_r, kMaxSmemPerBlock);
     return PMOC_EUNSUPPORTED;
   }
+  if (ctas == 0) return PMOC_OK;
   if (int rc = launch(k_wide_geo, 64, kWideThreads, 0, stream, a)) return rc;
-  if (diagnose_only) return launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a);
-  long long ii = it0;
-  if (post) {
-    const bool two = (m->flags & PMOC_HAS_NORTH) != 0;
-    const int lpt = m->nz <= 4 * kWideCol ? 4 : m->nz <= 8 * kWideCol ? 8 : 16;
-    auto kern = lpt == 4 ? (two ? k_wide_post<4, 2> : k_wide_post<4, 1>)
-              : lpt == 8 ? (two ? k_wide_post<8, 2> : k_wide_post<8, 1>)
-                         : (two ? k_wide_post<16, 2> : k_wide_post<16, 1>);
-    const size_t sm_s = wide_post_smem(lpt, two ? 2 : 1);
-    while (ii < it_end) {
-      const long long stop = ((ii + K - 1) / K) * K;  // first iteration with it % K == 0 at or after ii
-      const bool hits = stop < it_end;
-      a.it0 = ii;
-      a.nsteps = (hits ? stop + 1 : it_end) - ii;
-      if (int rc = launch(kern, m->M, kWideCol, sm_s, stream, a)) return rc;
-      ii += a.nsteps;
-      if (hits)
-        if (int rc = launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a)) return rc;
-    }
-    return PMOC_OK;
-  }
-  while (ii < it_end) {
-    if (ii % K == 0) {
-      if (int rc = launch(k_wide_refresh, m->M, kWideThreads, sm_r, stream, a)) return rc;
-      a.m.flags &= ~kFlagPsiPushed;  // the streamfunctions are the diagnosis's own from here on
-    }
-    long long stop = (ii / K + 1) * K;
-    if (stop > it_end) stop = it_end;
-    a.it0 = ii;
-    a.nsteps = stop - ii;
-    int rc;
-    if (m->nz <= 4 * kWideCol)
-      rc = launch(k_wide_steps2<4, 2, true>, m->M, kWideCol + 32, wide_steps2_smem(4, m->ny), stream, a);
-    else if (m->nz <= 8 * kWideCol)
-      rc = launch(k_wide_steps2<8, 3, true>, m->M, kWideCol + 32, wide_steps2_smem(8, m->ny), stream, a);
-    else
-      rc = launch(k_wide_steps2<16, 4, false>, m->M, kWideCol, wide_steps2_smem(16, m->ny), stream, a);
-    if (rc) return rc;
-    ii = stop;
-  }
-  return PMOC_OK;
+  return list.members ? wide_loop<true>(a, post, diagnose_only, nsteps, ctas, sm_r, stream)
+                      : wide_loop<false>(a, post, diagnose_only, nsteps, ctas, sm_r, stream);
 }

@@ -223,6 +223,28 @@ class Ensemble:
     if sync:
       self.be.sync()
 
+  def run_to_equilibrium(self, max_steps, every, tol):
+    """Spin-up: advance up to ``max_steps`` iterations in chunks of ``every`` (both multiples of K) and freeze each
+    member at the first check where no value of its state (every column's b, the mixed layer's bs) moved by more
+    than ``tol`` since the previous check; only the members still moving are stepped.  Non-finite members stop as
+    not converged.  Returns ``{'stopped_at': int64[M], 'converged': bool[M]}``; a member stopped at ``n`` holds
+    exactly what ``run`` to iteration ``n`` gives it, a valid pickup when ``n`` is a multiple of K.  ``self.it``
+    moves on by ``max_steps``: the loop reads the iteration counter only modulo K, so a later ``run`` continues
+    every member from its own stop."""
+    if self.spec.order == 'post' and not self._diagnosed:
+      self.diagnose()
+    need = int(self.lib.pmoc_equilibrate_work_bytes(ctypes.byref(self.model)))
+    work = self.be.upload(np.zeros((need + 7) // 8, dtype=np.float64))
+    stopped = self.be.upload(np.zeros(self.M, dtype=np.int64))
+    converged = self.be.upload(np.zeros(self.M, dtype=np.uint8))
+    with self._guard():
+      _abi.check(self.lib, self.lib.pmoc_model_equilibrate(
+          ctypes.byref(self.model), self.it, int(max_steps), int(every), float(tol), self.be.ptr(stopped),
+          self.be.ptr(converged), self.be.ptr(work), need, self.be.stream()))
+    self.it += int(max_steps)
+    self.be.sync()
+    return {'stopped_at': self.be.download(stopped), 'converged': self.be.download(converged).astype(bool)}
+
   # -------------------------------------------------------------------------------- output
   def state(self):
     """Prognostic arrays as numpy: b_basin[, b_north][, bs_ml] -- exactly what the reference's
@@ -289,6 +311,10 @@ class HostEnsemble(Ensemble):
 
   def diagnose(self):
     _abi.check(self.lib, self.lib.pmoc_host_step(self._handle, 0, 0, 0, _abi.IO_PSI | _abi.IO_DIAG))
+
+  def run_to_equilibrium(self, max_steps, every, tol):
+    raise NotImplementedError('HostEnsemble has no run_to_equilibrium: pmoc_model_equilibrate takes device buffers '
+                              '(use Ensemble)')
 
   def last_bytes(self):
     """(host->device, device->host) bytes of the last call."""

@@ -359,13 +359,14 @@ def _one(inp, m):
           for k, v in inp.items()}
 
 
-def column_batched(backend):
+def column_batched(backend, grid=_grid, stage_masks=(1, 2, 3, 7)):
+  """``grid(nz)``: the z levels (uniform by default); ``stage_masks``: the stage masks run at every size."""
   rng = np.random.default_rng(3)
   M = MOD_M
   worst = 0.0
-  cases = [(nz, st, dc, False) for nz in MOD_SIZES for st in (1, 2, 3, 7) for dc in (False, True)] + [(129, 3, False, True)]
+  cases = [(nz, st, dc, False) for nz in MOD_SIZES for st in stage_masks for dc in (False, True)] + [(129, 3, False, True)]
   for nz, stages, do_conv, bzbot in cases:
-    z = _grid(nz)
+    z = grid(nz)
     kap = (1e-5 + 3e-4 * np.exp(-z / 1000 - 4))[None, :] * np.linspace(0.5, 1.2, M)[:, None]
     area = 6e13 * (1. + 0.2 * z / 4000.)  # shared (stride 0)
     b = 0.03 * np.exp(z / 300.)[None, :] * np.linspace(0.8, 1.2, M)[:, None] - 0.001
@@ -374,7 +375,7 @@ def column_batched(backend):
                bs=np.linspace(0.025, 0.033, M), N2min=np.array(1.5e-7), bbot=np.linspace(-0.002, 0., M),
                bzbot=np.linspace(1e-7, 5e-7, M) if bzbot else None,
                wA=rng.normal(0, 2e6, (M, nz)), vdx=rng.normal(0, 1e7, (M, nz)), b_in=rng.uniform(-0.002, 0.03, (M, nz)),
-               dt=0.3 * (z[1] - z[0])**2 / kap.max())
+               dt=0.3 * np.diff(z).min()**2 / kap.max())
     tag = ('column', nz, stages, do_conv, bzbot)
     got = _column_call(backend, z, inp, stages, do_conv, M)
     _sentinel(got, M, tag)
@@ -404,11 +405,11 @@ def _tw_call(be, z, inp, M):
   return {'Psi': c.get(psi)}
 
 
-def thermwind_batched(backend):
+def thermwind_batched(backend, grid=_grid):
   M, worst = MOD_M, 0.0
   for nz in SIZES:
     for with_gmid in (False, True):
-      z = _grid(nz)
+      z = grid(nz)
       b1 = 0.03 * np.exp(z / 300.)[None, :] * np.linspace(0.7, 1.3, M)[:, None]
       b2 = 0.004 * np.exp(z / 500.)  # shared
       g = b2[None, :] - b1
@@ -466,11 +467,11 @@ def _so_model(c, z, y, inp, M):
   m.M, m.nz, m.ny = M, z.size, y.size
   m.z, m.y = c.ptr(z), c.ptr(y)
   m.so_tau, m.so_tau_on_y = c.vec(inp['tau'][:M] if inp['tau'].ndim == 2 else inp['tau'][:M, None]), int(inp['tau'].ndim == 2)
-  m.so_f, m.so_rho, m.so_smax = c.vec(inp['f']), c.vec(inp['rho']), c.vec(inp['smax'])  # shared
+  m.so_f, m.so_rho, m.so_smax = c.vec(inp['f']), c.vec(inp['rho']), c.vec(inp['smax'])  # 0-D shared, [M, 1] per member
   m.so_L, m.so_KGM = c.vec(inp['L'][:M, None]), c.vec(inp['KGM'][:M, None])
   m.so_c = c.vec(None if inp['c'] is None else inp['c'][:M, None])
   m.so_bvp_with_Ek = int(inp['c'] is not None)
-  m.so_sill_taper, m.so_ek_taper, m.so_top_taper, m.so_bot_taper = (c.ptr(t) for t in so_tapers(z))
+  m.so_sill_taper, m.so_ek_taper, m.so_top_taper, m.so_bot_taper = (c.ptr(t) for t in so_tapers(z, **inp.get('H', {})))
   return m
 
 
@@ -487,8 +488,8 @@ def _so_call(be, z, y, inp, M):
   return got
 
 
-def _so_inputs(nz, ny, tau_on_y, with_c, M):
-  z, y = _grid(nz), np.linspace(0, 2e6, ny)
+def _so_inputs(nz, ny, tau_on_y, with_c, M, grid=_grid):
+  z, y = grid(nz), np.linspace(0, 2e6, ny)
   bs = 0.03 * (y / y[-1])[None, :]**2 * np.linspace(0.8, 1.2, M)[:, None]
   b = 0.03 * np.exp(z / 300.)[None, :] * np.linspace(0.6, 1.1, M)[:, None] - 0.0005
   tau = np.linspace(0.05, 0.25, M)

@@ -42,7 +42,7 @@ def _on_grid(spec, z):
   on_z = lambda a: np.ascontiguousarray(np.apply_along_axis(lambda r: np.interp(z, z0, r), -1, a))
   col = lambda c: None if c is None else dataclasses.replace(c, kappa=on_z(c.kappa), Area=on_z(c.Area), b0=on_z(c.b0))
   tw = spec.tw if spec.tw is None or spec.tw.b2 is None else dataclasses.replace(spec.tw, b2=on_z(spec.tw.b2))
-  return dataclasses.replace(spec, z=z, basin=col(spec.basin), north=col(spec.north), tw=tw)
+  return dataclasses.replace(spec, z=z, basin=col(spec.basin), north=col(spec.north), pac=col(spec.pac), tw=tw)
 
 
 def variant(name, nz):

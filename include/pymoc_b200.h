@@ -223,6 +223,16 @@ int pmoc_model_run_members(const pmoc_model* m, const int64_t* members, int64_t 
 uint64_t pmoc_equilibrate_work_bytes(const pmoc_model* m);
 int pmoc_model_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
                            int64_t* stopped_at, uint8_t* converged, void* work, uint64_t work_bytes, void* stream);
+/* The same run for a consumer whose arrays are in HOST memory: pmoc_host_equilibrate through the persistent handle
+ * below, pmoc_model_equilibrate_host as its stateless form.  Same stops, flags and end state as
+ * pmoc_model_equilibrate; stopped_at[M] and converged[M] are HOST arrays; synchronous.  The library allocates the
+ * work buffer itself, from its private pool, for the duration of the call.  Argument errors are those of
+ * pmoc_model_equilibrate (and of pmoc_host_step for push / pull) and are found before anything is copied; topologies
+ * pmoc_model_run refuses are refused with its code and text, and the handle stays usable.  The stateless form moves
+ * what pmoc_model_run_host moves; the streamfunctions and diagnostics come back whenever the call diagnoses or
+ * steps.  pmoc_host_last_bytes counts the classes moved plus 9 bytes per member of results. */
+int pmoc_model_equilibrate_host(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                                int64_t* stopped_at, uint8_t* converged);
 
 /* Same as diagnose (when it0 == 0, order 'post') + run, but every pointer in `m` is a HOST pointer: the
  * stateless form of the handle below (open, one step, close), with the same device mirror and block loop.
@@ -231,8 +241,8 @@ int pmoc_model_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, 
  * diagnostics (PMOC_IO_PSI | PMOC_IO_DIAG) when the call diagnoses, and ml_Psi_s when it steps.
  * Synchronous.  This is the call a non-torch consumer binds. */
 int pmoc_model_run_host(const pmoc_model* m, int64_t it0, int64_t nsteps);
-/* bytes the last pmoc_model_run_host / pmoc_host_open / pmoc_host_step of this thread copied
- * host->device / device->host */
+/* bytes the last pmoc_model_run_host / pmoc_model_equilibrate_host / pmoc_host_open / pmoc_host_step /
+ * pmoc_host_equilibrate of this thread copied host->device / device->host */
 void pmoc_host_last_bytes(uint64_t* h2d, uint64_t* d2h);
 
 /* Persistent host-buffer handle: the same loop (the examples' `for ii in range(total_iters)` with its
@@ -253,6 +263,10 @@ void pmoc_host_last_bytes(uint64_t* h2d, uint64_t* d2h);
 typedef struct pmoc_host pmoc_host;
 int pmoc_host_open(const pmoc_model* m, pmoc_host** handle);
 int pmoc_host_step(pmoc_host* handle, int64_t it0, int64_t nsteps, uint32_t push, uint32_t pull);
+/* pmoc_model_equilibrate through the handle (see there): push / pull as in pmoc_host_step, the order-'post'
+ * diagnosis under its rule; a later pmoc_host_step from it0 + max_steps continues each member from its own stop. */
+int pmoc_host_equilibrate(pmoc_host* handle, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                          int64_t* stopped_at, uint8_t* converged, uint32_t push, uint32_t pull);
 int pmoc_host_close(pmoc_host* handle);
 
 /* ---- per-module entry points (the reference's method surface), batched over M ----------- */

@@ -64,7 +64,7 @@ class Model(C.Structure):
 EXPORTS = ('pmoc_abi_version', 'pmoc_last_error', 'pmoc_device_info', 'pmoc_model_scratch_bytes', 'pmoc_model_diagnose', 'pmoc_model_run',
            'pmoc_model_run_host', 'pmoc_host_last_bytes', 'pmoc_host_open', 'pmoc_host_step', 'pmoc_host_close', 'pmoc_column_timestep', 'pmoc_thermwind_solve', 'pmoc_thermwind_psib',
            'pmoc_so_solve', 'pmoc_ml_timestep', 'pmoc_fp64_peak', 'pmoc_model_run_members', 'pmoc_equilibrate_work_bytes',
-           'pmoc_model_equilibrate')
+           'pmoc_model_equilibrate', 'pmoc_model_equilibrate_host', 'pmoc_host_equilibrate')
 
 
 def declare(lib):
@@ -97,6 +97,10 @@ def declare(lib):
   lib.pmoc_equilibrate_work_bytes.argtypes = [P(Model)]
   lib.pmoc_model_equilibrate.argtypes = [P(Model), C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_uint64, C.c_void_p]
+  lib.pmoc_model_equilibrate_host.argtypes = [P(Model), C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p,
+                                              C.c_void_p]
+  lib.pmoc_host_equilibrate.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
+                                        C.c_uint32, C.c_uint32]
   for name in EXPORTS:
     if name not in ('pmoc_last_error', 'pmoc_model_scratch_bytes', 'pmoc_host_last_bytes', 'pmoc_equilibrate_work_bytes'):
       getattr(lib, name).restype = C.c_int

@@ -260,6 +260,10 @@ PM_DEV unsigned status_word(unsigned old, unsigned bits, bool carry) {
 
 // the checks pmoc_model_run applies to a model before it dispatches (pmoc_ops.cu)
 int check_model(const pmoc_model* m);
+// check_model and the argument checks of pmoc_model_equilibrate but its work buffer (pmoc_equil.cu); the host-buffer
+// entry points apply them before they copy anything
+int check_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                      const void* stopped_at, const void* converged);
 }  // namespace pmk
 using namespace pmk;
 

@@ -87,6 +87,17 @@ PM_GLOBAL void k_equil_check(EqArgs a) {
   }
 }
 
+int check_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                      const void* stopped_at, const void* converged) {
+  if (int rc = check_model(m)) return rc;
+  if (it0 < 0 || max_steps < 0) return fail(PMOC_EINVAL, "negative it0 / max_steps");
+  if (every <= 0 || every % m->K != 0) return fail(PMOC_EINVAL, "every must be a positive multiple of K");
+  if (max_steps % m->K != 0) return fail(PMOC_EINVAL, "max_steps must be a multiple of K");
+  if (!(tol >= 0.0)) return fail(PMOC_EINVAL, "tol must be >= 0");
+  if (!stopped_at || !converged) return fail(PMOC_EINVAL, "stopped_at / converged is NULL");
+  return PMOC_OK;
+}
+
 }  // namespace pmk
 
 extern "C" {
@@ -98,12 +109,7 @@ uint64_t pmoc_equilibrate_work_bytes(const pmoc_model* m) {
 
 int pmoc_model_equilibrate(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every, double tol,
                            int64_t* stopped_at, uint8_t* converged, void* work, uint64_t work_bytes, void* stream) {
-  if (int rc = check_model(m)) return rc;
-  if (it0 < 0 || max_steps < 0) return fail(PMOC_EINVAL, "negative it0 / max_steps");
-  if (every <= 0 || every % m->K != 0) return fail(PMOC_EINVAL, "every must be a positive multiple of K");
-  if (max_steps % m->K != 0) return fail(PMOC_EINVAL, "max_steps must be a multiple of K");
-  if (!(tol >= 0.0)) return fail(PMOC_EINVAL, "tol must be >= 0");
-  if (!stopped_at || !converged) return fail(PMOC_EINVAL, "stopped_at / converged is NULL");
+  if (int rc = check_equilibrate(m, it0, max_steps, every, tol, stopped_at, converged)) return rc;
   const EqLayout lay = eq_layout(*m);
   if (!work || work_bytes < lay.bytes()) return fail(PMOC_EINVAL, "work needs pmoc_equilibrate_work_bytes() bytes");
   EqArgs a;

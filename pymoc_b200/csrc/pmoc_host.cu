@@ -3,8 +3,9 @@
 // The stateless call (pmoc_model_run_host) and the persistent handle (pmoc_host_open / step / close) share one
 // device mirror of the caller's host arrays.  Every per-member array of the mirror carries a class bitmask; a
 // call names the classes that go up before its launches and come back after them, and one block loop moves
-// them (Mirror::pass, with Mirror::copy).  The emulator build runs this same code on host stand-ins of the
-// CUDA runtime calls (pmoc_rt.cuh).
+// them (Mirror::pass, with Mirror::copy).  Runs to equilibrium through either form (pmoc_model_equilibrate_host,
+// pmoc_host_equilibrate) share Mirror::equilibrate.  The emulator build runs this same code on host stand-ins of
+// the CUDA runtime calls (pmoc_rt.cuh).
 #include "pmoc_common.cuh"
 
 #include <algorithm>
@@ -280,6 +281,50 @@ struct Mirror {
     fresh = false;
     return rc;
   }
+  // stream `to` waits for the work queued so far on stream `from`
+  void join(int to, int from) {
+    if (err == cudaSuccess) err = cudaEventRecord(shared_ready, s[from]);
+    if (err == cudaSuccess) err = cudaStreamWaitEvent(s[to], shared_ready, 0);
+  }
+  // One run to equilibrium (pmoc_model_equilibrate): the classes in `push` go up and the model is diagnosed
+  // (`diag`) block by block; the run covers every member at once on stream 0 behind all three streams, since one
+  // active list per block would run the blocks' tails one after another; the classes in `pull` come back block by
+  // block behind it, and stopped_at / converged (HOST arrays) on stream 0.  The work buffer, the device results and,
+  // for nz > 256, a scratch buffer for all M members (the per-stream ones hold one block) are the call's own, freed
+  // on every path.  Returns the first launch error; a CUDA error is left in `err`.
+  int equilibrate(unsigned push, bool diag, long long it0, long long max_steps, long long every, double tol,
+                  int64_t* stopped_at, uint8_t* converged, unsigned pull) {
+    int rc = pass(push, diag, false, it0, 0, 0);
+    for (int i = 1; i < kStreams; ++i) join(0, i);
+    std::vector<void*> own;
+    auto take = [&](size_t bytes) {
+      void* p = nullptr;
+      if (err == cudaSuccess) err = cudaMallocFromPoolAsync(&p, bytes, pool, s[0]);
+      if (p) own.push_back(p);
+      return p;
+    };
+    pmoc_model w = d;  // the whole-M device model
+    w.scratch = nullptr;
+    w.scratch_bytes = pmoc_model_scratch_bytes(&w);
+    if (w.scratch_bytes) w.scratch = take((size_t)w.scratch_bytes);
+    const uint64_t work_bytes = pmoc_equilibrate_work_bytes(&w);
+    void* work = take((size_t)work_bytes);
+    int64_t* d_stopped = static_cast<int64_t*>(take((size_t)d.M * sizeof(int64_t)));
+    uint8_t* d_converged = static_cast<uint8_t*>(take((size_t)d.M));
+    if (rc == PMOC_OK && err == cudaSuccess)
+      rc = pmoc_model_equilibrate(&w, it0, max_steps, every, tol, d_stopped, d_converged, work, work_bytes, s[0]);
+    if (rc == PMOC_OK) {
+      for (int i = 1; i < kStreams; ++i) join(i, 0);
+      pass(0, false, false, it0, 0, pull);
+      if (err == cudaSuccess)
+        err = cudaMemcpyAsync(stopped_at, d_stopped, (size_t)d.M * sizeof(int64_t), cudaMemcpyDeviceToHost, s[0]);
+      if (err == cudaSuccess)
+        err = cudaMemcpyAsync(converged, d_converged, (size_t)d.M, cudaMemcpyDeviceToHost, s[0]);
+      if (err == cudaSuccess) g_d2h_bytes += (size_t)d.M * (sizeof(int64_t) + 1);
+    }
+    for (void* p : own) cudaFreeAsync(p, s[0]);  // behind everything that uses them, all of it on stream 0
+    return rc;
+  }
 };
 
 }  // namespace
@@ -301,6 +346,28 @@ extern "C" int pmoc_model_run_host(const pmoc_model* m, int64_t it0, int64_t nst
   int rc = PMOC_OK;
   if (mr.open(m) == cudaSuccess) rc = mr.pass(push, !jn && it0 == 0, true, it0, nsteps, pull);
   const cudaError_t e = mr.fini();  // every path: streams, event and device memory are returned
+  if (rc != PMOC_OK) return rc;
+  PM_CUDA_OK(mr.err);
+  PM_CUDA_OK(e);
+  return PMOC_OK;
+}
+
+extern "C" int pmoc_model_equilibrate_host(const pmoc_model* m, int64_t it0, int64_t max_steps, int64_t every,
+                                           double tol, int64_t* stopped_at, uint8_t* converged) {
+  g_h2d_bytes = g_d2h_bytes = 0;
+  if (int rc = check_equilibrate(m, it0, max_steps, every, tol, stopped_at, converged)) return rc;
+  // pushed as by pmoc_model_run_host; every member runs at least one chunk of K or more iterations when
+  // max_steps > 0, so every member diagnoses
+  const bool jn = (m->flags & PMOC_ORDER_JN) != 0;
+  const bool diag = !jn && it0 == 0;
+  const bool carry = jn ? (it0 % m->K != 0) : (it0 > 0);
+  const unsigned push = kIoParam | PMOC_IO_STATE | (carry ? PMOC_IO_PSI : 0);
+  const unsigned pull = PMOC_IO_STATE | (diag || max_steps > 0 ? PMOC_IO_PSI | PMOC_IO_DIAG : 0) |
+                        (max_steps > 0 ? kIoStepped : 0);
+  Mirror mr;
+  int rc = PMOC_OK;
+  if (mr.open(m) == cudaSuccess) rc = mr.equilibrate(push, diag, it0, max_steps, every, tol, stopped_at, converged, pull);
+  const cudaError_t e = mr.fini();
   if (rc != PMOC_OK) return rc;
   PM_CUDA_OK(mr.err);
   PM_CUDA_OK(e);
@@ -346,6 +413,30 @@ extern "C" int pmoc_host_step(pmoc_host* h, int64_t it0, int64_t nsteps, uint32_
   const bool need_diag = !jn && (it0 == 0 || ((push & PMOC_IO_STATE) && !(push & PMOC_IO_PSI) && !h->diagnosed));
   if (push & PMOC_IO_PSI) mr.d.flags |= kFlagPsiPushed;  // the caller's streamfunctions: no carried exemption
   const int rc = mr.pass(push, need_diag, nsteps > 0, it0, nsteps, pull);
+  mr.d.flags &= ~kFlagPsiPushed;
+  const cudaError_t e = mr.sync();
+  if (rc != PMOC_OK) return rc;
+  PM_CUDA_OK(mr.err);
+  PM_CUDA_OK(e);
+  h->diagnosed = true;
+  return PMOC_OK;
+}
+
+extern "C" int pmoc_host_equilibrate(pmoc_host* h, int64_t it0, int64_t max_steps, int64_t every, double tol,
+                                     int64_t* stopped_at, uint8_t* converged, uint32_t push, uint32_t pull) {
+  g_h2d_bytes = g_d2h_bytes = 0;
+  if (!h) return fail(PMOC_EINVAL, "handle is NULL");
+  if ((push | pull) & ~(PMOC_IO_STATE | PMOC_IO_PSI | PMOC_IO_DIAG)) return fail(PMOC_EINVAL, "unknown PMOC_IO_* bit");
+  if (push & PMOC_IO_DIAG) return fail(PMOC_EINVAL, "diagnostics are outputs: they cannot be pushed");
+  Mirror& mr = h->mr;
+  if (int rc = check_equilibrate(&mr.d, it0, max_steps, every, tol, stopped_at, converged)) return rc;
+  // diagnosed first, and the pushed streamfunctions flagged, as in pmoc_host_step.  The flag stays on for every
+  // chunk: a 'jn' chunk that starts between two diagnoses (it0 % K != 0) then classifies its carried Psi_so[1]
+  // from its value alone, which can add PMOC_ST_NOISE_SWITCH but changes no state
+  const bool jn = (mr.d.flags & PMOC_ORDER_JN) != 0;
+  const bool need_diag = !jn && (it0 == 0 || ((push & PMOC_IO_STATE) && !(push & PMOC_IO_PSI) && !h->diagnosed));
+  if (push & PMOC_IO_PSI) mr.d.flags |= kFlagPsiPushed;
+  const int rc = mr.equilibrate(push, need_diag, it0, max_steps, every, tol, stopped_at, converged, pull);
   mr.d.flags &= ~kFlagPsiPushed;
   const cudaError_t e = mr.sync();
   if (rc != PMOC_OK) return rc;

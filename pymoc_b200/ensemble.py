@@ -312,9 +312,18 @@ class HostEnsemble(Ensemble):
   def diagnose(self):
     _abi.check(self.lib, self.lib.pmoc_host_step(self._handle, 0, 0, 0, _abi.IO_PSI | _abi.IO_DIAG))
 
-  def run_to_equilibrium(self, max_steps, every, tol):
-    raise NotImplementedError('HostEnsemble has no run_to_equilibrium: pmoc_model_equilibrate takes device buffers '
-                              '(use Ensemble)')
+  def run_to_equilibrium(self, max_steps, every, tol, push=0, pull=_abi.IO_STATE | _abi.IO_PSI | _abi.IO_DIAG):
+    """:meth:`Ensemble.run_to_equilibrium` through the handle (``pmoc_host_equilibrate``): the same stops, flags and
+    end state, the same returned dict, and ``self.it`` moves on by ``max_steps``.  ``push`` / ``pull`` as in
+    :meth:`run`: the classes copied to the device before the run and back after it."""
+    if self._handle is None:
+      raise RuntimeError('HostEnsemble is closed')
+    stopped, converged = np.zeros(self.M, dtype=np.int64), np.zeros(self.M, dtype=np.uint8)
+    _abi.check(self.lib, self.lib.pmoc_host_equilibrate(self._handle, self.it, int(max_steps), int(every), float(tol),
+                                                        stopped.ctypes.data, converged.ctypes.data, int(push),
+                                                        int(pull)))
+    self.it += int(max_steps)
+    return {'stopped_at': stopped, 'converged': converged.astype(bool)}
 
   def last_bytes(self):
     """(host->device, device->host) bytes of the last call."""

@@ -12,20 +12,29 @@ Per workload (C4: the 32 768-member run_JansenNadeau_2018 lattice, K = 12, check
     chunking, the checks and the per-check read-back of the counter cost.
 Times are CUDA events around the call (the equilibrium call synchronises with the host after every check).  The card
 name and its power limit are recorded with the numbers.  Prints one JSON object.
+
+With ``--host`` (one tolerance, default 1e-4) each workload is instead run to equilibrium with its arrays in pinned
+HOST memory, alternately, twice each:
+  * ``host``: ``HostEnsemble.run_to_equilibrium`` (``pmoc_host_equilibrate``; state pushed, state, streamfunctions and
+    diagnostics pulled): wall time of the synchronous call and the bytes it moved;
+  * ``device_then_download``: ``Ensemble.run_to_equilibrium`` followed by a download of the same arrays into pinned
+    buffers: wall time to the end of the download.
+Both start from the same freshly built ensemble; the two results are compared bit for bit.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import time
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from pymoc_b200 import configs  # noqa: E402
-from pymoc_b200.ensemble import Ensemble  # noqa: E402
+from pymoc_b200 import _abi, configs  # noqa: E402
+from pymoc_b200.ensemble import Ensemble, HostEnsemble  # noqa: E402
 
 WORKLOADS = {  # name -> (builder, members, every)
     'C4': (lambda M: configs.c4_jansen_nadeau(M), 32768, 1200),
@@ -96,15 +105,66 @@ def bench(name, max_steps, tols):
   return out
 
 
+def bench_host(name, max_steps, tol, reps=2):
+  """The host-buffer leg: HostEnsemble.run_to_equilibrium against the device call plus a download of the same
+  arrays, alternated."""
+  import torch
+  build, M, every = WORKLOADS[name]
+  spec = build(M)
+  S, P, D = _abi.IO_STATE, _abi.IO_PSI, _abi.IO_DIAG
+  warm = HostEnsemble(spec)
+  warm.run_to_equilibrium(2 * every, every, 0.0)
+  warm.close()
+  out = {'workload': spec.name, 'members': M, 'nz': spec.nz, 'K': spec.K, 'every': every, 'max_steps': max_steps,
+         'tol': tol, 'host': [], 'device_then_download': []}
+  for _ in range(reps):
+    host = HostEnsemble(spec)
+    t0 = time.perf_counter()
+    r_host = host.run_to_equilibrium(max_steps, every, tol, push=S, pull=S | P | D)
+    ms = (time.perf_counter() - t0) * 1e3
+    h2d, d2h = host.last_bytes()
+    out['host'].append({'ms': ms, 'h2d_bytes': h2d, 'd2h_bytes': d2h})
+
+    dev = fresh(spec)
+    pinned = {k: torch.empty(tuple(b.shape), dtype=b.dtype, pin_memory=True) for k, b in dev._bufs.items()
+              if k != 'scratch'}
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    r_dev = dev.run_to_equilibrium(max_steps, every, tol)
+    for k, t in pinned.items():
+      t.copy_(dev._bufs[k], non_blocking=True)
+    torch.cuda.synchronize()
+    ms = (time.perf_counter() - t0) * 1e3
+    out['device_then_download'].append({'ms': ms, 'd2h_bytes': sum(t.numel() * t.element_size() for t in pinned.values())})
+
+    same = all(np.array_equal(r_host[k], r_dev[k]) for k in r_host)
+    same = same and all(np.array_equal(host.be.download(host._bufs[k]), t.numpy(), equal_nan=True)
+                        for k, t in pinned.items())
+    out.setdefault('identical', True)
+    out['identical'] = out['identical'] and bool(same)
+    out['converged_fraction'] = float(r_dev['converged'].mean())
+    host.close()
+    del host, dev, pinned
+  h, d = min(x['ms'] for x in out['host']), min(x['ms'] for x in out['device_then_download'])
+  out['host_vs_device_then_download'] = h / d
+  return out
+
+
 def main():
   ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
   ap.add_argument('--workloads', default='C4,C2')
   ap.add_argument('--max-steps', type=int, default=36000)
-  ap.add_argument('--tols', default='1e-8,1e-6', help='comma list of tolerances (buoyancy, m s^-2, per check)')
+  ap.add_argument('--tols', default=None,
+                  help='comma list of tolerances (buoyancy, m s^-2, per check); default 1e-8,1e-6, with --host 1e-4')
+  ap.add_argument('--host', action='store_true', help='the host-buffer leg (pinned arrays) instead')
   ap.add_argument('--out', default=None, help='also write the JSON object to this file')
   args = ap.parse_args()
-  res = {'card': card(), 'results': [bench(w, args.max_steps, [float(t) for t in args.tols.split(',')])
-                                     for w in args.workloads.split(',')]}
+  tols = [float(t) for t in (args.tols or ('1e-4' if args.host else '1e-8,1e-6')).split(',')]
+  if args.host:
+    results = [bench_host(w, args.max_steps, tols[0]) for w in args.workloads.split(',')]
+  else:
+    results = [bench(w, args.max_steps, tols) for w in args.workloads.split(',')]
+  res = {'card': card(), 'results': results}
   line = json.dumps(res)
   print(line)
   if args.out:

@@ -53,14 +53,21 @@ struct ThermwindArgs {
   const double* z;
   pmoc_vec b1, b2, f, gmid, Psi_in;
   double *Psi, *psib, *bgrid, *iso_b, *iso_n;
-  int nzp, nbp;
 };
+
+// Shared memory of k_thermwind (in doubles), per block: z on the warp's level slots and four more.
+struct ThermwindSmem {
+  int off_zs, nzs;
+  PM_HD constexpr size_t bytes() const { return sizeof(double) * (size_t)(off_zs + nzs); }
+};
+PM_HD constexpr ThermwindSmem thermwind_smem(int LPL) { return ThermwindSmem{0, 32 * LPL + 4}; }
 
 template <int LPL>
 PM_GLOBAL void k_thermwind(ThermwindArgs a) {
   const int nz = a.nz, L = rt::lane(), W = rt::warp_in_block(), nthr = rt::warps_per_block() * 32;
-  double* zs = rt::smem();
-  for (int i = W * 32 + L; i < 32 * LPL + 4; i += nthr) zs[i] = a.z[i < nz ? i : nz - 1];
+  constexpr ThermwindSmem sl = thermwind_smem(LPL);
+  double* zs = rt::smem() + sl.off_zs;
+  for (int i = W * 32 + L; i < sl.nzs; i += nthr) zs[i] = a.z[i < nz ? i : nz - 1];
   rt::syncblock();
   const long long m = rt::block_idx() * rt::warps_per_block() + W;
   if (m >= a.M) return;
@@ -71,18 +78,33 @@ PM_GLOBAL void k_thermwind(ThermwindArgs a) {
   pm::store_lev<LPL>(psi, a.Psi + m * nz, nz);
 }
 
+// Shared memory of k_psib (in doubles), per warp: the remap scratch (6 nzp), psib[nb] and the class counters
+// (nb + 1 ints).
+struct PsibSmem {
+  int w_remap, w_psib, w_cnt, per_warp;
+  PM_HD constexpr size_t bytes(int wpb) const { return sizeof(double) * (size_t)per_warp * wpb; }
+};
+PM_HD constexpr PsibSmem psib_smem(int LPL, int nb) {
+  PsibSmem s{};
+  const int nbp = (nb + 3) & ~3;
+  s.w_psib = s.w_remap + 6 * 32 * LPL; s.w_cnt = s.w_psib + nbp; s.per_warp = s.w_cnt + nbp / 2 + 2;
+  return s;
+}
+
 template <int LPL>
 PM_GLOBAL void k_psib(ThermwindArgs a) {
   const int nz = a.nz, nb = a.nb, L = rt::lane(), W = rt::warp_in_block();
   const long long m = rt::block_idx() * rt::warps_per_block() + W;
   if (m >= a.M) return;
-  double* ws = rt::smem() + (size_t)(6 * a.nzp + a.nbp + a.nbp / 2 + 2) * W;
+  const PsibSmem sl = psib_smem(LPL, nb);
+  double* ws = rt::smem() + (size_t)sl.per_warp * W;
   double b1[LPL], b2[LPL], psi[LPL];
   pm::load_lev<LPL>(b1, vrow(a.b1, m), nz, 0.0);
   pm::load_lev<LPL>(b2, vrow(a.b2, m), nz, 0.0);
   pm::load_lev<LPL>(psi, vrow(a.Psi_in, m), nz, 0.0);
-  double* psib_s = ws + 6 * a.nzp;
-  const pm::BGrid G = pm::tw_psib<LPL>(psi, b1, b2, nz, nb, ws, psib_s, reinterpret_cast<int*>(psib_s + a.nbp));
+  double* psib_s = ws + sl.w_psib;
+  const pm::BGrid G =
+      pm::tw_psib<LPL>(psi, b1, b2, nz, nb, ws + sl.w_remap, psib_s, reinterpret_cast<int*>(ws + sl.w_cnt));
   for (int i = L; i < nb; i += 32) {
     a.psib[m * nb + i] = psib_s[i];
     if (a.bgrid) a.bgrid[m * nb + i] = G.at(i);
@@ -105,40 +127,56 @@ struct SoArgs {
   pmoc_vec b, bs;
   double *Psi, *Psi_Ek, *Psi_GM, *ys;
   uint32_t* status;
-  int nzp, nyp;
 };
+
+// Shared memory of k_so (in doubles).  Per block: z (nzp + 4), y and the four tapers (4 nzp); per warp: bs, the
+// inverse slopes and tau on y.
+struct SoSmem {
+  int nzp, nyp, off_zs, off_ys, off_tap, off_warp0, w_bs, w_sinv, w_tau, per_warp;
+  PM_HD constexpr size_t bytes(int wpb) const { return sizeof(double) * (size_t)(off_warp0 + per_warp * wpb); }
+};
+PM_HD constexpr SoSmem so_smem(int LPL, int ny) {
+  SoSmem s{};
+  s.nzp = 32 * LPL; s.nyp = (ny + 3) & ~3;
+  s.off_ys = s.off_zs + s.nzp + 4; s.off_tap = s.off_ys + s.nyp; s.off_warp0 = s.off_tap + 4 * s.nzp;
+  s.w_sinv = s.w_bs + s.nyp; s.w_tau = s.w_sinv + s.nyp; s.per_warp = s.w_tau + s.nyp;
+  return s;
+}
 
 template <int LPL, bool BVP>
 PM_GLOBAL void k_so(SoArgs a) {
   const pmoc_model& M = a.m;
   const int nz = M.nz, ny = M.ny, L = rt::lane(), W = rt::warp_in_block(), nthr = rt::warps_per_block() * 32;
-  double* zs = rt::smem();
-  double* ysm = zs + a.nzp + 4;
-  double* tap = ysm + a.nyp;
-  double* bss = tap + 4 * a.nzp + (size_t)(3 * a.nyp) * W;
-  double* sinv = bss + a.nyp;
-  double* tau_s = sinv + a.nyp;
-  for (int i = W * 32 + L; i < a.nzp + 4; i += nthr) zs[i] = M.z[i < nz ? i : nz - 1];
-  for (int i = W * 32 + L; i < a.nyp; i += nthr) ysm[i] = M.y[i < ny ? i : ny - 1];
+  const SoSmem sl = so_smem(LPL, ny);
+  double* sm = rt::smem();
+  double* zs = sm + sl.off_zs;
+  double* ysm = sm + sl.off_ys;
+  double* tap = sm + sl.off_tap;
+  double* ws = sm + sl.off_warp0 + (size_t)sl.per_warp * W;
+  double* bss = ws + sl.w_bs;
+  double* sinv = ws + sl.w_sinv;
+  double* tau_s = ws + sl.w_tau;
+  for (int i = W * 32 + L; i < sl.nzp + 4; i += nthr) zs[i] = M.z[i < nz ? i : nz - 1];
+  for (int i = W * 32 + L; i < sl.nyp; i += nthr) ysm[i] = M.y[i < ny ? i : ny - 1];
   pm::taper_fill<LPL>(tap, M.so_sill_taper, M.so_ek_taper, M.so_top_taper, M.so_bot_taper, nz, W * 32 + L, nthr);
   rt::syncblock();
   const long long m = rt::block_idx() * rt::warps_per_block() + W;
   if (m >= M.M) return;
   const double* src = vrow(a.bs, m);
-  for (int i = L; i < a.nyp; i += 32) bss[i] = src[i < ny ? i : ny - 1];
+  for (int i = L; i < sl.nyp; i += 32) bss[i] = src[i < ny ? i : ny - 1];
   rt::syncwarp();
   pm::SoPar so{};
   so.tau_ave = M.so_tau_on_y ? 0.0 : pm::mean100(vat(M.so_tau, m));
   if (M.so_tau_on_y) {
     const double* t = vrow(M.so_tau, m);
-    for (int i = L; i < a.nyp; i += 32) tau_s[i] = t[i < ny ? i : ny - 1];
+    for (int i = L; i < sl.nyp; i += 32) tau_s[i] = t[i < ny ? i : ny - 1];
     so.tau_y = tau_s;
     rt::syncwarp();
   }
   so.f = vat(M.so_f, m); so.rho = vat(M.so_rho, m); so.L = vat(M.so_L, m);
   so.KGM = vat(M.so_KGM, m); so.smax = vat(M.so_smax, m);
   so.pre0 = so.tau_ave / so.f / so.rho * so.L;
-  so.sill = tap; so.ektap = tap + a.nzp; so.toptap = tap + 2 * a.nzp; so.bottap = tap + 3 * a.nzp;
+  so.sill = tap; so.ektap = tap + sl.nzp; so.toptap = tap + 2 * sl.nzp; so.bottap = tap + 3 * sl.nzp;
   so.c = BVP ? vat(M.so_c, m) : 0.0;
   so.with_Ek = M.so_bvp_with_Ek;
   double b[LPL], psi[LPL], ek[LPL], gm[LPL], ysv[LPL];
@@ -158,17 +196,32 @@ struct MlArgs {
   pmoc_vec b_basin, Psi_b;
   double dt;
   uint32_t* status;
-  int nzp, nyp;
 };
+
+// Shared memory of k_ml (in doubles).  Per block: y; per warp: b_basin and Psi_b on the levels, bs on y and the
+// scratch of pm::ml_setup.
+struct MlSmem {
+  int nyp, off_ys, off_warp0, w_bb, w_pm, w_bs, w_scan, per_warp;
+  PM_HD constexpr size_t bytes(int wpb) const { return sizeof(double) * (size_t)(off_warp0 + per_warp * wpb); }
+};
+PM_HD constexpr MlSmem ml_smem(int nz, int ny) {
+  MlSmem s{};
+  const int nzp = (nz + 3) & ~3;
+  s.nyp = (ny + 3) & ~3; s.off_warp0 = s.off_ys + s.nyp;
+  s.w_pm = s.w_bb + nzp; s.w_bs = s.w_pm + nzp; s.w_scan = s.w_bs + s.nyp; s.per_warp = s.w_scan + 10 * 32;
+  return s;
+}
 
 // SO_ML.timestep for every member: one warp per member, b_basin / Psi_b staged in shared memory
 PM_GLOBAL void k_ml(MlArgs a) {
   const pmoc_model& M = a.m;
   const int nz = M.nz, ny = M.ny, L = rt::lane(), W = rt::warp_in_block(), nthr = rt::warps_per_block() * 32;
-  double* ysm = rt::smem();
-  double* ws = ysm + a.nyp + (size_t)(2 * a.nzp + a.nyp + 320) * W;
-  double *bb_s = ws, *pm_s = ws + a.nzp, *bs_s = ws + 2 * a.nzp, *scan_s = bs_s + a.nyp;
-  for (int i = W * 32 + L; i < a.nyp; i += nthr) ysm[i] = M.y[i < ny ? i : ny - 1];
+  const MlSmem sl = ml_smem(nz, ny);
+  double* sm = rt::smem();
+  double* ysm = sm + sl.off_ys;
+  double* ws = sm + sl.off_warp0 + (size_t)sl.per_warp * W;
+  double *bb_s = ws + sl.w_bb, *pm_s = ws + sl.w_pm, *bs_s = ws + sl.w_bs, *scan_s = ws + sl.w_scan;
+  for (int i = W * 32 + L; i < sl.nyp; i += nthr) ysm[i] = M.y[i < ny ? i : ny - 1];
   rt::syncblock();
   const long long m = rt::block_idx() * rt::warps_per_block() + W;
   if (m >= M.M) return;
@@ -384,8 +437,8 @@ int pmoc_thermwind_solve(int64_t M, int32_t nz, const double* z, pmoc_vec b1, pm
   if (M <= 0 || nz < 3 || !z || !b1.ptr || !b2.ptr || !f.ptr || !Psi) return fail(PMOC_EINVAL, "bad thermwind arguments");
   ThermwindArgs a{};
   a.M = M; a.nz = nz; a.z = z; a.b1 = b1; a.b2 = b2; a.f = f; a.gmid = gmid; a.Psi = Psi;
-  PM_DISPATCH_LPL(nz, return launch(k_thermwind<LPL>, blocks_for(M), 32 * kWarpsPerBlock,
-                                    sizeof(double) * (32 * LPL + 4), stream, a));
+  PM_DISPATCH_LPL(nz, return launch(k_thermwind<LPL>, blocks_for(M), 32 * kWarpsPerBlock, thermwind_smem(LPL).bytes(),
+                                    stream, a));
   return PMOC_OK;
 }
 
@@ -395,10 +448,8 @@ int pmoc_thermwind_psib(int64_t M, int32_t nz, int32_t nb, pmoc_vec Psi, pmoc_ve
   ThermwindArgs a{};
   a.M = M; a.nz = nz; a.nb = nb; a.Psi_in = Psi; a.b1 = b1; a.b2 = b2;
   a.psib = psib; a.bgrid = bgrid; a.iso_b = iso_b; a.iso_n = iso_n;
-  a.nbp = (nb + 3) & ~3;
   PM_DISPATCH_LPL(nz, {
-    a.nzp = 32 * LPL;
-    const size_t smem = sizeof(double) * (size_t)(6 * a.nzp + a.nbp + a.nbp / 2 + 2) * kWarpsPerBlock;
+    const size_t smem = psib_smem(LPL, nb).bytes(kWarpsPerBlock);
     if (smem > kMaxSmemPerBlock) return fail_smem("nb", nb, smem);
     return launch(k_psib<LPL>, blocks_for(M), 32 * kWarpsPerBlock, smem, stream, a);
   });
@@ -414,12 +465,9 @@ int pmoc_so_solve(const pmoc_model* so, pmoc_vec b, pmoc_vec bs, double* Psi, do
     return fail(PMOC_EINVAL, "Psi_SO parameters incomplete");
   SoArgs a{};
   a.m = *so; a.b = b; a.bs = bs; a.Psi = Psi; a.Psi_Ek = Psi_Ek; a.Psi_GM = Psi_GM; a.ys = ys; a.status = status;
-  a.nyp = (so->ny + 3) & ~3;
   const bool bvp = so->so_c.ptr != nullptr;
   PM_DISPATCH_LPL(so->nz, {
-    a.nzp = 32 * LPL;
-    const size_t smem =
-        sizeof(double) * (size_t)(a.nzp + 4 + a.nyp + 4 * a.nzp + 3 * a.nyp * kWarpsPerBlock);
+    const size_t smem = so_smem(LPL, so->ny).bytes(kWarpsPerBlock);
     if (smem > kMaxSmemPerBlock) return fail_smem("ny", so->ny, smem);
     if (bvp) return launch(k_so<LPL, true>, blocks_for(so->M), 32 * kWarpsPerBlock, smem, stream, a);
     return launch(k_so<LPL, false>, blocks_for(so->M), 32 * kWarpsPerBlock, smem, stream, a);
@@ -435,9 +483,7 @@ int pmoc_ml_timestep(const pmoc_model* ml, pmoc_vec b_basin, pmoc_vec Psi_b, dou
     return fail(PMOC_EINVAL, "SO_ML parameters incomplete");
   MlArgs a{};
   a.m = *ml; a.b_basin = b_basin; a.Psi_b = Psi_b; a.dt = dt; a.status = status;
-  a.nzp = (ml->nz + 3) & ~3;
-  a.nyp = (ml->ny + 3) & ~3;
-  const size_t smem = sizeof(double) * (size_t)(a.nyp + (2 * a.nzp + a.nyp + 320) * kWarpsPerBlock);
+  const size_t smem = ml_smem(ml->nz, ml->ny).bytes(kWarpsPerBlock);
   if (smem > 200 * 1024) return fail(PMOC_EUNSUPPORTED, "nz too large for the stand-alone SO_ML kernel");
   return launch(k_ml, blocks_for(ml->M), 32 * kWarpsPerBlock, smem, stream, a);
 }

@@ -23,19 +23,36 @@ struct TwColArgs {
   MemberList list;
 };
 
+// Shared memory of k_twcol (in doubles).  Per block: nine level tables of the grid; per member (32 / G a warp): five
+// of its own.  Each table has a slot j*G + s for level s*LPL + j.
+struct TwcolSmem {
+  int nl, off_tab, off_warp0, per_member, per_warp;
+  PM_HD constexpr size_t bytes(int wpb) const { return sizeof(double) * (size_t)(off_warp0 + wpb * per_warp); }
+};
+PM_HD constexpr TwcolSmem twcol_smem(int G, int LPL) {
+  TwcolSmem s{};
+  s.nl = G * LPL;
+  s.off_warp0 = s.off_tab + 9 * s.nl;
+  s.per_member = 5 * s.nl;
+  s.per_warp = 32 / G * s.per_member;
+  return s;
+}
+
 // LIST: launched over an active list (a.list.members != NULL); the plain launch compiles without its extra path
 template <int G, int LPL, bool LIST>
 PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
   constexpr int MPW = 32 / G;   // members per warp
-  constexpr int NL = G * LPL;   // level slots of a member
+  constexpr TwcolSmem sl = twcol_smem(G, LPL);
+  constexpr int NL = sl.nl;     // level slots of a member
   const pmoc_model& M = a.m;
   const int nz = M.nz;
   const int L = rt::lane(), W = rt::warp_in_block(), nthr = rt::warps_per_block() * 32, tid = W * 32 + L;
   const int s = L & (G - 1), grp = L / G;
   double* sm = rt::smem();
-  // block tables, slot j*G + s (all groups of a warp read the same words: broadcast)
-  double *t_h = sm, *t_hh = sm + NL, *t_a = sm + 2 * NL, *t_c = sm + 3 * NL, *t_zf = sm + 4 * NL, *t_rdu = sm + 5 * NL,
-         *t_rdd = sm + 6 * NL, *t_ruu = sm + 7 * NL, *t_rdd2 = sm + 8 * NL;
+  // block tables (all groups of a warp read the same words: broadcast)
+  double* tab = sm + sl.off_tab;
+  double *t_h = tab, *t_hh = tab + NL, *t_a = tab + 2 * NL, *t_c = tab + 3 * NL, *t_zf = tab + 4 * NL,
+         *t_rdu = tab + 5 * NL, *t_rdd = tab + 6 * NL, *t_ruu = tab + 7 * NL, *t_rdd2 = tab + 8 * NL;
   {
     const double* z = M.z;
     const double z0 = z[0], H = z[nz - 1] - z[0];
@@ -59,8 +76,8 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
   const long long m = LIST ? a.list.members[slot] : slot;
   if (rt::ballot(live) == 0) return;
   auto group_mask = [&]() { return (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (grp * G); };
-  // per-member tables (slot j*G + s): the four stream-function independent products of the folded stencil, d(A kappa)/dz
-  double* mt = sm + 9 * NL + (size_t)(W * MPW + grp) * 5 * NL;
+  // per-member tables: the four stream-function independent products of the folded stencil, d(A kappa)/dz
+  double* mt = sm + sl.off_warp0 + (size_t)(W * MPW + grp) * sl.per_member;
   double *m_pk = mt, *m_qk = mt + NL, *m_pa = mt + 2 * NL, *m_qa = mt + 3 * NL, *m_dak = mt + 4 * NL;
   const double dt = M.dt;
   double b[LPL], b2[LPL], p[LPL], q[LPL];
@@ -296,10 +313,10 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(128, 4) k_twcol(TwColArgs a) {
 
 template <int G, int LPL>
 static int launch_twcol(const TwColArgs& a, void* stream) {
-  constexpr int wpb = 4, MPW = 32 / G, NL = G * LPL;
+  constexpr int wpb = 4, MPW = 32 / G;
   const long long per_block = (long long)wpb * MPW;
   const long long grid = (a.list.slots(a.m.M) + per_block - 1) / per_block;
-  const size_t smem = sizeof(double) * (size_t)(9 * NL + wpb * MPW * 5 * NL);
+  constexpr size_t smem = twcol_smem(G, LPL).bytes(wpb);
   if (a.list.members) return launch(k_twcol<G, LPL, true>, grid, 32 * wpb, smem, stream, a);
   return launch(k_twcol<G, LPL, false>, grid, 32 * wpb, smem, stream, a);
 }

@@ -866,6 +866,20 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol + (PIPE ? 32 : 0), 1) k_wide_steps2(Wid
   if (t == 0 && M.status) M.status[m] = status_word(M.status[m], all, so1_exact);
 }
 
+// Shared memory of k_wide_post (in doubles): -weff and kappa of each column ([NCOL][nzp] each), the first and last
+// level of every thread ([2][NCOL][2 * kWideCol]), the convection flags ([3][NCOL][2] ints: any level above bs, top
+// stable level) and 4 ints for the block collectives.
+struct WidePostSmem {
+  int off_nw, off_kp, off_edge, off_flg, off_cbox, size;
+  PM_HD constexpr size_t bytes() const { return sizeof(double) * (size_t)size; }
+};
+PM_HD constexpr WidePostSmem wide_post_smem(int LPT, int NCOL) {
+  WidePostSmem s{};
+  s.off_kp = s.off_nw + NCOL * kWideCol * LPT; s.off_edge = s.off_kp + NCOL * kWideCol * LPT;
+  s.off_flg = s.off_edge + 4 * NCOL * kWideCol; s.off_cbox = s.off_flg + 3 * NCOL; s.size = s.off_cbox + 2;
+  return s;
+}
+
 // ---- the steps of the 'post' order (example_twocol_plusSO.py:99-115) ----------------------------
 // NCOL columns (the basin; and the northern column of the two-column models), each advanced by
 // Column.timestep(wA, dt, do_conv) with the streamfunctions of the last diagnosis, which the host loop
@@ -887,12 +901,13 @@ PM_GLOBAL void PM_LAUNCH_BOUNDS(kWideCol, LPT == 4 ? 2 : 1) k_wide_post(WideArgs
   const long long m = wide_member<LIST>(a);
   const double dt = M.dt;
   constexpr int nzp = kWideCol * LPT;
+  constexpr WidePostSmem sl = wide_post_smem(LPT, NCOL);
   double* sm = rt::smem();
-  double* nws = sm;                                  // [NCOL][nzp] -weff
-  double* kps = sm + NCOL * nzp;                     // [NCOL][nzp] kappa
-  double* edge = sm + 2 * NCOL * nzp;                // [2][NCOL][2 * kWideCol] first / last level of every thread
-  int* flg = reinterpret_cast<int*>(edge + 4 * NCOL * kWideCol);  // [3][NCOL][2] any level above bs, top stable level
-  int* cbox = flg + 6 * NCOL;                        // the block collectives
+  double* nws = sm + sl.off_nw;
+  double* kps = sm + sl.off_kp;
+  double* edge = sm + sl.off_edge;
+  int* flg = reinterpret_cast<int*>(sm + sl.off_flg);
+  int* cbox = reinterpret_cast<int*>(sm + sl.off_cbox);
   const double* z = M.z;
   const int lo = t * LPT;
   double* rarea = a.memb + (size_t)m * 6 * nz;       // [NCOL][nz] 1 / Area (non-uniform Area)
@@ -1069,10 +1084,6 @@ size_t wide_steps2_smem(int lpt, int ny) {
   return sizeof(double) * (size_t)(6 * nzp + kWideCol + 2 * kWideCol + 2 + 2 * nyp + 320 + 8 + 10 + pm::kMlSave);
 }
 
-size_t wide_post_smem(int lpt, int ncol) {
-  return sizeof(double) * (size_t)(2 * ncol * kWideCol * lpt + 4 * ncol * kWideCol) + sizeof(int) * (size_t)(6 * ncol + 4);
-}
-
 size_t wide_refresh_smem(int nz, int ny, int nb) {
   const int nbp = (nb + 3) & ~3, nyp = (ny + 3) & ~3;
   return sizeof(double) * (size_t)(6 * nz + nbp + nbp / 2 + 2 + 64 + kWideThreads + 3 * nyp + 4);
@@ -1097,7 +1108,7 @@ static int wide_loop(WideArgs a, bool post, int diagnose_only, long long nsteps,
     auto kern = lpt == 4 ? (two ? k_wide_post<4, 2, LIST> : k_wide_post<4, 1, LIST>)
               : lpt == 8 ? (two ? k_wide_post<8, 2, LIST> : k_wide_post<8, 1, LIST>)
                          : (two ? k_wide_post<16, 2, LIST> : k_wide_post<16, 1, LIST>);
-    const size_t sm_s = wide_post_smem(lpt, two ? 2 : 1);
+    const size_t sm_s = wide_post_smem(lpt, two ? 2 : 1).bytes();
     while (ii < it_end) {
       const long long stop = ((ii + K - 1) / K) * K;  // first iteration with it % K == 0 at or after ii
       const bool hits = stop < it_end;
